@@ -17,8 +17,12 @@ config-5 microbenchmark (batched edit distance, 2^20 tasks per cell).  `--only c
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA path through the C ABI)
   python bench.py --impl reference [...]                         CPU arm: the multithreaded CPU port of the reference path
                                                                  (the reference binary cannot be built offline, DESIGN.md)
+  python bench.py [...] --dump-outputs bench_outputs             also writes the headline's result of its last timed step
+                                                                 as .npy files to that directory (dump_outputs); the inputs
+                                                                 are seeded, so two builds compare file by file
 
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  Runs from the tree as build() left it and writes nothing into it: the tree may be
+read-only.
 """
 from __future__ import annotations
 
@@ -35,6 +39,7 @@ import zlib
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # no __pycache__ in the tree from a benchmark run
 
 # the library asks for 32 hardware work queues when it is loaded (floxer_gpu.cu, fxg_on_load); torch may create the CUDA
 # context before that, so the same default is set here, before torch is imported
@@ -127,6 +132,39 @@ def digest(al, cg, with_cigars: bool) -> int:
     return h
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, al, cg, stats: dict):
+    """Writes what one verification job hands its caller, so that two builds can be compared output for output:
+
+      alignments.npy  float64 [n, 7]: alignment index, read_index, reference_id, orientation, start_in_reference,
+                      num_errors, cigar_len -- in the job's output order
+      cigars.npy      float32: the cigars of those alignments one after the other, every operation as count << 4 | code
+                      (exact in float32: a count stays far below 2^20)
+      stats.npy       float64 [8]: the job's statistics in abi.Stats order
+
+    cigar_offset and the gaps of the cigar pool are layout, not result, and are left out.  Where the files would pass
+    DUMP_LIMIT_BYTES, a fixed, seeded sample of the alignments (kept in output order) is written instead."""
+    n = len(al)
+    ln = al["cigar_len"].astype(np.int64)
+    row_bytes = 7 * 8 + 4 * ln
+    keep = np.arange(n)
+    budget = DUMP_LIMIT_BYTES - 8 * 8 - 3 * 4096            # stats and the three .npy headers
+    if int(row_bytes.sum()) > budget:
+        order = np.random.default_rng(20240000).permutation(n)
+        keep = np.sort(order[np.cumsum(row_bytes[order]) <= budget])
+    sel, ln = al[keep], ln[keep]
+    rows = np.stack([keep, sel["read_index"], sel["reference_id"], sel["orientation"], sel["start_in_reference"],
+                     sel["num_errors"], ln], axis=1).astype(np.float64)
+    first = np.cumsum(ln) - ln
+    at = np.repeat(sel["cigar_offset"].astype(np.int64) - first, ln) + np.arange(int(ln.sum()))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "alignments.npy"), rows)
+    np.save(os.path.join(out_dir, "cigars.npy"), cg[at].astype(np.float32))
+    np.save(os.path.join(out_dir, "stats.npy"), np.array(list(stats.values()), dtype=np.float64))
+
+
 def cpu_arm(refs, batch, cfg, threads: int, target_s: float):
     """Times the multithreaded CPU port on a bounded sample (first reads of the batch); returns a cpu_baseline object.
     A probe of one read per thread gives the rate; the sample is sized for about target_s seconds of wall time on all
@@ -189,9 +227,10 @@ def step_spread(done, n_each):
 
 
 def measure(ctx, g, torch, dist, refs, batch, cfg, lanes: int, steps: int, warmup: int, int32_peak: float, sampler, pageable: bool,
-            cpu_threads: int, cpu_target_s: float, rank: int):
+            cpu_threads: int, cpu_target_s: float, rank: int, dump_dir: str | None = None):
     """Device-resident arm, end-to-end arm (page-locked inputs; pageable as well if asked), result check, roofline and CPU
-    baseline of one workload.  Returns (record for rank 0, [ms_total, e2e_ms_total], [cells, reads])."""
+    baseline of one workload.  Returns (record for rank 0, [ms_total, e2e_ms_total], [cells, reads]).  With dump_dir, rank 0
+    writes the result of the device-resident arm's last timed step there (dump_outputs)."""
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
     def barrier():
@@ -252,6 +291,11 @@ def measure(ctx, g, torch, dist, refs, batch, cfg, lanes: int, steps: int, warmu
         bad += digest(a, c, True) != want
     if bad:
         raise RuntimeError(f"{bad} of {lanes} lanes of the device-resident arm ended with results that differ from a batch run alone")
+    if dump_dir and rank == 0:
+        # every lane ran the same batch and, as checked above, ended with the same result: lane 0's stands for the step
+        a, c = jobs[0].alignments(copy=False)
+        dump_outputs(dump_dir, a, c, jobs[0].stats())
+        del a, c
     spread = step_spread(done, steps)
     for j in jobs:
         j.free()
@@ -473,7 +517,12 @@ def main() -> int:
     ap.add_argument("--cpu-seconds", type=float, default=2.0, help="wall time of every CPU baseline sample on all host threads (about 30 core-seconds on 16 cores)")
     ap.add_argument("--big-lanes", type=int, default=4, help="host threads that submit batches concurrently (configs 3 and 4: one batch fills the machine; "
                     "the others keep it fed while a caller stages its next batch -- measured 2 -> 4: config-4 shard end to end 18 k -> 25 k reads/s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's result of its last timed step (with --impl reference: the CPU port's) to "
+                         "DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -503,8 +552,10 @@ def main() -> int:
         times, stats = [], None
         for _ in range(max(args.steps, 1)):
             t0 = time.perf_counter()
-            _, _, stats = cpu_baseline.verify_reads(refs, sample, cfg, threads=threads)
+            al, cg, stats = cpu_baseline.verify_reads(refs, sample, cfg, threads=threads)
             times.append(time.perf_counter() - t0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, al, cg, stats)
         sec = sum(times) / len(times)
         gcups = (stats["cells_inner"] + stats["cells_root"]) / sec / 1e9
         line = {"impl": "reference", "metric": "pex_verification_gcups", "value": gcups, "unit": "GCUPS",
@@ -577,7 +628,7 @@ def main() -> int:
             ("config2_seeded", False, args.lanes, max(3, args.steps // 2), False),
             ("config3", False, args.big_lanes, max(3, args.steps // 4), False), ("config3", True, args.big_lanes, max(3, args.steps // 4), False),
             ("config4_shard", False, args.big_lanes, max(3, args.steps // 5), False), ("config4_shard", True, args.big_lanes, max(3, args.steps // 5), False)]
-    current = None
+    current, measured = None, False
     for name, ivopt, lanes, steps, is_head in plan:
         key = name + ("_ivopt" if ivopt else "")
         if name not in made or not (want(key) or (ivopt and want(name) and name != "config2")):
@@ -589,8 +640,10 @@ def main() -> int:
             if int32_peak is None:
                 int32_peak = ctx.measure_int32_peak()
         cfg = VerifyConfig(interval_optimization=ivopt, without_cigar=os.environ.get("BENCH_WITHOUT_CIGAR") == "1")      # (development: the path without tracebacks)
+        # the first workload measured is the headline, or what stands in for it under --only
         rec = measure(ctx, g, torch, dist, refs, batch, cfg, lanes, steps, args.warmup, int32_peak, sampler, pageable=is_head,
-                      cpu_threads=threads, cpu_target_s=args.cpu_seconds, rank=rank)
+                      cpu_threads=threads, cpu_target_s=args.cpu_seconds, rank=rank, dump_dir=None if measured else args.dump_outputs)
+        measured = True
         if rec is not None:
             rec["config"] = {"workload": describe(name, ivopt, len(batch), anchors), "lanes": lanes, "steps": steps,
                              "l2": "256 MiB written to HBM between batches (twice the 126 MB L2); the lanes run concurrently, so a batch never finds its own data in L2"}
