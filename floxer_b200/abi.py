@@ -65,6 +65,14 @@ class Counters(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class SeedStats(C.Structure):
+    _fields_ = [(n, C.c_uint64) for n in (
+        "seeds", "candidates", "checked", "hits", "dropped_hard", "cut_soft", "erased", "reserved")]
+
+    def as_dict(self) -> dict:
+        return {n: int(getattr(self, n)) for n, _ in self._fields_ if n != "reserved"}
+
+
 def cigar_to_string(ops) -> str:
     return "".join(f"{int(o) >> 4}{CIGAR_CHARS[int(o) & 15]}" for o in ops)
 

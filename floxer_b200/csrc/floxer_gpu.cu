@@ -12,9 +12,11 @@
 #include "../../include/floxer_gpu.h"
 #include "dp_kernels.cuh"
 #include "root_kernels.cuh"
+#include "seed_kernels.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
 
 #include <algorithm>
 #include <atomic>
@@ -382,6 +384,7 @@ struct fxg_ctx {
     std::mutex class_mu;
     ClassDef classes[kMaxLevelClasses];
     int n_classes = 0;
+    int seeders_reading = 0;             // fxg_gpu_seeder_create / fxg_seed_reads calls that read the packed store without mu
 };
 
 struct fxg_batch {
@@ -2801,6 +2804,7 @@ int fxg_set_references(fxg_ctx* c, size_t n_refs, const uint8_t* const* ranks, c
     for (int i = 0; i < c->n_groups; ++i)
         if (c->groups[i].busy) return fail(c->err, FXG_ERR_STATE, "fxg_set_references while a run is in flight");
     if (!c->pending.empty()) return fail(c->err, FXG_ERR_STATE, "fxg_set_references while a run is in flight");
+    if (c->seeders_reading) return fail(c->err, FXG_ERR_STATE, "fxg_set_references while a seeding call is in flight");
     // everything new is built beside the old store and takes its place only when every upload has succeeded
     std::vector<uint64_t> base(n_refs, 0), len(lens, lens + n_refs);
     uint64_t total = 0;
@@ -3543,6 +3547,363 @@ int fxg_measure_int32_peak(fxg_ctx* c, double* out) {
     }
     *out = best;
     return FXG_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ device seeder
+
+struct fxg_gpu_seeder {
+    uint64_t ctx_serial = 0;
+    uint64_t refs_version = 0;           // RefStore::version the index was built from
+    uint32_t q = 0, n_refs = 0;
+    DevBuf bucket, pos;                  // 4^q + 1 offsets, positions in the unpadded concatenation
+    DevBuf ubase, pbase, len;            // per reference: unpadded start, start in the store, length
+    uint64_t budget = 0;                 // FXG_SEED_CANDIDATES: q-gram occurrences per chunk
+    void release() { bucket.release(); pos.release(); ubase.release(); pbase.release(); len.release(); }
+};
+
+namespace {
+
+constexpr uint32_t kSeedChunkSeeds = 1u << 27;      // hit keys hold the seed of a chunk in 28 bits
+
+// Keeps the context's packed store in place while a seeding call reads it without holding mu: fxg_set_references
+// refuses to replace the store while the count is non-zero.
+struct StoreReader {
+    fxg_ctx* c;
+    bool on = false;
+    ~StoreReader() { if (on) { std::lock_guard<std::mutex> lock(c->mu); c->seeders_reading--; } }
+};
+
+// a call's own stream and buffers; the stream is drained before the buffers go back to the pool
+struct SeedCall {
+    explicit SeedCall(fxg_ctx* ctx) : c(ctx) {}
+    fxg_ctx* c;
+    cudaStream_t st = nullptr;
+    DevBuf bufs[20];
+    PinnedBuf host;
+    ~SeedCall() {
+        if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
+        for (DevBuf& b : bufs) b.release();
+        if (host.p) { std::lock_guard<std::mutex> lock(c->mu); give_staging(c, host); }
+    }
+};
+
+int bits_for(uint64_t v) { int b = 1; while (b < 64 && (v >> b)) ++b; return b; }     // bits that hold 0..v
+
+uint32_t seed_grid(uint64_t n, uint32_t threads = 256) { return uint32_t(std::max<uint64_t>(1, (n + threads - 1) / threads)); }
+
+// the store's tables as the seeder's kernels read them
+SeedRefs seed_refs(const fxg_gpu_seeder* S, const uint32_t* packed) {
+    return SeedRefs{packed, S->ubase.as<uint64_t>(), S->pbase.as<uint64_t>(), S->len.as<uint64_t>(), S->n_refs};
+}
+
+// takes the store for a seeding call: the references must be those the seeder was made from (if it is given)
+int take_store(fxg_ctx* c, const fxg_gpu_seeder* S, StoreReader& guard, const uint32_t*& packed, std::vector<uint64_t>* len,
+               std::vector<uint64_t>* pbase, uint64_t* version, std::string& err) {
+    std::lock_guard<std::mutex> lock(c->mu);
+    if (!c->have_refs) return fail(err, FXG_ERR_STATE, "fxg_set_references must be called first");
+    if (S && (S->ctx_serial != c->serial || S->refs_version != c->refs.version))
+        return fail(err, FXG_ERR_STATE, "the references were replaced after the seeder was made (or it belongs to another context)");
+    packed = c->refs.packed.as<uint32_t>();
+    if (len) *len = c->refs.len;
+    if (pbase) *pbase = c->refs.base;
+    if (version) *version = c->refs.version;
+    c->seeders_reading++;
+    guard.on = true;
+    return FXG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fxg_gpu_seeder_create(fxg_ctx* c, uint32_t q, fxg_gpu_seeder** out) {
+    if (!c || !out) return FXG_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    std::string err;
+    if (q < 4 || q > 14) return fail(err, FXG_ERR_INVALID_ARGUMENT, "q = %u: the index takes q-grams of 4..14 bases", q);
+    CUDA_TRY(err, cudaSetDevice(c->device));
+    std::unique_ptr<fxg_gpu_seeder> S(new (std::nothrow) fxg_gpu_seeder());
+    if (!S) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate the seeder");
+    StoreReader guard{c};
+    const uint32_t* packed = nullptr;
+    std::vector<uint64_t> len, pbase;
+    if (int rc = take_store(c, nullptr, guard, packed, &len, &pbase, &S->refs_version, err)) return rc;
+    S->ctx_serial = c->serial;
+    S->q = q;
+    S->n_refs = uint32_t(len.size());
+    std::vector<uint64_t> ubase(len.size());
+    uint64_t total = 0;
+    for (size_t r = 0; r < len.size(); ++r) { ubase[r] = total; total += len[r]; }
+    if (total >= (uint64_t(1) << 32))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "the references hold %llu bases: positions are 32-bit, index below 4 Gbp", (unsigned long long)total);
+    S->budget = uint64_t(env_int("FXG_SEED_CANDIDATES", 1 << 26, 1, INT32_MAX));
+    SeedCall K{c};
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    size_t const nr = std::max<size_t>(len.size(), 1);
+    CUDA_TRY(err, S->ubase.ensure(nr * 8));
+    CUDA_TRY(err, S->pbase.ensure(nr * 8));
+    CUDA_TRY(err, S->len.ensure(nr * 8));
+    if (!len.empty()) {
+        CUDA_TRY(err, cudaMemcpyAsync(S->ubase.p, ubase.data(), len.size() * 8, cudaMemcpyHostToDevice, K.st));
+        CUDA_TRY(err, cudaMemcpyAsync(S->pbase.p, pbase.data(), len.size() * 8, cudaMemcpyHostToDevice, K.st));
+        CUDA_TRY(err, cudaMemcpyAsync(S->len.p, len.data(), len.size() * 8, cudaMemcpyHostToDevice, K.st));
+    }
+    // counting sort: counts per code, exclusive scan into the buckets, scatter through a copy of the buckets
+    size_t const n_codes = size_t(1) << (2 * q);
+    DevBuf& counts = K.bufs[0];
+    DevBuf& tmp = K.bufs[1];
+    CUDA_TRY(err, counts.ensure((n_codes + 1) * 4));
+    CUDA_TRY(err, S->bucket.ensure((n_codes + 1) * 4));
+    CUDA_TRY(err, cudaMemsetAsync(counts.p, 0, (n_codes + 1) * 4, K.st));
+    SeedRefs const R = seed_refs(S.get(), packed);
+    uint32_t const grid = uint32_t(std::min<uint64_t>(seed_grid(total), uint64_t(c->num_sms) * 16));
+    if (total) {
+        seed_index_count_kernel<<<grid, 256, 0, K.st>>>(R, total, q, counts.as<uint32_t>());
+        CUDA_TRY(err, cudaGetLastError());
+    }
+    size_t tmp_bytes = 0;
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts.as<uint32_t>(), S->bucket.as<uint32_t>(), n_codes + 1, K.st));
+    CUDA_TRY(err, tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, counts.as<uint32_t>(), S->bucket.as<uint32_t>(), n_codes + 1, K.st));
+    uint32_t n_pos = 0;
+    CUDA_TRY(err, cudaMemcpyAsync(&n_pos, S->bucket.as<uint32_t>() + n_codes, 4, cudaMemcpyDeviceToHost, K.st));
+    CUDA_TRY(err, cudaStreamSynchronize(K.st));
+    CUDA_TRY(err, S->pos.ensure(std::max<size_t>(n_pos, 1) * 4));
+    CUDA_TRY(err, cudaMemcpyAsync(counts.p, S->bucket.p, (n_codes + 1) * 4, cudaMemcpyDeviceToDevice, K.st));
+    if (n_pos) {
+        seed_index_fill_kernel<<<grid, 256, 0, K.st>>>(R, total, q, counts.as<uint32_t>(), S->pos.as<uint32_t>());
+        CUDA_TRY(err, cudaGetLastError());
+    }
+    CUDA_TRY(err, cudaStreamSynchronize(K.st));
+    *out = S.release();
+    return FXG_OK;
+}
+
+void fxg_gpu_seeder_free(fxg_ctx* c, fxg_gpu_seeder* S) {
+    if (!S) return;
+    if (c) cudaSetDevice(c->device);
+    S->release();
+    delete S;
+}
+
+int fxg_seed_reads(fxg_ctx* c, const fxg_gpu_seeder* S, fxg_read* reads, size_t n_reads,
+                   const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                   const fxg_pex_node* nodes, size_t n_nodes,
+                   uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                   fxg_anchor** anchors, size_t* n_anchors, fxg_seed_stats* stats) {
+    if (!c || !S || !anchors || !n_anchors || (n_reads && !reads) || (pool_len && (!forward_pool || !reverse_complement_pool)) || (n_nodes && !nodes))
+        return FXG_ERR_INVALID_ARGUMENT;
+    *anchors = nullptr; *n_anchors = 0;
+    fxg_seed_stats st{};
+    std::string err;
+    // ---- every read and leaf on the host, before any launch: what fxg_seeder_search refuses fails the whole call ----
+    if (pool_len >= (uint64_t(1) << 38)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "query pools of %zu bytes: at most 2^38", pool_len);
+    std::vector<uint32_t> seed_base(n_reads + 1), leaf_base(n_reads + 1);
+    uint64_t n_leaves = 0;
+    for (size_t i = 0; i < n_reads; ++i) {
+        fxg_read const& R = reads[i];
+        if (R.query_offset > pool_len || R.query_len > pool_len - R.query_offset) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: query outside the pool", i);
+        if (R.query_len > FXG_MAX_QUERY_LENGTH) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: longer than %d", i, FXG_MAX_QUERY_LENGTH);
+        if (R.node_offset > n_nodes || uint64_t(R.num_inner) + R.num_leaves > n_nodes - R.node_offset)
+            return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad node range", i);
+        leaf_base[i] = uint32_t(n_leaves);
+        seed_base[i] = uint32_t(2 * n_leaves);
+        n_leaves += R.num_leaves;
+        if (2 * n_leaves >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "more than 2^30 leaves in one call");
+    }
+    leaf_base[n_reads] = uint32_t(n_leaves);
+    seed_base[n_reads] = uint32_t(2 * n_leaves);
+    std::vector<uint64_t> leaf_info(n_leaves);
+    for (size_t i = 0; i < n_reads; ++i) {
+        fxg_read const& R = reads[i];
+        const fxg_pex_node* lv = nodes + R.node_offset + R.num_inner;
+        for (uint32_t li = 0; li < R.num_leaves; ++li) {
+            fxg_pex_node const& leaf = lv[li];
+            if (leaf.query_index_to < leaf.query_index_from || leaf.query_index_to >= R.query_len)
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: outside the query", i, li);
+            uint32_t const m = uint32_t(leaf.query_index_to - leaf.query_index_from + 1), e = uint32_t(leaf.num_errors);
+            if (e > uint32_t(kSeedMaxErrors) || m / (e + 1) < S->q)
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: %u bases with %u errors (at most %d errors and q * (errors + 1) = %u bases)",
+                            i, li, m, e, kSeedMaxErrors, S->q * (e + 1));
+            leaf_info[leaf_base[i] + li] = seed_pack(R.query_offset + leaf.query_index_from, m, e);
+        }
+    }
+    uint32_t const n_seeds = uint32_t(2 * n_leaves);
+    st.seeds = n_seeds;
+    auto finish = [&](std::vector<uint32_t> const& per_read) {
+        uint64_t at = 0;
+        for (size_t i = 0; i < n_reads; ++i) {
+            reads[i].anchor_offset = at;
+            reads[i].num_anchors_forward = per_read.empty() ? 0 : per_read[2 * i];
+            reads[i].num_anchors_reverse = per_read.empty() ? 0 : per_read[2 * i + 1];
+            at += uint64_t(reads[i].num_anchors_forward) + reads[i].num_anchors_reverse;
+        }
+        if (stats) *stats = st;
+        return FXG_OK;
+    };
+    StoreReader guard{c};
+    const uint32_t* packed = nullptr;
+    if (int rc = take_store(c, S, guard, packed, nullptr, nullptr, nullptr, err)) return rc;
+    if (n_seeds == 0) return finish({});
+    CUDA_TRY(err, cudaSetDevice(c->device));
+
+    // ---- uploads and the seeds' plan ----
+    SeedCall K{c};
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
+    DevBuf &d_pool = K.bufs[0], &d_seed_base = K.bufs[1], &d_leaf_base = K.bufs[2], &d_leaves = K.bufs[3], &d_info = K.bufs[4],
+           &d_occ = K.bufs[5], &d_off = K.bufs[6], &d_ctr = K.bufs[7], &d_per_read = K.bufs[8], &d_keys = K.bufs[9], &d_sorted = K.bufs[10],
+           &d_uniq = K.bufs[11], &d_nuniq = K.bufs[12], &d_hits = K.bufs[13], &d_hits2 = K.bufs[14], &d_gone = K.bufs[15], &d_at = K.bufs[16],
+           &d_out = K.bufs[17], &d_tmp = K.bufs[18];
+    cudaStream_t const s = K.st;
+    CUDA_TRY(err, d_pool.ensure(2 * pool_len + 64));
+    if (pool_len) {
+        CUDA_TRY(err, cudaMemcpyAsync(d_pool.p, forward_pool, pool_len, cudaMemcpyHostToDevice, s));
+        CUDA_TRY(err, cudaMemcpyAsync(d_pool.as<uint8_t>() + pool_len, reverse_complement_pool, pool_len, cudaMemcpyHostToDevice, s));
+    }
+    CUDA_TRY(err, d_seed_base.ensure((n_reads + 1) * 4));
+    CUDA_TRY(err, d_leaf_base.ensure((n_reads + 1) * 4));
+    CUDA_TRY(err, d_leaves.ensure(n_leaves * 8));
+    CUDA_TRY(err, cudaMemcpyAsync(d_seed_base.p, seed_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(err, cudaMemcpyAsync(d_leaf_base.p, leaf_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(err, cudaMemcpyAsync(d_leaves.p, leaf_info.data(), n_leaves * 8, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(err, d_info.ensure(size_t(n_seeds) * 8));
+    CUDA_TRY(err, d_occ.ensure(size_t(n_seeds) * 8));
+    CUDA_TRY(err, d_off.ensure((size_t(n_seeds) + 1) * 8));
+    CUDA_TRY(err, d_ctr.ensure(8 * 8));
+    CUDA_TRY(err, d_per_read.ensure(n_reads * 8));
+    CUDA_TRY(err, cudaMemsetAsync(d_per_read.p, 0, n_reads * 8, s));
+    CUDA_TRY(err, cudaMemsetAsync(d_off.p, 0, 8, s));
+    SeedRefs const R = seed_refs(S, packed);
+    SeedBatch const B{d_pool.as<uint8_t>(), pool_len, d_seed_base.as<uint32_t>(), d_leaf_base.as<uint32_t>(), d_leaves.as<uint64_t>(),
+                      uint32_t(n_reads), n_seeds, S->bucket.as<uint32_t>(), S->pos.as<uint32_t>(), S->q};
+    seed_plan_kernel<<<seed_grid(n_seeds), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_occ.as<uint64_t>());
+    CUDA_TRY(err, cudaGetLastError());
+    size_t tmp_bytes = 0;
+    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
+    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(d_tmp.p, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
+    CUDA_TRY(err, K.host.ensure(std::max<size_t>(4096, n_reads * 8)));
+    uint64_t* h_ctr = K.host.as<uint64_t>();             // (moves when the buffer grows)
+    CUDA_TRY(err, cudaMemcpyAsync(h_ctr, d_off.as<uint64_t>() + n_seeds, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    uint64_t const total_occ = h_ctr[0];
+
+    // ---- chunks of whole seeds under the budget of q-gram occurrences (a seed above it gets a chunk of its own) ----
+    std::vector<uint64_t> off;                     // host copy of the offsets, only when the batch needs several chunks
+    if (total_occ > S->budget || n_seeds > kSeedChunkSeeds) {
+        off.resize(size_t(n_seeds) + 1);
+        CUDA_TRY(err, cudaMemcpyAsync(off.data(), d_off.p, off.size() * 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+    }
+    auto off_at = [&](uint32_t i) { return off.empty() ? (i == 0 ? 0 : total_occ) : off[i]; };
+    fxg_anchor* result = nullptr;
+    size_t n_result = 0;
+    struct FreeResult { fxg_anchor*& p; bool keep = false; ~FreeResult() { if (!keep) std::free(p); } } free_result{result};
+    for (uint32_t s0 = 0; s0 < n_seeds;) {
+        uint32_t s1 = n_seeds;
+        if (!off.empty()) {
+            s1 = uint32_t(std::upper_bound(off.begin() + s0 + 1, off.end(), off[s0] + S->budget) - off.begin()) - 1;
+            s1 = std::min(std::max(s1, s0 + 1), std::min(n_seeds, s0 + kSeedChunkSeeds));
+        }
+        uint64_t const N = off_at(s1) - off_at(s0);
+        uint32_t const ns = s1 - s0;
+        if (N == 0) { s0 = s1; continue; }
+        if (N >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "seeds %u..%u have %llu q-gram occurrences: build the index with a larger q",
+                                                  s0, s1 - 1, (unsigned long long)N);
+        int const n_items = int(N);
+        // candidates: (seed, nominal start) keys, sorted and made unique
+        CUDA_TRY(err, d_keys.ensure(N * 8));
+        CUDA_TRY(err, d_sorted.ensure(N * 8));
+        CUDA_TRY(err, d_uniq.ensure(N * 8));
+        CUDA_TRY(err, d_nuniq.ensure(8));
+        CUDA_TRY(err, cudaMemsetAsync(d_ctr.p, 0, 64, s));
+        unsigned long long* const ctr = d_ctr.as<unsigned long long>();
+        seed_emit_kernel<<<seed_grid(ns), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_off.as<uint64_t>(), s0, s1, d_keys.as<uint64_t>(), ctr);
+        CUDA_TRY(err, cudaGetLastError());
+        int const key_bits = std::min(64, kSeedKeyShift + bits_for(ns - 1));
+        size_t sort_bytes = 0, uniq_bytes = 0;
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
+        CUDA_TRY(err, cub::DeviceSelect::Unique(nullptr, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
+        CUDA_TRY(err, d_tmp.ensure(std::max(sort_bytes, uniq_bytes)));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
+        CUDA_TRY(err, cub::DeviceSelect::Unique(d_tmp.p, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
+        // check every distinct start; the hit buffer grows and the check runs again if it was too small
+        uint64_t hit_cap = std::max<uint64_t>(d_hits.cap / 8, N + 1024);
+        uint64_t n_hits = 0;
+        for (;;) {
+            CUDA_TRY(err, d_hits.ensure(hit_cap * 8));
+            seed_check_kernel<<<seed_grid(N), 256, 0, s>>>(R, B, d_info.as<uint64_t>(), s0, d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(),
+                                                           d_hits.as<uint64_t>(), hit_cap, ctr);
+            CUDA_TRY(err, cudaGetLastError());
+            CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(err, cudaStreamSynchronize(s));
+            n_hits = h_ctr[2];
+            if (n_hits <= hit_cap) break;
+            hit_cap = n_hits;
+            CUDA_TRY(err, cudaMemsetAsync(ctr + 1, 0, 16, s));
+        }
+        st.candidates += h_ctr[0]; st.checked += h_ctr[1]; st.hits += n_hits;
+        if (n_hits == 0) { s0 = s1; continue; }
+        // caps on hits ordered by (seed, errors, position), then the kept ones by (seed, position)
+        int const hit_items = int(n_hits);
+        CUDA_TRY(err, d_hits2.ensure(n_hits * 8));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
+        CUDA_TRY(err, d_tmp.ensure(sort_bytes));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0,
+                                                     std::min(64, kHitKeyShift + bits_for(ns - 1)), s));
+        seed_caps_kernel<<<seed_grid(n_hits), 256, 0, s>>>(d_hits2.as<uint64_t>(), n_hits, max_anchors_hard, max_anchors_soft, d_hits.as<uint64_t>(), ctr);
+        CUDA_TRY(err, cudaGetLastError());
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        st.dropped_hard += h_ctr[3]; st.cut_soft += h_ctr[4];
+        uint64_t const n_kept = n_hits - h_ctr[3] - h_ctr[4];
+        if (n_kept == 0) { s0 = s1; continue; }
+        // erase_useless_anchors, then the survivors in order
+        CUDA_TRY(err, d_gone.ensure(n_kept * 4));
+        CUDA_TRY(err, d_at.ensure(n_kept * 4));
+        CUDA_TRY(err, d_out.ensure(n_kept * sizeof(fxg_anchor)));
+        CUDA_TRY(err, cudaMemsetAsync(d_gone.p, 0, n_kept * 4, s));
+        if (erase_useless_anchors) {
+            seed_erase_kernel<<<seed_grid(n_kept), 256, 0, s>>>(R, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>());
+            CUDA_TRY(err, cudaGetLastError());
+        }
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
+        CUDA_TRY(err, d_tmp.ensure(tmp_bytes));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
+        seed_output_kernel<<<seed_grid(n_kept), 256, 0, s>>>(R, B, s0, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>(), d_at.as<uint32_t>(),
+                                                             d_out.as<uint64_t>(), d_per_read.as<uint32_t>(), ctr);
+        CUDA_TRY(err, cudaGetLastError());
+        // back through page-locked memory: the counters, then up to n_kept records
+        CUDA_TRY(err, K.host.ensure(64 + n_kept * sizeof(fxg_anchor)));
+        uint64_t* const h = h_ctr = K.host.as<uint64_t>();
+        CUDA_TRY(err, cudaMemcpyAsync(h, ctr, 64, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h + 8, d_out.p, n_kept * sizeof(fxg_anchor), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        st.erased += h[5];
+        uint64_t const n_out = n_kept - h[5];
+        if (n_out) {
+            fxg_anchor* grown = static_cast<fxg_anchor*>(std::realloc(result, (n_result + n_out) * sizeof(fxg_anchor)));
+            if (!grown) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate %llu anchors", (unsigned long long)(n_result + n_out));
+            result = grown;
+            std::memcpy(result + n_result, h + 8, n_out * sizeof(fxg_anchor));
+            n_result += n_out;
+        }
+        s0 = s1;
+    }
+    std::vector<uint32_t> per_read(2 * n_reads);
+    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_per_read.p, n_reads * 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    std::memcpy(per_read.data(), K.host.p, n_reads * 8);
+    uint64_t sum = 0;
+    for (uint32_t v : per_read) sum += v;
+    if (sum != n_result) return fail(err, FXG_ERR_CUDA, "internal: %llu anchors counted per read, %zu written", (unsigned long long)sum, n_result);
+    *anchors = result; *n_anchors = n_result;
+    free_result.keep = true;
+    return finish(per_read);
 }
 
 }  // extern "C"

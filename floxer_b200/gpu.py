@@ -23,6 +23,7 @@ EXPORTS = [
     "fxg_get_counters", "fxg_reset_counters", "fxg_measure_int32_peak", "fxg_engine_shape",
     "fxg_pex_build", "fxg_pex_free", "fxg_job_write_sam", "fxg_free", "fxg_write_bam", "fxg_job_write_bam",
     "fxg_seeder_create", "fxg_seeder_free", "fxg_seeder_search",
+    "fxg_gpu_seeder_create", "fxg_gpu_seeder_free", "fxg_seed_reads",
 ]
 
 _lib = None
@@ -88,6 +89,11 @@ def lib() -> C.CDLL:
     L.fxg_seeder_free.argtypes = [vp]
     L.fxg_seeder_free.restype = None
     L.fxg_seeder_search.argtypes = [vp, vp, sz, vp, sz, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(vp), C.POINTER(sz)]
+    L.fxg_gpu_seeder_create.argtypes = [vp, C.c_uint32, C.POINTER(vp)]
+    L.fxg_gpu_seeder_free.argtypes = [vp, vp]
+    L.fxg_gpu_seeder_free.restype = None
+    L.fxg_seed_reads.argtypes = [vp, vp, vp, sz, vp, vp, sz, vp, sz, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(vp), C.POINTER(sz),
+                                 C.POINTER(abi.SeedStats)]
     _lib = L
     return L
 
@@ -185,6 +191,27 @@ class Seeder:
     def close(self):
         if self._h:
             lib().fxg_seeder_free(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class GpuSeeder:
+    """fxg_gpu_seeder: the q-gram index of the references resident in `ctx`, built on the device; Context.seed_reads
+    searches whole read batches with it.  Invalid once ctx.set_references replaces the references."""
+
+    def __init__(self, ctx: "Context", q: int = 10):
+        self._ctx, self.q = ctx, q
+        self._h = C.c_void_p()
+        ctx._check(lib().fxg_gpu_seeder_create(ctx._h, q, C.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            lib().fxg_gpu_seeder_free(self._ctx._h, self._h)
             self._h = None
 
     def __del__(self):
@@ -386,6 +413,27 @@ class Context:
         h = C.c_void_p()
         self._check(lib().fxg_verify_reads(self._h, *args, C.byref(h)))
         return Job(self, h, (batch, cfg))
+
+    # ---- seeding on the device ----
+    def seed_reads(self, seeder: GpuSeeder, batch: ReadBatch, max_anchors_hard: int = 500, max_anchors_soft: int = 50,
+                   erase_useless: bool = True):
+        """fxg_seed_reads: both orientations of every read of `batch` (its pools, trees and read records; its anchors are
+        ignored).  Returns (a new ReadBatch with the anchors and the updated read records, stats dict); `batch` is not
+        modified.  The anchors of read i and orientation o equal Seeder.search(pool_o[i], leaves of i, ...)."""
+        reads = batch.reads.copy()
+        out, n, st = C.c_void_p(), C.c_size_t(0), abi.SeedStats()
+        self._check(lib().fxg_seed_reads(self._h, seeder._h, reads.ctypes.data, len(reads), batch.forward_pool.ctypes.data,
+                                         batch.reverse_pool.ctypes.data, len(batch.forward_pool), batch.nodes.ctypes.data,
+                                         len(batch.nodes), max_anchors_hard, max_anchors_soft, int(erase_useless),
+                                         C.byref(out), C.byref(n), C.byref(st)))
+        if n.value:
+            try:
+                anchors = np.frombuffer(C.string_at(out, n.value * abi.ANCHOR_DTYPE.itemsize), dtype=abi.ANCHOR_DTYPE).copy()
+            finally:
+                lib().fxg_free(out)
+        else:
+            anchors = np.zeros(0, dtype=abi.ANCHOR_DTYPE)
+        return ReadBatch(reads, batch.forward_pool, batch.reverse_pool, batch.nodes, anchors, dict(batch.meta)), st.as_dict()
 
     # ---- accounting ----
     def counters(self) -> dict:

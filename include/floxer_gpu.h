@@ -16,6 +16,9 @@
  *                        complement (src/lib/parallelization.cpp:14-43), including the shared
  *                        verified-interval sets (src/lib/intervals.cpp:84-127).
  *   *_stage/_run/_fetch  the same work split so that a caller can keep inputs resident in HBM.
+ *   fxg_seed_reads       search::searcher::search_seeds (src/lib/search.cpp:143-324) for both orientations of every read
+ *                        of a batch (src/lib/parallelization.cpp:94-101), on the device: the q-gram seeder of
+ *                        fxg_seeder_search with its index (fxg_gpu_seeder_create) built from the resident references.
  *
  * Struct layouts fxg_pex_node and fxg_anchor are byte-identical to pex::pex_tree::node
  * (include/pex.hpp:59-70) and search::anchor_t (include/search.hpp:27-31) on LP64, so the
@@ -165,6 +168,8 @@ typedef struct {
  *   FXG_SHARE_ROOTS   [1]   0: every root window is scored on its own
  *   FXG_ROOT_CHUNKS / FXG_ROOT_CHUNK_MIN, FXG_MERGED_PARTS, FXG_DEVICE_ROOTS, FXG_FORCE_WIDE, FXG_LATENCY_WEIGHT, FXG_PROFILE,
  *   FXG_TRACE_WAVES, FXG_TRACE_BATCHES: development aids (DESIGN.md)
+ *   FXG_SEED_CANDIDATES [2^26]  (read by fxg_gpu_seeder_create) q-gram occurrences one chunk of an fxg_seed_reads call
+ *                           sorts at a time (a seed with more gets a chunk of its own): bounds its device memory
  * None of them changes a result.  When the library is loaded it sets CUDA_DEVICE_MAX_CONNECTIONS=32 unless the variable is
  * already set (INTEGRATION.md, section 4). */
 int fxg_create(int device, fxg_ctx** out);
@@ -256,6 +261,39 @@ int fxg_seeder_create(size_t n_references, const uint8_t* const* rank_sequences,
 void fxg_seeder_free(fxg_seeder* seeder);
 int fxg_seeder_search(const fxg_seeder* seeder, const uint8_t* query, size_t query_len, const fxg_pex_node* leaves, size_t n_leaves,
                       uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors, fxg_anchor** anchors, size_t* n_anchors);
+
+/* ---- the same seeder on the device, for whole read batches ---- */
+typedef struct fxg_gpu_seeder fxg_gpu_seeder;
+typedef struct {
+    uint64_t seeds;              /* (read, strand, leaf) triples searched */
+    uint64_t candidates;         /* candidate starts before de-duplication */
+    uint64_t checked;            /* distinct candidate starts checked with the banded DP */
+    uint64_t hits;               /* raw anchors (distance <= leaf errors) */
+    uint64_t dropped_hard;       /* raw anchors of seeds removed by the hard cap */
+    uint64_t cut_soft;           /* raw anchors removed by the soft cap */
+    uint64_t erased;             /* anchors removed by erase_useless_anchors */
+    uint64_t reserved;
+} fxg_seed_stats;
+
+/* q-gram index (q = 4..14) of the references resident in ctx (fxg_set_references), built on the device from the packed
+ * store (no second copy of the references): 4^(q+1) bytes of buckets + 4 bytes per indexed position of device memory.
+ * FXG_ERR_INVALID_ARGUMENT for references of 2^32 bases or more (as fxg_seeder_create), FXG_ERR_STATE without references. */
+int  fxg_gpu_seeder_create(fxg_ctx* ctx, uint32_t q, fxg_gpu_seeder** out);
+void fxg_gpu_seeder_free(fxg_ctx* ctx, fxg_gpu_seeder* seeder);
+/* fxg_seeder_search for both orientations of every read of a batch.  `reads` is in/out: query_offset, query_len,
+ * node_offset, num_inner, num_leaves are read; anchor_offset, num_anchors_forward, num_anchors_reverse are written, so
+ * (reads, pools, nodes, *anchors) can be passed to fxg_verify_stage / fxg_verify_reads as they are.  Anchors: malloc'ed,
+ * release with fxg_free; per read the forward orientation's anchors, then the reverse complement's, each in
+ * seed -> reference -> position order, equal to what fxg_seeder_search returns for that orientation.  stats may be NULL.
+ * A leaf fxg_seeder_search refuses fails the whole call with FXG_ERR_INVALID_ARGUMENT before any device work;
+ * FXG_ERR_STATE once fxg_set_references has replaced the references the seeder was made from (and fxg_set_references
+ * fails with FXG_ERR_STATE while a seeding call runs).  Several threads may seed on one context at a time, beside
+ * verification runs: each call works on a stream of its own. */
+int  fxg_seed_reads(fxg_ctx* ctx, const fxg_gpu_seeder* seeder, fxg_read* reads, size_t n_reads,
+                    const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                    const fxg_pex_node* nodes, size_t n_nodes,
+                    uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                    fxg_anchor** anchors, size_t* n_anchors, fxg_seed_stats* stats);
 
 /* ---- accounting / measurement helpers ---- */
 int fxg_get_counters(const fxg_ctx* ctx, fxg_counters* out);
