@@ -1477,18 +1477,19 @@ void build_walks(fxg_ctx* c, fxg_job const* J, uint32_t read_lo, uint32_t read_h
 }
 
 int validate_reads_range(fxg_ctx* c, std::string& err, const fxg_read* reads, size_t lo, size_t hi, size_t pool_len,
-                         const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors);
+                         const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors, bool with_anchors);
 
-// every read's ranges, tree shape and anchors; large batches on several threads
+// every read's ranges, tree shape and anchors; large batches on several threads.  with_anchors = false: the reads' anchors
+// are not known yet (fxg_seed_verify_reads checks the batch before it seeds; the seeder's anchors are valid by construction)
 int validate_reads(fxg_ctx* c, std::string& err, const fxg_read* reads, size_t lo, size_t hi, size_t pool_len,
-                   const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors) {
+                   const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors, bool with_anchors = true) {
     size_t const n_threads = (n_nodes + n_anchors) < (size_t(1) << 20) ? 1 : std::min<size_t>({size_t(8), hi - lo, std::max<size_t>(1, std::thread::hardware_concurrency() / 2)});
-    if (n_threads <= 1) return validate_reads_range(c, err, reads, lo, hi, pool_len, nodes, n_nodes, anchors, n_anchors);
+    if (n_threads <= 1) return validate_reads_range(c, err, reads, lo, hi, pool_len, nodes, n_nodes, anchors, n_anchors, with_anchors);
     std::vector<int> rcs(n_threads, FXG_OK); std::vector<std::string> errs(n_threads);
     std::vector<std::thread> threads;
     for (size_t t = 0; t < n_threads; ++t) {
         size_t const a = lo + (hi - lo) * t / n_threads, b = lo + (hi - lo) * (t + 1) / n_threads;
-        threads.emplace_back([&, t, a, b] { rcs[t] = validate_reads_range(c, errs[t], reads, a, b, pool_len, nodes, n_nodes, anchors, n_anchors); });
+        threads.emplace_back([&, t, a, b] { rcs[t] = validate_reads_range(c, errs[t], reads, a, b, pool_len, nodes, n_nodes, anchors, n_anchors, with_anchors); });
     }
     for (auto& th : threads) th.join();
     for (size_t t = 0; t < n_threads; ++t) if (rcs[t] != FXG_OK) { err = errs[t]; tls_last_error = err; return rcs[t]; }
@@ -1496,13 +1497,13 @@ int validate_reads(fxg_ctx* c, std::string& err, const fxg_read* reads, size_t l
 }
 
 int validate_reads_range(fxg_ctx* c, std::string& err, const fxg_read* reads, size_t lo, size_t hi, size_t pool_len,
-                         const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors) {
+                         const fxg_pex_node* nodes, size_t n_nodes, const fxg_anchor* anchors, size_t n_anchors, bool with_anchors) {
     for (size_t i = lo; i < hi; ++i) {
         fxg_read const& R = reads[i];
         if (R.query_offset + R.query_len > pool_len) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: query outside the pool", i);
         if (R.query_len > FXG_MAX_QUERY_LENGTH) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: longer than %d", i, FXG_MAX_QUERY_LENGTH);
         if (R.node_offset + R.num_inner + R.num_leaves > n_nodes || R.num_leaves == 0) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad node range", i);
-        if (R.anchor_offset + R.num_anchors_forward + R.num_anchors_reverse > n_anchors) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad anchor range", i);
+        if (with_anchors && R.anchor_offset + R.num_anchors_forward + R.num_anchors_reverse > n_anchors) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad anchor range", i);
         const fxg_pex_node* nd = nodes + R.node_offset;
         for (uint32_t q = 0; q < R.num_inner + R.num_leaves; ++q) {
             if (nd[q].query_index_to < nd[q].query_index_from || nd[q].query_index_to >= R.query_len) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: node %u outside the query", i, q);
@@ -1526,6 +1527,7 @@ int validate_reads_range(fxg_ctx* c, std::string& err, const fxg_read* reads, si
                 for (uint64_t x = q; depth[x] == 0xff; x = nd[x].parent_id) depth[x] = uint8_t(d--);
             }
         }
+        if (!with_anchors) continue;
         const fxg_anchor* an = anchors + R.anchor_offset;
         for (uint32_t q = 0; q < R.num_anchors_forward + R.num_anchors_reverse; ++q) {
             if (an[q].pex_leaf_index >= R.num_leaves) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: anchor %u names leaf %llu", i, q, (unsigned long long)an[q].pex_leaf_index);
@@ -1627,9 +1629,21 @@ std::vector<ConfigCacheEntry>& thread_config_cache(const fxg_ctx* c) {
     return cache;
 }
 
+// Where a job's records go in Prepared::dev and its staging: nodes | leaves | reads | anchors, each on a 256-byte boundary.
+// Returns the end of the anchors.
+size_t carve_records(Prepared& P, uint64_t n_nodes, uint64_t n_leaves, uint64_t n_reads, uint64_t n_walks) {
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { size_t const at = off; off += (bytes + 255) & ~size_t(255); return at; };
+    P.o_nodes = carve(n_nodes * sizeof(NodeRec)); P.o_leaves = carve(n_leaves * sizeof(LeafRec));
+    P.o_reads = carve(n_reads * sizeof(ReadRec)); P.o_anchors = carve(n_walks * sizeof(AnchorRec16));
+    return off;
+}
+
 // Builds and uploads the job's records (asynchronously, on the context's staging stream; J->prep.ready marks the end).
 // J->prep.ok tells whether the device-side walk can take the job; if not, the host-driven levels run it.
-int prepare_job(fxg_ctx* c, fxg_job* J, std::string& err, fxg_counters& ctr) {
+// anchors_on_device: the AnchorRec16 records are already in P.dev at P.o_anchors (fxg_seed_verify_reads wrote them there,
+// on a stream its caller has drained); only the nodes, leaves and reads are built and go up.
+int prepare_job(fxg_ctx* c, fxg_job* J, std::string& err, fxg_counters& ctr, bool anchors_on_device = false) {
     Prepared& P = J->prep;
     P.ok = false;
     size_t const n_reads = J->n_reads;
@@ -1643,13 +1657,12 @@ int prepare_job(fxg_ctx* c, fxg_job* J, std::string& err, fxg_counters& ctr) {
     if (n_walks == 0 || n_walks >= kMaxDeviceWalks || n_nodes >= (1u << 30) || n_leaves >= (1u << 30) || n_reads >= (1u << 30)) return FXG_OK;
     if (c->refs.total >= (uint64_t(1) << (64 - kWalkBits))) return FXG_OK;
     static_assert(sizeof(AnchorRec16) == 16 && sizeof(ReadRec) == 64 && sizeof(LeafRec) == 8 && sizeof(NodeRec) == 16 && sizeof(WalkRec) == 32 && sizeof(RootEntry) == 16, "record layouts");
-    size_t off = 0;
-    auto carve = [&](size_t bytes) { size_t const at = off; off += (bytes + 255) & ~size_t(255); return at; };
-    P.o_nodes = carve(n_nodes * sizeof(NodeRec)); P.o_leaves = carve(n_leaves * sizeof(LeafRec));
-    P.o_reads = carve(n_reads * sizeof(ReadRec)); P.o_anchors = carve(n_walks * sizeof(AnchorRec16));
+    size_t const off = carve_records(P, n_nodes, n_leaves, n_reads, n_walks);
+    size_t const up = anchors_on_device ? P.o_anchors : off;          // what goes up from the host
     P.staging.tag = "page-locked job records";
-    if (P.staging.ensure(off + 64) != cudaSuccess) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate staging for the job's records");
-    P.used = off;
+    if (P.staging.ensure(up + 64) != cudaSuccess) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate staging for the job's records");
+    P.used = up;
+    if (anchors_on_device && P.dev.cap < off + 64) return fail(err, FXG_ERR_CUDA, "internal: the seeded anchors do not fit the job's record buffer");
     CUDA_TRY(err, P.dev.ensure(off + 64));
     uint8_t* const H = P.staging.as<uint8_t>();
     NodeRec* const nrec = reinterpret_cast<NodeRec*>(H + P.o_nodes);
@@ -1747,6 +1760,7 @@ int prepare_job(fxg_ctx* c, fxg_job* J, std::string& err, fxg_counters& ctr) {
                     lrec[rr.leaf_base + q].parent = leaves[q].parent_id == FXG_NULL_ID ? kNoParent : uint32_t(leaves[q].parent_id);
                 }
             }
+            if (anchors_on_device) continue;
             const fxg_anchor* an = J->anchors_p + R.anchor_offset;
             AnchorRec16* const dst = arec + rr.walk_begin;
             for (uint32_t q = 0; q < rr.n_walks; ++q) {
@@ -1775,9 +1789,9 @@ int prepare_job(fxg_ctx* c, fxg_job* J, std::string& err, fxg_counters& ctr) {
     P.n_nodes = node_at; P.n_leaves = leaf_at; P.n_walks = walk_at; P.n_reads = uint32_t(n_reads);
     P.hreads.assign(rrec, rrec + n_reads);
     if (!P.ready) CUDA_TRY(err, cudaEventCreateWithFlags(&P.ready, cudaEventDisableTiming));
-    CUDA_TRY(err, cudaMemcpyAsync(P.dev.p, H, off, cudaMemcpyHostToDevice, c->stage_stream));
+    CUDA_TRY(err, cudaMemcpyAsync(P.dev.p, H, up, cudaMemcpyHostToDevice, c->stage_stream));
     CUDA_TRY(err, cudaEventRecord(P.ready, c->stage_stream));
-    ctr.h2d_bytes += off;
+    ctr.h2d_bytes += up;
     P.ok = true;
     return FXG_OK;
 }
@@ -3366,6 +3380,63 @@ void release_job_buffers(fxg_ctx* c, fxg_job* j) {        // call with c->mu hel
     j->prep.dev = DevBuf{};
 }
 
+// A job of fxg_verify_reads / fxg_seed_verify_reads: it reads the caller's arrays in place during the one call that runs it.
+// Call with c->mu held.
+fxg_job* new_borrowed_job(fxg_ctx* c, const fxg_verify_config* cfg, const fxg_read* reads, size_t n_reads, const fxg_pex_node* nodes,
+                          size_t n_nodes, size_t pool_len) {
+    fxg_job* j = new (std::nothrow) fxg_job();
+    if (!j) return nullptr;
+    j->cfg = *cfg;
+    j->reads_p = reads; j->nodes_p = nodes;
+    j->n_reads = n_reads; j->n_nodes = n_nodes;
+    j->borrowed = true;
+    j->pool_len = pool_len;
+    j->pool = take_pool(c);
+    j->prep.staging = take_staging(c);
+    if (!c->spare_dev.empty()) { j->prep.dev = c->spare_dev.back(); c->spare_dev.pop_back(); }
+    return j;
+}
+
+// The rest of a borrowed job's call once its pools and records are enqueued (rc: how that went): the queue, the check of
+// the pools' ranks, and the job handed to the caller -- or released.
+int run_borrowed_job(fxg_ctx* c, fxg_job* j, int rc, std::string& err, fxg_counters const& ctr, fxg_job** out) {
+    std::unique_lock<std::mutex> lock(c->mu);
+    add_counters(c->ctr, ctr);
+    if (rc == FXG_OK) {
+        rc = submit_and_wait(c, j, lock);
+        if (rc != FXG_OK) err = c->err;
+    }
+    lock.unlock();
+    if (rc == FXG_OK) {
+        // (waits on an event of its own, asleep: cudaStreamSynchronize would spin -- one core per caller -- until every other
+        //  caller's uploads on the staging stream are through as well)
+        uint32_t bad_pageable = 0;
+        // (into page-locked memory where the job has some: a copy into pageable memory blocks, spinning, as well)
+        uint32_t* const bad_p = j->prep.staging.p && j->prep.used ? reinterpret_cast<uint32_t*>(j->prep.staging.as<uint8_t>() + j->prep.used) : &bad_pageable;
+        if (cudaMemcpyAsync(bad_p, j->pool.bad_rank.p, 4, cudaMemcpyDeviceToHost, c->stage_stream) != cudaSuccess ||
+            cudaEventRecord(j->pool_ready, c->stage_stream) != cudaSuccess ||
+            cudaEventSynchronize(j->pool_ready) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "staging failed");
+        uint32_t const bad = *bad_p;
+        if (rc != FXG_OK) {}
+        else if (bad) rc = fail(err, FXG_ERR_INVALID_ARGUMENT, "query pools contain a rank above %d (allowed 0..%d)", FXG_MAX_RANK, FXG_MAX_RANK);
+    } else {
+        cudaStreamSynchronize(c->stage_stream);          // nothing may still read the caller's arrays when the call returns
+    }
+    // the caller's arrays are not looked at after this point
+    j->reads_p = nullptr; j->nodes_p = nullptr; j->anchors_p = nullptr;
+    lock.lock();
+    if (rc != FXG_OK) {
+        c->err = err; tls_last_error = err;
+        release_job_buffers(c, j);
+        if (j->prep.ready) cudaEventDestroy(j->prep.ready);
+        if (j->pool_ready) cudaEventDestroy(j->pool_ready);
+        delete j;
+        return rc;
+    }
+    *out = j;
+    return FXG_OK;
+}
+
 }  // namespace
 
 int fxg_verify_stage(fxg_ctx* c, const fxg_verify_config* cfg, const fxg_read* reads, size_t n_reads,
@@ -3442,16 +3513,9 @@ int fxg_verify_reads(fxg_ctx* c, const fxg_verify_config* cfg, const fxg_read* r
     int rc = check_verify_call(c, cfg);
     if (rc != FXG_OK) return rc;
     CUDA_TRY(c->err, cudaSetDevice(c->device));
-    fxg_job* j = new (std::nothrow) fxg_job();
+    fxg_job* j = new_borrowed_job(c, cfg, reads, n_reads, nodes, n_nodes, pool_len);
     if (!j) return FXG_ERR_OUT_OF_MEMORY;
-    j->cfg = *cfg;
-    j->reads_p = reads; j->nodes_p = nodes; j->anchors_p = anchors;
-    j->n_reads = n_reads; j->n_nodes = n_nodes; j->n_anchors = n_anchors;
-    j->borrowed = true;
-    j->pool_len = pool_len;
-    j->pool = take_pool(c);
-    j->prep.staging = take_staging(c);
-    if (!c->spare_dev.empty()) { j->prep.dev = c->spare_dev.back(); c->spare_dev.pop_back(); }
+    j->anchors_p = anchors; j->n_anchors = n_anchors;
     lock.unlock();
     std::string err; fxg_counters ctr{};
     auto const tp0 = std::chrono::steady_clock::now();
@@ -3469,42 +3533,9 @@ int fxg_verify_reads(fxg_ctx* c, const fxg_verify_config* cfg, const fxg_read* r
     double const t_stage = lap_ms();
     if (rc == FXG_OK) rc = prepare_job(c, j, err, ctr);
     double const t_prepare = lap_ms();
-    lock.lock();
-    add_counters(c->ctr, ctr);
-    if (rc == FXG_OK) {
-        rc = submit_and_wait(c, j, lock);
-        if (rc != FXG_OK) err = c->err;
-    }
-    lock.unlock();
+    rc = run_borrowed_job(c, j, rc, err, ctr, out);
     if (g_prof.on) fprintf(stderr, "[fxg] verify_reads: validated %.3f, pools enqueued %.3f, records prepared %.3f, run done %.3f ms\n", t_validate, t_stage, t_prepare, lap_ms());
-    if (rc == FXG_OK) {
-        // (waits on an event of its own, asleep: cudaStreamSynchronize would spin -- one core per caller -- until every other
-        //  caller's uploads on the staging stream are through as well)
-        uint32_t bad_pageable = 0;
-        // (into page-locked memory where the job has some: a copy into pageable memory blocks, spinning, as well)
-        uint32_t* const bad_p = j->prep.staging.p && j->prep.used ? reinterpret_cast<uint32_t*>(j->prep.staging.as<uint8_t>() + j->prep.used) : &bad_pageable;
-        if (cudaMemcpyAsync(bad_p, j->pool.bad_rank.p, 4, cudaMemcpyDeviceToHost, c->stage_stream) != cudaSuccess ||
-            cudaEventRecord(j->pool_ready, c->stage_stream) != cudaSuccess ||
-            cudaEventSynchronize(j->pool_ready) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "staging failed");
-        uint32_t const bad = *bad_p;
-        if (rc != FXG_OK) {}
-        else if (bad) rc = fail(err, FXG_ERR_INVALID_ARGUMENT, "query pools contain a rank above %d (allowed 0..%d)", FXG_MAX_RANK, FXG_MAX_RANK);
-    } else {
-        cudaStreamSynchronize(c->stage_stream);          // nothing may still read the caller's arrays when the call returns
-    }
-    // the caller's arrays are not looked at after this point
-    j->reads_p = nullptr; j->nodes_p = nullptr; j->anchors_p = nullptr;
-    lock.lock();
-    if (rc != FXG_OK) {
-        c->err = err; tls_last_error = err;
-        release_job_buffers(c, j);
-        if (j->prep.ready) cudaEventDestroy(j->prep.ready);
-        if (j->pool_ready) cudaEventDestroy(j->pool_ready);
-        delete j;
-        return rc;
-    }
-    *out = j;
-    return FXG_OK;
+    return rc;
 }
 
 // ------------------------------------------------------------------------------------------------ engine shape
@@ -3614,6 +3645,251 @@ int take_store(fxg_ctx* c, const fxg_gpu_seeder* S, StoreReader& guard, const ui
     return FXG_OK;
 }
 
+// The seeds of a batch, from the reads and their trees, on the host: a read or leaf fxg_seeder_search refuses fails the
+// whole call before any device work.
+struct SeedPlan {
+    std::vector<uint32_t> seed_base, leaf_base;     // per read (+1): first seed, first leaf
+    std::vector<uint64_t> leaf_info;                // per (read, leaf): seed_pack(query_offset + from, m, e)
+    uint32_t n_seeds = 0;
+};
+
+int plan_seeds(const fxg_gpu_seeder* S, const fxg_read* reads, size_t n_reads, size_t pool_len, const fxg_pex_node* nodes, size_t n_nodes,
+               SeedPlan& plan, std::string& err) {
+    if (pool_len >= (uint64_t(1) << 38)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "query pools of %zu bytes: at most 2^38", pool_len);
+    std::vector<uint32_t>& seed_base = plan.seed_base;
+    std::vector<uint32_t>& leaf_base = plan.leaf_base;
+    seed_base.resize(n_reads + 1); leaf_base.resize(n_reads + 1);
+    uint64_t n_leaves = 0;
+    for (size_t i = 0; i < n_reads; ++i) {
+        fxg_read const& R = reads[i];
+        if (R.query_offset > pool_len || R.query_len > pool_len - R.query_offset) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: query outside the pool", i);
+        if (R.query_len > FXG_MAX_QUERY_LENGTH) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: longer than %d", i, FXG_MAX_QUERY_LENGTH);
+        if (R.node_offset > n_nodes || uint64_t(R.num_inner) + R.num_leaves > n_nodes - R.node_offset)
+            return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad node range", i);
+        leaf_base[i] = uint32_t(n_leaves);
+        seed_base[i] = uint32_t(2 * n_leaves);
+        n_leaves += R.num_leaves;
+        if (2 * n_leaves >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "more than 2^30 leaves in one call");
+    }
+    leaf_base[n_reads] = uint32_t(n_leaves);
+    seed_base[n_reads] = uint32_t(2 * n_leaves);
+    plan.leaf_info.resize(n_leaves);
+    for (size_t i = 0; i < n_reads; ++i) {
+        fxg_read const& R = reads[i];
+        const fxg_pex_node* lv = nodes + R.node_offset + R.num_inner;
+        for (uint32_t li = 0; li < R.num_leaves; ++li) {
+            fxg_pex_node const& leaf = lv[li];
+            if (leaf.query_index_to < leaf.query_index_from || leaf.query_index_to >= R.query_len)
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: outside the query", i, li);
+            uint32_t const m = uint32_t(leaf.query_index_to - leaf.query_index_from + 1), e = uint32_t(leaf.num_errors);
+            if (e > uint32_t(kSeedMaxErrors) || m / (e + 1) < S->q)
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: %u bases with %u errors (at most %d errors and q * (errors + 1) = %u bases)",
+                            i, li, m, e, kSeedMaxErrors, S->q * (e + 1));
+            plan.leaf_info[leaf_base[i] + li] = seed_pack(R.query_offset + leaf.query_index_from, m, e);
+        }
+    }
+    plan.n_seeds = uint32_t(2 * n_leaves);
+    return FXG_OK;
+}
+
+// Where seed_batch delivers the surviving anchors: a malloc'ed fxg_anchor array (fxg_seed_reads), or -- `dev` set -- a
+// verification job's AnchorRec16 records at dev + dev_offset (fxg_seed_verify_reads), in the same order either way.
+struct SeedSink {
+    DevBuf* dev = nullptr; size_t dev_offset = 0;
+    fxg_anchor* host = nullptr;                     // (host) owned by the caller, also when the call fails
+    size_t n = 0;                                   // anchors delivered
+    std::vector<uint32_t> per_read;                 // per (read, orientation)
+    uint64_t h2d_bytes = 0, d2h_bytes = 0;          // what the call copied, besides the query pools
+};
+
+// the reads' anchor ranges as the seeder laid the anchors out
+void set_read_anchors(fxg_read* reads, size_t n_reads, std::vector<uint32_t> const& per_read) {
+    uint64_t at = 0;
+    for (size_t i = 0; i < n_reads; ++i) {
+        reads[i].anchor_offset = at;
+        reads[i].num_anchors_forward = per_read.empty() ? 0 : per_read[2 * i];
+        reads[i].num_anchors_reverse = per_read.empty() ? 0 : per_read[2 * i + 1];
+        at += uint64_t(reads[i].num_anchors_forward) + reads[i].num_anchors_reverse;
+    }
+}
+
+// The device seeder on a planned batch (plan.n_seeds > 0) whose query pools -- forward, then reverse complement -- are at
+// d_pool on the device, on K's stream (which first waits for `pool_ready`, if given).  Returns with the stream drained.
+int seed_batch(fxg_ctx* c, const fxg_gpu_seeder* S, const uint32_t* packed, SeedPlan const& plan, size_t n_reads, SeedCall& K,
+               const uint8_t* d_pool, uint64_t pool_len, cudaEvent_t pool_ready, uint64_t max_anchors_hard, uint64_t max_anchors_soft,
+               int erase_useless_anchors, SeedSink& out, fxg_seed_stats& st, std::string& err) {
+    uint32_t const n_seeds = plan.n_seeds;
+    uint64_t const n_leaves = plan.leaf_info.size();
+    { std::lock_guard<std::mutex> lock(c->mu); if (!K.host.p) K.host = take_staging(c); }
+    DevBuf &d_seed_base = K.bufs[1], &d_leaf_base = K.bufs[2], &d_leaves = K.bufs[3], &d_info = K.bufs[4],
+           &d_occ = K.bufs[5], &d_off = K.bufs[6], &d_ctr = K.bufs[7], &d_per_read = K.bufs[8], &d_keys = K.bufs[9], &d_sorted = K.bufs[10],
+           &d_uniq = K.bufs[11], &d_nuniq = K.bufs[12], &d_hits = K.bufs[13], &d_hits2 = K.bufs[14], &d_gone = K.bufs[15], &d_at = K.bufs[16],
+           &d_out = K.bufs[17], &d_tmp = K.bufs[18];
+    cudaStream_t const s = K.st;
+    if (pool_ready) CUDA_TRY(err, cudaStreamWaitEvent(s, pool_ready, 0));
+
+    // ---- uploads and the seeds' plan ----
+    CUDA_TRY(err, d_seed_base.ensure((n_reads + 1) * 4));
+    CUDA_TRY(err, d_leaf_base.ensure((n_reads + 1) * 4));
+    CUDA_TRY(err, d_leaves.ensure(n_leaves * 8));
+    CUDA_TRY(err, cudaMemcpyAsync(d_seed_base.p, plan.seed_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(err, cudaMemcpyAsync(d_leaf_base.p, plan.leaf_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(err, cudaMemcpyAsync(d_leaves.p, plan.leaf_info.data(), n_leaves * 8, cudaMemcpyHostToDevice, s));
+    out.h2d_bytes += (n_reads + 1) * 8 + n_leaves * 8;
+    CUDA_TRY(err, d_info.ensure(size_t(n_seeds) * 8));
+    CUDA_TRY(err, d_occ.ensure(size_t(n_seeds) * 8));
+    CUDA_TRY(err, d_off.ensure((size_t(n_seeds) + 1) * 8));
+    CUDA_TRY(err, d_ctr.ensure(8 * 8));
+    CUDA_TRY(err, d_per_read.ensure(n_reads * 8));
+    CUDA_TRY(err, cudaMemsetAsync(d_per_read.p, 0, n_reads * 8, s));
+    CUDA_TRY(err, cudaMemsetAsync(d_off.p, 0, 8, s));
+    SeedRefs const R = seed_refs(S, packed);
+    SeedBatch const B{d_pool, pool_len, d_seed_base.as<uint32_t>(), d_leaf_base.as<uint32_t>(), d_leaves.as<uint64_t>(),
+                      uint32_t(n_reads), n_seeds, S->bucket.as<uint32_t>(), S->pos.as<uint32_t>(), S->q};
+    seed_plan_kernel<<<seed_grid(n_seeds), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_occ.as<uint64_t>());
+    CUDA_TRY(err, cudaGetLastError());
+    size_t tmp_bytes = 0;
+    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
+    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(d_tmp.p, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
+    CUDA_TRY(err, K.host.ensure(std::max<size_t>(4096, n_reads * 8)));
+    uint64_t* h_ctr = K.host.as<uint64_t>();             // (moves when the buffer grows)
+    CUDA_TRY(err, cudaMemcpyAsync(h_ctr, d_off.as<uint64_t>() + n_seeds, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    out.d2h_bytes += 8;
+    uint64_t const total_occ = h_ctr[0];
+
+    // ---- chunks of whole seeds under the budget of q-gram occurrences (a seed above it gets a chunk of its own) ----
+    std::vector<uint64_t> off;                     // host copy of the offsets, only when the batch needs several chunks
+    if (total_occ > S->budget || n_seeds > kSeedChunkSeeds) {
+        off.resize(size_t(n_seeds) + 1);
+        CUDA_TRY(err, cudaMemcpyAsync(off.data(), d_off.p, off.size() * 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        out.d2h_bytes += off.size() * 8;
+    }
+    auto off_at = [&](uint32_t i) { return off.empty() ? (i == 0 ? 0 : total_occ) : off[i]; };
+    for (uint32_t s0 = 0; s0 < n_seeds;) {
+        uint32_t s1 = n_seeds;
+        if (!off.empty()) {
+            s1 = uint32_t(std::upper_bound(off.begin() + s0 + 1, off.end(), off[s0] + S->budget) - off.begin()) - 1;
+            s1 = std::min(std::max(s1, s0 + 1), std::min(n_seeds, s0 + kSeedChunkSeeds));
+        }
+        uint64_t const N = off_at(s1) - off_at(s0);
+        uint32_t const ns = s1 - s0;
+        if (N == 0) { s0 = s1; continue; }
+        if (N >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "seeds %u..%u have %llu q-gram occurrences: build the index with a larger q",
+                                                  s0, s1 - 1, (unsigned long long)N);
+        int const n_items = int(N);
+        // candidates: (seed, nominal start) keys, sorted and made unique
+        CUDA_TRY(err, d_keys.ensure(N * 8));
+        CUDA_TRY(err, d_sorted.ensure(N * 8));
+        CUDA_TRY(err, d_uniq.ensure(N * 8));
+        CUDA_TRY(err, d_nuniq.ensure(8));
+        CUDA_TRY(err, cudaMemsetAsync(d_ctr.p, 0, 64, s));
+        unsigned long long* const ctr = d_ctr.as<unsigned long long>();
+        seed_emit_kernel<<<seed_grid(ns), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_off.as<uint64_t>(), s0, s1, d_keys.as<uint64_t>(), ctr);
+        CUDA_TRY(err, cudaGetLastError());
+        int const key_bits = std::min(64, kSeedKeyShift + bits_for(ns - 1));
+        size_t sort_bytes = 0, uniq_bytes = 0;
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
+        CUDA_TRY(err, cub::DeviceSelect::Unique(nullptr, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
+        CUDA_TRY(err, d_tmp.ensure(std::max(sort_bytes, uniq_bytes)));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
+        CUDA_TRY(err, cub::DeviceSelect::Unique(d_tmp.p, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
+        // check every distinct start; the hit buffer grows and the check runs again if it was too small
+        uint64_t hit_cap = std::max<uint64_t>(d_hits.cap / 8, N + 1024);
+        uint64_t n_hits = 0;
+        for (;;) {
+            CUDA_TRY(err, d_hits.ensure(hit_cap * 8));
+            seed_check_kernel<<<seed_grid(N), 256, 0, s>>>(R, B, d_info.as<uint64_t>(), s0, d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(),
+                                                           d_hits.as<uint64_t>(), hit_cap, ctr);
+            CUDA_TRY(err, cudaGetLastError());
+            CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(err, cudaStreamSynchronize(s));
+            out.d2h_bytes += 64;
+            n_hits = h_ctr[2];
+            if (n_hits <= hit_cap) break;
+            hit_cap = n_hits;
+            CUDA_TRY(err, cudaMemsetAsync(ctr + 1, 0, 16, s));
+        }
+        st.candidates += h_ctr[0]; st.checked += h_ctr[1]; st.hits += n_hits;
+        if (n_hits == 0) { s0 = s1; continue; }
+        // caps on hits ordered by (seed, errors, position), then the kept ones by (seed, position)
+        int const hit_items = int(n_hits);
+        CUDA_TRY(err, d_hits2.ensure(n_hits * 8));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
+        CUDA_TRY(err, d_tmp.ensure(sort_bytes));
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0,
+                                                     std::min(64, kHitKeyShift + bits_for(ns - 1)), s));
+        seed_caps_kernel<<<seed_grid(n_hits), 256, 0, s>>>(d_hits2.as<uint64_t>(), n_hits, max_anchors_hard, max_anchors_soft, d_hits.as<uint64_t>(), ctr);
+        CUDA_TRY(err, cudaGetLastError());
+        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        out.d2h_bytes += 64;
+        st.dropped_hard += h_ctr[3]; st.cut_soft += h_ctr[4];
+        uint64_t const n_kept = n_hits - h_ctr[3] - h_ctr[4];
+        if (n_kept == 0) { s0 = s1; continue; }
+        // erase_useless_anchors, then the survivors in order
+        CUDA_TRY(err, d_gone.ensure(n_kept * 4));
+        CUDA_TRY(err, d_at.ensure(n_kept * 4));
+        CUDA_TRY(err, cudaMemsetAsync(d_gone.p, 0, n_kept * 4, s));
+        if (erase_useless_anchors) {
+            seed_erase_kernel<<<seed_grid(n_kept), 256, 0, s>>>(R, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>());
+            CUDA_TRY(err, cudaGetLastError());
+        }
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
+        CUDA_TRY(err, d_tmp.ensure(tmp_bytes));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
+        uint64_t n_out = 0;
+        if (out.dev) {
+            // straight into the job's record buffer, behind the records of the earlier chunks (room for every kept anchor and
+            // for the 256-byte rounding of prepare_job's layout; a growing buffer keeps what the earlier chunks wrote)
+            size_t const done = out.dev_offset + out.n * sizeof(AnchorRec16);
+            size_t const need = out.dev_offset + ((out.n + n_kept) * sizeof(AnchorRec16) + 255) / 256 * 256 + 64;
+            CUDA_TRY(err, out.n ? out.dev->ensure_preserving(need, done, s) : out.dev->ensure(need));
+            seed_output_kernel<true><<<seed_grid(n_kept), 256, 0, s>>>(R, B, s0, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>(), d_at.as<uint32_t>(),
+                                                                       out.dev->as<uint8_t>() + done, d_per_read.as<uint32_t>(), ctr);
+            CUDA_TRY(err, cudaGetLastError());
+            CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(err, cudaStreamSynchronize(s));
+            out.d2h_bytes += 64;
+            n_out = n_kept - h_ctr[5];
+        } else {
+            CUDA_TRY(err, d_out.ensure(n_kept * sizeof(fxg_anchor)));
+            seed_output_kernel<false><<<seed_grid(n_kept), 256, 0, s>>>(R, B, s0, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>(), d_at.as<uint32_t>(),
+                                                                        d_out.p, d_per_read.as<uint32_t>(), ctr);
+            CUDA_TRY(err, cudaGetLastError());
+            // back through page-locked memory: the counters, then up to n_kept records
+            CUDA_TRY(err, K.host.ensure(64 + n_kept * sizeof(fxg_anchor)));
+            uint64_t* const h = h_ctr = K.host.as<uint64_t>();
+            CUDA_TRY(err, cudaMemcpyAsync(h, ctr, 64, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(err, cudaMemcpyAsync(h + 8, d_out.p, n_kept * sizeof(fxg_anchor), cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(err, cudaStreamSynchronize(s));
+            out.d2h_bytes += 64 + n_kept * sizeof(fxg_anchor);
+            n_out = n_kept - h[5];
+            if (n_out) {
+                fxg_anchor* grown = static_cast<fxg_anchor*>(std::realloc(out.host, (out.n + n_out) * sizeof(fxg_anchor)));
+                if (!grown) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate %llu anchors", (unsigned long long)(out.n + n_out));
+                out.host = grown;
+                std::memcpy(out.host + out.n, h + 8, n_out * sizeof(fxg_anchor));
+            }
+        }
+        st.erased += h_ctr[5];
+        out.n += n_out;
+        s0 = s1;
+    }
+    out.per_read.resize(2 * n_reads);
+    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_per_read.p, n_reads * 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    out.d2h_bytes += n_reads * 8;
+    std::memcpy(out.per_read.data(), K.host.p, n_reads * 8);
+    uint64_t sum = 0;
+    for (uint32_t v : out.per_read) sum += v;
+    if (sum != out.n) return fail(err, FXG_ERR_CUDA, "internal: %llu anchors counted per read, %zu written", (unsigned long long)sum, out.n);
+    return FXG_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -3696,214 +3972,104 @@ int fxg_seed_reads(fxg_ctx* c, const fxg_gpu_seeder* S, fxg_read* reads, size_t 
     if (!c || !S || !anchors || !n_anchors || (n_reads && !reads) || (pool_len && (!forward_pool || !reverse_complement_pool)) || (n_nodes && !nodes))
         return FXG_ERR_INVALID_ARGUMENT;
     *anchors = nullptr; *n_anchors = 0;
-    fxg_seed_stats st{};
     std::string err;
-    // ---- every read and leaf on the host, before any launch: what fxg_seeder_search refuses fails the whole call ----
-    if (pool_len >= (uint64_t(1) << 38)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "query pools of %zu bytes: at most 2^38", pool_len);
-    std::vector<uint32_t> seed_base(n_reads + 1), leaf_base(n_reads + 1);
-    uint64_t n_leaves = 0;
-    for (size_t i = 0; i < n_reads; ++i) {
-        fxg_read const& R = reads[i];
-        if (R.query_offset > pool_len || R.query_len > pool_len - R.query_offset) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: query outside the pool", i);
-        if (R.query_len > FXG_MAX_QUERY_LENGTH) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: longer than %d", i, FXG_MAX_QUERY_LENGTH);
-        if (R.node_offset > n_nodes || uint64_t(R.num_inner) + R.num_leaves > n_nodes - R.node_offset)
-            return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: bad node range", i);
-        leaf_base[i] = uint32_t(n_leaves);
-        seed_base[i] = uint32_t(2 * n_leaves);
-        n_leaves += R.num_leaves;
-        if (2 * n_leaves >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "more than 2^30 leaves in one call");
-    }
-    leaf_base[n_reads] = uint32_t(n_leaves);
-    seed_base[n_reads] = uint32_t(2 * n_leaves);
-    std::vector<uint64_t> leaf_info(n_leaves);
-    for (size_t i = 0; i < n_reads; ++i) {
-        fxg_read const& R = reads[i];
-        const fxg_pex_node* lv = nodes + R.node_offset + R.num_inner;
-        for (uint32_t li = 0; li < R.num_leaves; ++li) {
-            fxg_pex_node const& leaf = lv[li];
-            if (leaf.query_index_to < leaf.query_index_from || leaf.query_index_to >= R.query_len)
-                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: outside the query", i, li);
-            uint32_t const m = uint32_t(leaf.query_index_to - leaf.query_index_from + 1), e = uint32_t(leaf.num_errors);
-            if (e > uint32_t(kSeedMaxErrors) || m / (e + 1) < S->q)
-                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu, leaf %u: %u bases with %u errors (at most %d errors and q * (errors + 1) = %u bases)",
-                            i, li, m, e, kSeedMaxErrors, S->q * (e + 1));
-            leaf_info[leaf_base[i] + li] = seed_pack(R.query_offset + leaf.query_index_from, m, e);
-        }
-    }
-    uint32_t const n_seeds = uint32_t(2 * n_leaves);
-    st.seeds = n_seeds;
-    auto finish = [&](std::vector<uint32_t> const& per_read) {
-        uint64_t at = 0;
-        for (size_t i = 0; i < n_reads; ++i) {
-            reads[i].anchor_offset = at;
-            reads[i].num_anchors_forward = per_read.empty() ? 0 : per_read[2 * i];
-            reads[i].num_anchors_reverse = per_read.empty() ? 0 : per_read[2 * i + 1];
-            at += uint64_t(reads[i].num_anchors_forward) + reads[i].num_anchors_reverse;
-        }
-        if (stats) *stats = st;
-        return FXG_OK;
-    };
+    SeedPlan plan;
+    if (int rc = plan_seeds(S, reads, n_reads, pool_len, nodes, n_nodes, plan, err)) return rc;
+    fxg_seed_stats st{};
+    st.seeds = plan.n_seeds;
     StoreReader guard{c};
     const uint32_t* packed = nullptr;
     if (int rc = take_store(c, S, guard, packed, nullptr, nullptr, nullptr, err)) return rc;
-    if (n_seeds == 0) return finish({});
-    CUDA_TRY(err, cudaSetDevice(c->device));
+    SeedSink sink;
+    if (plan.n_seeds) {
+        CUDA_TRY(err, cudaSetDevice(c->device));
+        SeedCall K{c};
+        CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+        DevBuf& d_pool = K.bufs[0];
+        CUDA_TRY(err, d_pool.ensure(2 * pool_len + 64));
+        if (pool_len) {
+            CUDA_TRY(err, cudaMemcpyAsync(d_pool.p, forward_pool, pool_len, cudaMemcpyHostToDevice, K.st));
+            CUDA_TRY(err, cudaMemcpyAsync(d_pool.as<uint8_t>() + pool_len, reverse_complement_pool, pool_len, cudaMemcpyHostToDevice, K.st));
+        }
+        int const rc = seed_batch(c, S, packed, plan, n_reads, K, d_pool.as<uint8_t>(), pool_len, nullptr, max_anchors_hard, max_anchors_soft,
+                                  erase_useless_anchors, sink, st, err);
+        if (rc != FXG_OK) { std::free(sink.host); return rc; }
+    }
+    set_read_anchors(reads, n_reads, sink.per_read);
+    if (stats) *stats = st;
+    *anchors = sink.host; *n_anchors = sink.n;
+    return FXG_OK;
+}
 
-    // ---- uploads and the seeds' plan ----
-    SeedCall K{c};
-    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
-    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
-    DevBuf &d_pool = K.bufs[0], &d_seed_base = K.bufs[1], &d_leaf_base = K.bufs[2], &d_leaves = K.bufs[3], &d_info = K.bufs[4],
-           &d_occ = K.bufs[5], &d_off = K.bufs[6], &d_ctr = K.bufs[7], &d_per_read = K.bufs[8], &d_keys = K.bufs[9], &d_sorted = K.bufs[10],
-           &d_uniq = K.bufs[11], &d_nuniq = K.bufs[12], &d_hits = K.bufs[13], &d_hits2 = K.bufs[14], &d_gone = K.bufs[15], &d_at = K.bufs[16],
-           &d_out = K.bufs[17], &d_tmp = K.bufs[18];
-    cudaStream_t const s = K.st;
-    CUDA_TRY(err, d_pool.ensure(2 * pool_len + 64));
-    if (pool_len) {
-        CUDA_TRY(err, cudaMemcpyAsync(d_pool.p, forward_pool, pool_len, cudaMemcpyHostToDevice, s));
-        CUDA_TRY(err, cudaMemcpyAsync(d_pool.as<uint8_t>() + pool_len, reverse_complement_pool, pool_len, cudaMemcpyHostToDevice, s));
-    }
-    CUDA_TRY(err, d_seed_base.ensure((n_reads + 1) * 4));
-    CUDA_TRY(err, d_leaf_base.ensure((n_reads + 1) * 4));
-    CUDA_TRY(err, d_leaves.ensure(n_leaves * 8));
-    CUDA_TRY(err, cudaMemcpyAsync(d_seed_base.p, seed_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(err, cudaMemcpyAsync(d_leaf_base.p, leaf_base.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(err, cudaMemcpyAsync(d_leaves.p, leaf_info.data(), n_leaves * 8, cudaMemcpyHostToDevice, s));
-    CUDA_TRY(err, d_info.ensure(size_t(n_seeds) * 8));
-    CUDA_TRY(err, d_occ.ensure(size_t(n_seeds) * 8));
-    CUDA_TRY(err, d_off.ensure((size_t(n_seeds) + 1) * 8));
-    CUDA_TRY(err, d_ctr.ensure(8 * 8));
-    CUDA_TRY(err, d_per_read.ensure(n_reads * 8));
-    CUDA_TRY(err, cudaMemsetAsync(d_per_read.p, 0, n_reads * 8, s));
-    CUDA_TRY(err, cudaMemsetAsync(d_off.p, 0, 8, s));
-    SeedRefs const R = seed_refs(S, packed);
-    SeedBatch const B{d_pool.as<uint8_t>(), pool_len, d_seed_base.as<uint32_t>(), d_leaf_base.as<uint32_t>(), d_leaves.as<uint64_t>(),
-                      uint32_t(n_reads), n_seeds, S->bucket.as<uint32_t>(), S->pos.as<uint32_t>(), S->q};
-    seed_plan_kernel<<<seed_grid(n_seeds), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_occ.as<uint64_t>());
-    CUDA_TRY(err, cudaGetLastError());
-    size_t tmp_bytes = 0;
-    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
-    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
-    CUDA_TRY(err, cub::DeviceScan::InclusiveSum(d_tmp.p, tmp_bytes, d_occ.as<uint64_t>(), d_off.as<uint64_t>() + 1, n_seeds, s));
-    CUDA_TRY(err, K.host.ensure(std::max<size_t>(4096, n_reads * 8)));
-    uint64_t* h_ctr = K.host.as<uint64_t>();             // (moves when the buffer grows)
-    CUDA_TRY(err, cudaMemcpyAsync(h_ctr, d_off.as<uint64_t>() + n_seeds, 8, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(err, cudaStreamSynchronize(s));
-    uint64_t const total_occ = h_ctr[0];
+int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_config* cfg, fxg_read* reads, size_t n_reads,
+                          const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                          const fxg_pex_node* nodes, size_t n_nodes,
+                          uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                          fxg_seed_stats* stats, fxg_job** out) {
+    if (!c || !S || !cfg || !out || (n_reads && !reads) || (pool_len && (!forward_pool || !reverse_complement_pool)) || (n_nodes && !nodes))
+        return FXG_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    std::string err;
+    // ---- what fxg_seed_reads, then fxg_verify_reads would refuse, in that order, before any device work ----
+    SeedPlan plan;
+    if (int rc = plan_seeds(S, reads, n_reads, pool_len, nodes, n_nodes, plan, err)) return rc;
+    StoreReader guard{c};                // (until the job has run: seeding and verification both read the store)
+    const uint32_t* packed = nullptr;
+    if (int rc = take_store(c, S, guard, packed, nullptr, nullptr, nullptr, err)) return rc;
+    std::unique_lock<std::mutex> lock(c->mu);
+    if (int rc = check_verify_call(c, cfg)) return rc;
+    lock.unlock();
+    if (int rc = validate_reads(c, err, reads, 0, n_reads, pool_len, nodes, n_nodes, nullptr, 0, false)) return rc;
+    lock.lock();
+    CUDA_TRY(c->err, cudaSetDevice(c->device));
+    fxg_job* j = new_borrowed_job(c, cfg, reads, n_reads, nodes, n_nodes, pool_len);
+    if (!j) return FXG_ERR_OUT_OF_MEMORY;
+    lock.unlock();
 
-    // ---- chunks of whole seeds under the budget of q-gram occurrences (a seed above it gets a chunk of its own) ----
-    std::vector<uint64_t> off;                     // host copy of the offsets, only when the batch needs several chunks
-    if (total_occ > S->budget || n_seeds > kSeedChunkSeeds) {
-        off.resize(size_t(n_seeds) + 1);
-        CUDA_TRY(err, cudaMemcpyAsync(off.data(), d_off.p, off.size() * 8, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
+    // ---- the pools go up once: the seeder reads the job's pool (forward, then reverse complement, as SeedBatch wants) ----
+    fxg_counters ctr{};
+    int rc = stage_pool(c, j->pool, forward_pool, pool_len, reverse_complement_pool, pool_len, err, ctr, true);
+    if (rc == FXG_OK && cudaEventCreateWithFlags(&j->pool_ready, cudaEventDisableTiming | cudaEventBlockingSync) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "cannot create an event");
+    if (rc == FXG_OK && cudaEventRecord(j->pool_ready, c->stage_stream) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "staging failed");
+    // ---- seeding: the survivors land in the job's record buffer where prepare_job's layout puts the anchors ----
+    fxg_seed_stats st{};
+    st.seeds = plan.n_seeds;
+    SeedSink sink;
+    sink.dev = &j->prep.dev;
+    {
+        uint64_t n_inner = 0;
+        for (size_t i = 0; i < n_reads; ++i) n_inner += reads[i].num_inner;
+        Prepared layout;
+        carve_records(layout, n_inner, plan.leaf_info.size(), n_reads, 0);
+        sink.dev_offset = layout.o_anchors;
     }
-    auto off_at = [&](uint32_t i) { return off.empty() ? (i == 0 ? 0 : total_occ) : off[i]; };
-    fxg_anchor* result = nullptr;
-    size_t n_result = 0;
-    struct FreeResult { fxg_anchor*& p; bool keep = false; ~FreeResult() { if (!keep) std::free(p); } } free_result{result};
-    for (uint32_t s0 = 0; s0 < n_seeds;) {
-        uint32_t s1 = n_seeds;
-        if (!off.empty()) {
-            s1 = uint32_t(std::upper_bound(off.begin() + s0 + 1, off.end(), off[s0] + S->budget) - off.begin()) - 1;
-            s1 = std::min(std::max(s1, s0 + 1), std::min(n_seeds, s0 + kSeedChunkSeeds));
-        }
-        uint64_t const N = off_at(s1) - off_at(s0);
-        uint32_t const ns = s1 - s0;
-        if (N == 0) { s0 = s1; continue; }
-        if (N >= (uint64_t(1) << 31)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "seeds %u..%u have %llu q-gram occurrences: build the index with a larger q",
-                                                  s0, s1 - 1, (unsigned long long)N);
-        int const n_items = int(N);
-        // candidates: (seed, nominal start) keys, sorted and made unique
-        CUDA_TRY(err, d_keys.ensure(N * 8));
-        CUDA_TRY(err, d_sorted.ensure(N * 8));
-        CUDA_TRY(err, d_uniq.ensure(N * 8));
-        CUDA_TRY(err, d_nuniq.ensure(8));
-        CUDA_TRY(err, cudaMemsetAsync(d_ctr.p, 0, 64, s));
-        unsigned long long* const ctr = d_ctr.as<unsigned long long>();
-        seed_emit_kernel<<<seed_grid(ns), 256, 0, s>>>(B, d_info.as<uint64_t>(), d_off.as<uint64_t>(), s0, s1, d_keys.as<uint64_t>(), ctr);
-        CUDA_TRY(err, cudaGetLastError());
-        int const key_bits = std::min(64, kSeedKeyShift + bits_for(ns - 1));
-        size_t sort_bytes = 0, uniq_bytes = 0;
-        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
-        CUDA_TRY(err, cub::DeviceSelect::Unique(nullptr, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
-        CUDA_TRY(err, d_tmp.ensure(std::max(sort_bytes, uniq_bytes)));
-        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_keys.as<uint64_t>(), d_sorted.as<uint64_t>(), n_items, 0, key_bits, s));
-        CUDA_TRY(err, cub::DeviceSelect::Unique(d_tmp.p, uniq_bytes, d_sorted.as<uint64_t>(), d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(), n_items, s));
-        // check every distinct start; the hit buffer grows and the check runs again if it was too small
-        uint64_t hit_cap = std::max<uint64_t>(d_hits.cap / 8, N + 1024);
-        uint64_t n_hits = 0;
-        for (;;) {
-            CUDA_TRY(err, d_hits.ensure(hit_cap * 8));
-            seed_check_kernel<<<seed_grid(N), 256, 0, s>>>(R, B, d_info.as<uint64_t>(), s0, d_uniq.as<uint64_t>(), d_nuniq.as<uint32_t>(),
-                                                           d_hits.as<uint64_t>(), hit_cap, ctr);
-            CUDA_TRY(err, cudaGetLastError());
-            CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(err, cudaStreamSynchronize(s));
-            n_hits = h_ctr[2];
-            if (n_hits <= hit_cap) break;
-            hit_cap = n_hits;
-            CUDA_TRY(err, cudaMemsetAsync(ctr + 1, 0, 16, s));
-        }
-        st.candidates += h_ctr[0]; st.checked += h_ctr[1]; st.hits += n_hits;
-        if (n_hits == 0) { s0 = s1; continue; }
-        // caps on hits ordered by (seed, errors, position), then the kept ones by (seed, position)
-        int const hit_items = int(n_hits);
-        CUDA_TRY(err, d_hits2.ensure(n_hits * 8));
-        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
-        CUDA_TRY(err, d_tmp.ensure(sort_bytes));
-        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0,
-                                                     std::min(64, kHitKeyShift + bits_for(ns - 1)), s));
-        seed_caps_kernel<<<seed_grid(n_hits), 256, 0, s>>>(d_hits2.as<uint64_t>(), n_hits, max_anchors_hard, max_anchors_soft, d_hits.as<uint64_t>(), ctr);
-        CUDA_TRY(err, cudaGetLastError());
-        CUDA_TRY(err, cub::DeviceRadixSort::SortKeys(d_tmp.p, sort_bytes, d_hits.as<uint64_t>(), d_hits2.as<uint64_t>(), hit_items, 0, 64, s));
-        CUDA_TRY(err, cudaMemcpyAsync(h_ctr, ctr, 64, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
-        st.dropped_hard += h_ctr[3]; st.cut_soft += h_ctr[4];
-        uint64_t const n_kept = n_hits - h_ctr[3] - h_ctr[4];
-        if (n_kept == 0) { s0 = s1; continue; }
-        // erase_useless_anchors, then the survivors in order
-        CUDA_TRY(err, d_gone.ensure(n_kept * 4));
-        CUDA_TRY(err, d_at.ensure(n_kept * 4));
-        CUDA_TRY(err, d_out.ensure(n_kept * sizeof(fxg_anchor)));
-        CUDA_TRY(err, cudaMemsetAsync(d_gone.p, 0, n_kept * 4, s));
-        if (erase_useless_anchors) {
-            seed_erase_kernel<<<seed_grid(n_kept), 256, 0, s>>>(R, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>());
-            CUDA_TRY(err, cudaGetLastError());
-        }
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
-        CUDA_TRY(err, d_tmp.ensure(tmp_bytes));
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_gone.as<uint32_t>(), d_at.as<uint32_t>(), int(n_kept), s));
-        seed_output_kernel<<<seed_grid(n_kept), 256, 0, s>>>(R, B, s0, d_hits2.as<uint64_t>(), n_kept, d_gone.as<uint32_t>(), d_at.as<uint32_t>(),
-                                                             d_out.as<uint64_t>(), d_per_read.as<uint32_t>(), ctr);
-        CUDA_TRY(err, cudaGetLastError());
-        // back through page-locked memory: the counters, then up to n_kept records
-        CUDA_TRY(err, K.host.ensure(64 + n_kept * sizeof(fxg_anchor)));
-        uint64_t* const h = h_ctr = K.host.as<uint64_t>();
-        CUDA_TRY(err, cudaMemcpyAsync(h, ctr, 64, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaMemcpyAsync(h + 8, d_out.p, n_kept * sizeof(fxg_anchor), cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
-        st.erased += h[5];
-        uint64_t const n_out = n_kept - h[5];
-        if (n_out) {
-            fxg_anchor* grown = static_cast<fxg_anchor*>(std::realloc(result, (n_result + n_out) * sizeof(fxg_anchor)));
-            if (!grown) return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate %llu anchors", (unsigned long long)(n_result + n_out));
-            result = grown;
-            std::memcpy(result + n_result, h + 8, n_out * sizeof(fxg_anchor));
-            n_result += n_out;
-        }
-        s0 = s1;
+    if (rc == FXG_OK && plan.n_seeds) {
+        SeedCall K{c};
+        if (cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "cannot create a stream");
+        if (rc == FXG_OK) rc = seed_batch(c, S, packed, plan, n_reads, K, j->pool.bytes.as<uint8_t>(), pool_len, j->pool_ready, max_anchors_hard,
+                                          max_anchors_soft, erase_useless_anchors, sink, st, err);
     }
-    std::vector<uint32_t> per_read(2 * n_reads);
-    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_per_read.p, n_reads * 8, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(err, cudaStreamSynchronize(s));
-    std::memcpy(per_read.data(), K.host.p, n_reads * 8);
-    uint64_t sum = 0;
-    for (uint32_t v : per_read) sum += v;
-    if (sum != n_result) return fail(err, FXG_ERR_CUDA, "internal: %llu anchors counted per read, %zu written", (unsigned long long)sum, n_result);
-    *anchors = result; *n_anchors = n_result;
-    free_result.keep = true;
-    return finish(per_read);
+    ctr.h2d_bytes += sink.h2d_bytes; ctr.d2h_bytes += sink.d2h_bytes;
+    if (rc == FXG_OK) {
+        set_read_anchors(reads, n_reads, sink.per_read);
+        index_walks(j);
+        // (seed_batch drained its stream before it returned: Prepared::ready, recorded behind the records' upload, covers
+        //  the anchors it wrote as well)
+        rc = prepare_job(c, j, err, ctr, true);
+    }
+    if (rc == FXG_OK && !j->prep.ok && sink.n) {
+        // the host-driven levels take the job: they read fxg_anchor records on the host (the walks do not use num_errors)
+        std::vector<AnchorRec16> back(sink.n);
+        if (cudaMemcpy(back.data(), j->prep.dev.as<uint8_t>() + sink.dev_offset, sink.n * sizeof(AnchorRec16), cudaMemcpyDeviceToHost) != cudaSuccess)
+            rc = fail(err, FXG_ERR_CUDA, "cannot copy the anchors back");
+        ctr.d2h_bytes += sink.n * sizeof(AnchorRec16);
+        j->anchors.resize(sink.n);
+        for (size_t i = 0; i < sink.n; ++i) j->anchors[i] = fxg_anchor{back[i].pex_leaf_index, back[i].reference_id, back[i].reference_position, 0};
+        j->anchors_p = j->anchors.data(); j->n_anchors = sink.n;
+    }
+    rc = run_borrowed_job(c, j, rc, err, ctr, out);
+    if (rc == FXG_OK && stats) *stats = st;
+    return rc;
 }
 
 }  // extern "C"

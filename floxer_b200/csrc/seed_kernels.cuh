@@ -10,7 +10,8 @@
 //             banded prefix_distance, band in registers;
 //   caps      seed_caps_kernel on hits sorted by (seed, errors, position): hard cap, soft cap;
 //   erase     seed_erase_kernel on kept hits sorted by (seed, position): the host's erase_useless per (seed, reference);
-//   output    seed_output_kernel: fxg_anchor records in seed order, counts per (read, orientation).
+//   output    seed_output_kernel<J>: the survivors in seed order -- fxg_anchor records (fxg_seed_reads) or a verification job's
+//             AnchorRec16 (fxg_seed_verify_reads) -- and counts per (read, orientation).
 #pragma once
 
 #include <cstdint>
@@ -321,9 +322,12 @@ __global__ void seed_erase_kernel(SeedRefs R, const uint64_t* __restrict__ kept,
     }
 }
 
-// survivors (they go to i - at[i], at = exclusive prefix sum of erased) as fxg_anchor-shaped records, counted per (read, orientation)
+// survivors (they go to i - at[i], at = exclusive prefix sum of erased), counted per (read, orientation): as fxg_anchor-shaped
+// records (four words: leaf, reference, position, errors), or with kJobRecords as the AnchorRec16 a verification job reads
+// (position, leaf, reference; the walks do not use the errors)
+template <bool kJobRecords>
 __global__ void seed_output_kernel(SeedRefs R, SeedBatch B, uint32_t s0, const uint64_t* __restrict__ kept, uint64_t n,
-                                   const uint32_t* __restrict__ erased, const uint32_t* __restrict__ at, uint64_t* __restrict__ out,
+                                   const uint32_t* __restrict__ erased, const uint32_t* __restrict__ at, void* __restrict__ out,
                                    uint32_t* __restrict__ per_read, unsigned long long* __restrict__ ctr) {
     uint64_t const i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
     uint64_t gone = 0;
@@ -336,11 +340,18 @@ __global__ void seed_output_kernel(SeedRefs R, SeedBatch B, uint32_t s0, const u
             uint32_t const local = s - B.seed_base[rd], nl = B.leaf_base[rd + 1] - B.leaf_base[rd];
             uint32_t const strand = local >= nl;
             uint32_t const r = seed_ref_of(R.ubase, R.n_refs, g);
-            uint64_t* o = out + 4 * (i - at[i]);
-            o[0] = local - strand * nl;
-            o[1] = r;
-            o[2] = g - R.ubase[r];
-            o[3] = kept[i] & 15u;
+            if constexpr (kJobRecords) {
+                AnchorRec16& o = static_cast<AnchorRec16*>(out)[i - at[i]];
+                o.reference_position = g - R.ubase[r];
+                o.pex_leaf_index = local - strand * nl;
+                o.reference_id = r;
+            } else {
+                uint64_t* o = static_cast<uint64_t*>(out) + 4 * (i - at[i]);
+                o[0] = local - strand * nl;
+                o[1] = r;
+                o[2] = g - R.ubase[r];
+                o[3] = kept[i] & 15u;
+            }
             atomicAdd(&per_read[2 * rd + strand], 1u);
         }
     }

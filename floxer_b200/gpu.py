@@ -23,7 +23,7 @@ EXPORTS = [
     "fxg_get_counters", "fxg_reset_counters", "fxg_measure_int32_peak", "fxg_engine_shape",
     "fxg_pex_build", "fxg_pex_free", "fxg_job_write_sam", "fxg_free", "fxg_write_bam", "fxg_job_write_bam",
     "fxg_seeder_create", "fxg_seeder_free", "fxg_seeder_search",
-    "fxg_gpu_seeder_create", "fxg_gpu_seeder_free", "fxg_seed_reads",
+    "fxg_gpu_seeder_create", "fxg_gpu_seeder_free", "fxg_seed_reads", "fxg_seed_verify_reads",
 ]
 
 _lib = None
@@ -94,6 +94,8 @@ def lib() -> C.CDLL:
     L.fxg_gpu_seeder_free.restype = None
     L.fxg_seed_reads.argtypes = [vp, vp, vp, sz, vp, vp, sz, vp, sz, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(vp), C.POINTER(sz),
                                  C.POINTER(abi.SeedStats)]
+    L.fxg_seed_verify_reads.argtypes = [vp, vp, vp, vp, sz, vp, vp, sz, vp, sz, C.c_uint64, C.c_uint64, C.c_int,
+                                        C.POINTER(abi.SeedStats), C.POINTER(vp)]
     _lib = L
     return L
 
@@ -434,6 +436,21 @@ class Context:
         else:
             anchors = np.zeros(0, dtype=abi.ANCHOR_DTYPE)
         return ReadBatch(reads, batch.forward_pool, batch.reverse_pool, batch.nodes, anchors, dict(batch.meta)), st.as_dict()
+
+    def seed_verify_reads(self, seeder: GpuSeeder, batch: ReadBatch, config: VerifyConfig, max_anchors_hard: int = 500,
+                          max_anchors_soft: int = 50, erase_useless: bool = True):
+        """fxg_seed_verify_reads: seed_reads then verify_reads in one call, the anchors kept in device memory.  Returns
+        (Job, a new ReadBatch with the updated read records and no anchors -- what Job.sam / Job.bam take --, stats dict);
+        `batch` is not modified.  The results equal those of verify_reads on seed_reads's batch."""
+        reads = batch.reads.copy()
+        cfg = config.to_c()
+        h, st = C.c_void_p(), abi.SeedStats()
+        self._check(lib().fxg_seed_verify_reads(self._h, seeder._h, C.byref(cfg), reads.ctypes.data, len(reads),
+                                                batch.forward_pool.ctypes.data, batch.reverse_pool.ctypes.data,
+                                                len(batch.forward_pool), batch.nodes.ctypes.data, len(batch.nodes),
+                                                max_anchors_hard, max_anchors_soft, int(erase_useless), C.byref(st), C.byref(h)))
+        seeded = ReadBatch(reads, batch.forward_pool, batch.reverse_pool, batch.nodes, np.zeros(0, dtype=abi.ANCHOR_DTYPE), dict(batch.meta))
+        return Job(self, h, (seeded, cfg)), seeded, st.as_dict()
 
     # ---- accounting ----
     def counters(self) -> dict:

@@ -19,6 +19,8 @@
  *   fxg_seed_reads       search::searcher::search_seeds (src/lib/search.cpp:143-324) for both orientations of every read
  *                        of a batch (src/lib/parallelization.cpp:94-101), on the device: the q-gram seeder of
  *                        fxg_seeder_search with its index (fxg_gpu_seeder_create) built from the resident references.
+ *   fxg_seed_verify_reads a search task's seeding and verification of a batch in one call (src/lib/parallelization.cpp:94-101
+ *                        then :230-249): fxg_seed_reads + fxg_verify_reads with the anchors kept in device memory.
  *
  * Struct layouts fxg_pex_node and fxg_anchor are byte-identical to pex::pex_tree::node
  * (include/pex.hpp:59-70) and search::anchor_t (include/search.hpp:27-31) on LP64, so the
@@ -294,6 +296,24 @@ int  fxg_seed_reads(fxg_ctx* ctx, const fxg_gpu_seeder* seeder, fxg_read* reads,
                     const fxg_pex_node* nodes, size_t n_nodes,
                     uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
                     fxg_anchor** anchors, size_t* n_anchors, fxg_seed_stats* stats);
+
+/* fxg_seed_reads followed by fxg_verify_reads on the same batch, without the anchors leaving the device.  `reads` is
+ * in/out exactly as for fxg_seed_reads (anchor_offset, num_anchors_forward, num_anchors_reverse are written).  The job
+ * is the one fxg_verify_reads would return for the seeded batch: the same alignments in the same order, the same CIGARs
+ * and statistics; it is read with fxg_job_* / fxg_job_write_sam / fxg_job_write_bam and, like fxg_verify_reads's job,
+ * cannot be run again.  stats may be NULL.
+ * The query pools go up once; the seeder writes the surviving anchors straight into the job's device records and only
+ * their counts per read (8 bytes) come back.  An input either call refuses is refused with its code and text before any
+ * device work (a seeding refusal first); a rank above 5 in a pool is reported after the run, as fxg_verify_reads does.
+ * The job joins the batch queue like an fxg_verify_reads job and merges with jobs of the same fxg_verify_config;
+ * fxg_set_references fails with FXG_ERR_STATE while the call runs.  The copies it makes, seeding included, are counted
+ * in fxg_counters h2d_bytes / d2h_bytes. */
+int  fxg_seed_verify_reads(fxg_ctx* ctx, const fxg_gpu_seeder* seeder, const fxg_verify_config* config,
+                           fxg_read* reads, size_t n_reads,
+                           const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                           const fxg_pex_node* nodes, size_t n_nodes,
+                           uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                           fxg_seed_stats* stats, fxg_job** out);
 
 /* ---- accounting / measurement helpers ---- */
 int fxg_get_counters(const fxg_ctx* ctx, fxg_counters* out);
