@@ -10,6 +10,7 @@
 // split over one or more host workers with their own CUDA streams and buffers.
 // No CPU fallback exists: every alignment result comes from dp_kernels.cuh.
 #include "../../include/floxer_gpu.h"
+#include "bam_kernels.cuh"
 #include "dp_kernels.cuh"
 #include "root_kernels.cuh"
 #include "seed_kernels.cuh"
@@ -4070,6 +4071,245 @@ int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_
     rc = run_borrowed_job(c, j, rc, err, ctr, out);
     if (rc == FXG_OK && stats) *stats = st;
     return rc;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ BAM on the device
+
+namespace {
+
+// The batch as the BAM kernels read it, and what fxg_write_bam would refuse.  bam_output.cpp walks the reads in order,
+// a read's alignments in their stable order by reference id, and checks every record as it appends it; the first
+// failure it would meet decides the code returned here.
+struct BamPlan {
+    std::vector<BamReadRec> reads;
+    std::string header;                                    // the BAM header bytes (empty without it)
+    uint64_t cigar_lo = UINT64_MAX, cigar_hi = 0, seq_lo = UINT64_MAX, seq_hi = 0, names_len = 0, quals_len = 0;
+    uint64_t n_rec = 0;
+};
+
+int plan_bam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references, const char* const* reference_ids,
+             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const fxg_sam_query* queries, int with_header,
+             BamPlan& P, std::string& err) {
+    P.reads.resize(n_reads);
+    size_t a = 0;
+    for (size_t ri = 0; ri < n_reads; ++ri) {
+        size_t const a0 = a;
+        while (a < n_al && al[a].read_index == ri) ++a;
+        if (a < n_al && al[a].read_index < ri)
+            return fail(err, FXG_ERR_STATE, "alignment %zu (read %u) follows read %zu: alignments must be grouped by read", a, al[a].read_index, ri);
+        const char* const qname = queries[ri].id ? queries[ri].id : "*";
+        size_t const l_name = std::strlen(qname) + 1;
+        if (a == a0 && l_name > 255) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: the name has %zu characters (254 at most)", ri, l_name - 1);
+        // the first failing alignment in (reference id, index) order
+        uint64_t first = UINT64_MAX;
+        int code = FXG_OK;
+        for (size_t k = a0; k < a; ++k) {
+            fxg_alignment const& A = al[k];
+            int e = FXG_OK;
+            if (A.reference_id >= n_references || (A.cigar_len && !cigar_pool) || l_name > 255) e = FXG_ERR_INVALID_ARGUMENT;
+            else if (A.cigar_len > 65535) {
+                int64_t rs = 0, qs = 0;
+                for (uint32_t i = 0; i < A.cigar_len; ++i) {
+                    uint32_t const v = cigar_pool[A.cigar_offset + i], op = v & 15u;
+                    if (op == FXG_CIGAR_D || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) rs += v >> 4;
+                    if (op == FXG_CIGAR_I || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) qs += v >> 4;
+                }
+                if (qs >= (int64_t(1) << 28) || rs >= (int64_t(1) << 28)) e = FXG_ERR_OVERFLOW;
+            }
+            uint64_t const key = uint64_t(A.reference_id) << 32 | (k - a0);
+            if (e != FXG_OK && key < first) { first = key; code = e; }
+            if (A.cigar_len) { P.cigar_lo = std::min<uint64_t>(P.cigar_lo, A.cigar_offset); P.cigar_hi = std::max<uint64_t>(P.cigar_hi, A.cigar_offset + A.cigar_len); }
+        }
+        if (code == FXG_ERR_OVERFLOW)
+            return fail(err, code, "read %zu: a CIGAR of more than 65535 operations spans 2^28 bases or more (the CG tag's placeholder cannot hold it)", ri);
+        if (code != FXG_OK) return fail(err, code, "read %zu: a reference id out of range, a CIGAR without a pool or a name of more than 254 characters", ri);
+        fxg_read const& R = reads[ri];
+        const char* const q = queries[ri].quality;
+        bool const have_qual = q && q[0] && std::strlen(q) == R.query_len;
+        BamReadRec& B = P.reads[ri];
+        B.seq = R.query_offset;
+        B.qual = have_qual ? P.quals_len : ~uint64_t(0);
+        B.l_seq = R.query_len;
+        B.name = uint32_t(P.names_len);
+        B.al0 = uint32_t(a0); B.n_al = uint32_t(a - a0);
+        B.rec0 = uint32_t(P.n_rec); B.l_name = uint32_t(l_name);
+        P.names_len += l_name;
+        if (have_qual) P.quals_len += R.query_len;
+        if (R.query_len) { P.seq_lo = std::min<uint64_t>(P.seq_lo, R.query_offset); P.seq_hi = std::max<uint64_t>(P.seq_hi, R.query_offset + R.query_len); }
+        P.n_rec += std::max<size_t>(a - a0, 1);
+    }
+    if (a != n_al) return fail(err, FXG_ERR_STATE, "alignment %zu names read %u of %zu: alignments must be grouped by read in read order", a, al[a].read_index, n_reads);
+    if (P.n_rec >= (uint64_t(1) << 32) || P.names_len >= (uint64_t(1) << 32))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "%llu records: split the batch", (unsigned long long)P.n_rec);
+    if (P.seq_lo > P.seq_hi) P.seq_lo = P.seq_hi = 0;
+    if (P.cigar_lo > P.cigar_hi) P.cigar_lo = P.cigar_hi = 0;
+    for (BamReadRec& B : P.reads) B.seq -= std::min(B.seq, P.seq_lo);
+    if (with_header) {                                     // bam_output.cpp's header, byte for byte
+        std::string text = "@HD\tVN:1.6\tSO:unknown\tGO:none\n";
+        for (size_t r = 0; r < n_references; ++r) { text += "@SQ\tSN:"; text += reference_ids[r]; text += "\tLN:"; text += std::to_string(reference_lengths[r]); text += '\n'; }
+        auto u32 = [&](uint32_t v) { for (int i = 0; i < 4; ++i) P.header += char(uint8_t(v >> (8 * i))); };
+        P.header += "BAM\1";
+        u32(uint32_t(text.size())); P.header += text;
+        u32(uint32_t(n_references));
+        for (size_t r = 0; r < n_references; ++r) {
+            size_t const l = std::strlen(reference_ids[r]) + 1;
+            u32(uint32_t(l)); P.header.append(reference_ids[r], l);
+            u32(uint32_t(std::min<uint64_t>(reference_lengths[r], uint64_t(INT32_MAX))));
+        }
+    }
+    return FXG_OK;
+}
+
+constexpr uint8_t kBgzfEof[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+
+static_assert(sizeof(DeflateSmem) <= 227 * 1024, "the deflate kernel's shared memory exceeds a block's 227 KB");
+
+size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+}  // namespace
+
+extern "C" {
+
+int fxg_write_bam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
+                         const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
+                         const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len) {
+    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
+        return FXG_ERR_INVALID_ARGUMENT;
+    *bytes = nullptr; *bytes_len = 0;
+    std::string err;
+    try {
+    BamPlan P;
+    if (int rc = plan_bam(al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
+    if (P.n_rec == 0 && P.header.empty()) {                // nothing but the end-of-file block
+        uint8_t* buf = static_cast<uint8_t*>(std::malloc(sizeof kBgzfEof));
+        if (!buf) return FXG_ERR_OUT_OF_MEMORY;
+        std::memcpy(buf, kBgzfEof, sizeof kBgzfEof);
+        *bytes = buf; *bytes_len = sizeof kBgzfEof;
+        return FXG_OK;
+    }
+
+    // ---- one upload through page-locked staging: reads, alignments, CIGAR range, forward-pool range, names, qualities, header ----
+    size_t const o_reads = 0;
+    size_t const o_al = align_up(o_reads + n_reads * sizeof(BamReadRec), 256);
+    size_t const o_cig = align_up(o_al + n_al * sizeof(fxg_alignment), 256);
+    size_t const o_seq = align_up(o_cig + (P.cigar_hi - P.cigar_lo) * 4, 256);
+    size_t const o_names = align_up(o_seq + (P.seq_hi - P.seq_lo), 256);
+    size_t const o_quals = align_up(o_names + P.names_len, 256);
+    size_t const o_header = align_up(o_quals + P.quals_len, 256);
+    size_t const up = align_up(o_header + P.header.size(), 256);
+    CUDA_TRY(err, cudaSetDevice(c->device));
+    SeedCall K{c};
+    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    cudaStream_t const s = K.st;
+    CUDA_TRY(err, K.host.ensure(up + 64));
+    uint8_t* const h = K.host.as<uint8_t>();
+    if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(BamReadRec));
+    if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
+    if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
+    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
+    for (size_t ri = 0; ri < n_reads; ++ri) {
+        BamReadRec const& B = P.reads[ri];
+        std::memcpy(h + o_names + B.name, queries[ri].id ? queries[ri].id : "*", B.l_name);
+        if (B.qual != ~uint64_t(0)) std::memcpy(h + o_quals + B.qual, queries[ri].quality, B.l_seq);
+    }
+    std::memcpy(h + o_header, P.header.data(), P.header.size());
+    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_raw = K.bufs[5],
+           &d_work = K.bufs[6], &d_slots = K.bufs[7], &d_info = K.bufs[8], &d_bsize = K.bufs[9], &d_boff = K.bufs[10], &d_img = K.bufs[11];
+    CUDA_TRY(err, d_in.ensure(up));
+    CUDA_TRY(err, cudaMemcpyAsync(d_in.p, h, up, cudaMemcpyHostToDevice, s));
+    uint64_t h2d = up, d2h = 0, launches = 0;
+    uint8_t* const din = d_in.as<uint8_t>();
+    BamArgs A{};
+    A.reads = reinterpret_cast<const BamReadRec*>(din + o_reads); A.n_reads = uint32_t(n_reads);
+    A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
+    A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
+    A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = din + o_quals;
+
+    // ---- record sizes, their offsets, the stream's length ----
+    uint32_t const n_rec = uint32_t(P.n_rec);
+    uint64_t* const h_word = reinterpret_cast<uint64_t*>(h + up);           // (read-backs go behind the upload)
+    uint64_t body = 0;
+    if (n_rec) {
+        CUDA_TRY(err, d_rec.ensure(size_t(n_rec) * sizeof(BamRecord)));
+        CUDA_TRY(err, d_size.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, d_off.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, cudaMemsetAsync(d_size.as<uint64_t>() + n_rec, 0, 8, s));
+        A.recs = d_rec.as<BamRecord>(); A.rec_off = d_size.as<uint64_t>();
+        bam_size_kernel<<<uint32_t((uint64_t(n_reads) * 32 + 255) / 256), 256, 0, s>>>(A);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+        size_t tmp_bytes = 0;
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_word, d_off.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        d2h += 8;
+        body = h_word[0];
+    }
+    uint64_t const raw_len = P.header.size() + body;
+    uint32_t const n_chunks = uint32_t((raw_len + kBgzfChunk - 1) / kBgzfChunk);
+
+    // ---- the raw stream: the header, then the records ----
+    CUDA_TRY(err, d_raw.ensure(raw_len + 16));
+    if (!P.header.empty()) CUDA_TRY(err, cudaMemcpyAsync(d_raw.p, din + o_header, P.header.size(), cudaMemcpyDeviceToDevice, s));
+    A.rec_off = d_off.as<uint64_t>(); A.raw = d_raw.as<uint8_t>(); A.body = P.header.size();
+    if (n_rec) {
+        bam_write_kernel<<<uint32_t((uint64_t(n_rec) * 32 + 255) / 256), 256, 0, s>>>(A, n_rec);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+    }
+
+    // ---- BGZF blocks: deflate per chunk, block offsets, the image ----
+    CUDA_TRY(err, d_work.ensure(raw_len * 4));
+    CUDA_TRY(err, d_slots.ensure(size_t(n_chunks) * kBgzfSlotWords * 4));
+    CUDA_TRY(err, d_info.ensure(size_t(n_chunks) * sizeof(BgzfBlockInfo)));
+    CUDA_TRY(err, d_bsize.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, d_boff.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, cudaFuncSetAttribute(bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(DeflateSmem))));
+    bgzf_deflate_kernel<<<n_chunks, kDeflateThreads, sizeof(DeflateSmem), s>>>(d_raw.as<uint8_t>(), raw_len, d_work.as<uint32_t>(),
+                                                                              d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(),
+                                                                              d_bsize.as<uint64_t>(), n_chunks);
+    CUDA_TRY(err, cudaGetLastError());
+    size_t tmp_bytes = 0;
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
+    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
+    // (the image is at most the raw stream stored, plus framing)
+    CUDA_TRY(err, d_img.ensure(raw_len + (uint64_t(n_chunks) + 1) * 31 + 28));
+    bgzf_assemble_kernel<<<n_chunks + 1, 256, 0, s>>>(d_raw.as<uint8_t>(), d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(),
+                                                      d_boff.as<uint64_t>(), n_chunks, d_img.as<uint8_t>());
+    CUDA_TRY(err, cudaGetLastError());
+    launches += 2;
+    CUDA_TRY(err, cudaMemcpyAsync(h_word, d_boff.as<uint64_t>() + n_chunks + 1, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    d2h += 8;
+    size_t const img_len = size_t(h_word[0]);
+    CUDA_TRY(err, K.host.ensure(img_len));
+    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_img.p, img_len, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    d2h += img_len;
+    {
+        std::lock_guard<std::mutex> lock(c->mu);
+        c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
+    }
+    uint8_t* buf = static_cast<uint8_t*>(std::malloc(img_len));
+    if (!buf) return FXG_ERR_OUT_OF_MEMORY;
+    std::memcpy(buf, K.host.p, img_len);
+    *bytes = buf; *bytes_len = img_len;
+    return FXG_OK;
+    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+}
+
+int fxg_job_write_bam_device(fxg_ctx* c, const fxg_job* job, size_t n_references, const char* const* reference_ids,
+                             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool,
+                             const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len) {
+    if (!job) return FXG_ERR_INVALID_ARGUMENT;
+    return fxg_write_bam_device(c, fxg_job_alignments(job), fxg_job_num_alignments(job), fxg_job_cigar_pool(job), n_references, reference_ids,
+                                reference_lengths, reads, n_reads, forward_pool, queries, with_header, bytes, bytes_len);
 }
 
 }  // extern "C"

@@ -24,6 +24,7 @@ EXPORTS = [
     "fxg_pex_build", "fxg_pex_free", "fxg_job_write_sam", "fxg_free", "fxg_write_bam", "fxg_job_write_bam",
     "fxg_seeder_create", "fxg_seeder_free", "fxg_seeder_search",
     "fxg_gpu_seeder_create", "fxg_gpu_seeder_free", "fxg_seed_reads", "fxg_seed_verify_reads",
+    "fxg_write_bam_device", "fxg_job_write_bam_device",
 ]
 
 _lib = None
@@ -85,6 +86,8 @@ def lib() -> C.CDLL:
     L.fxg_free.restype = None
     L.fxg_write_bam.argtypes = [vp, sz, vp, sz, vp, vp, vp, sz, vp, vp, C.c_int, C.POINTER(vp), C.POINTER(sz)]
     L.fxg_job_write_bam.argtypes = [vp, sz, vp, vp, vp, sz, vp, vp, C.c_int, C.POINTER(vp), C.POINTER(sz)]
+    L.fxg_write_bam_device.argtypes = [vp, *L.fxg_write_bam.argtypes]
+    L.fxg_job_write_bam_device.argtypes = [vp, *L.fxg_job_write_bam.argtypes]
     L.fxg_seeder_create.argtypes = [sz, vp, vp, C.c_uint32, C.POINTER(vp)]
     L.fxg_seeder_free.argtypes = [vp]
     L.fxg_seeder_free.restype = None
@@ -279,15 +282,21 @@ class Job:
         finally:
             L.fxg_free(text)
 
-    def bam(self, batch: ReadBatch, reference_ids, reference_lengths, query_ids, qualities=None, header: bool = True) -> bytes:
-        """The same records as a BAM file image (BGZF blocks incl. the end-of-file block): fxg_job_write_bam."""
+    def bam(self, batch: ReadBatch, reference_ids, reference_lengths, query_ids, qualities=None, header: bool = True,
+            on_device: bool = False) -> bytes:
+        """The same records as a BAM file image (BGZF blocks incl. the end-of-file block): fxg_job_write_bam, or with
+        on_device=True fxg_job_write_bam_device on the job's context (the same records and blocks, compressed on the GPU)."""
         L = lib()
         n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
         out, length = C.c_void_p(), C.c_size_t(0)
-        rc = L.fxg_job_write_bam(self._h, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data,
-                                 qs, int(header), C.byref(out), C.byref(length))
-        if rc != 0:
-            raise FloxerGpuError(rc, "fxg_job_write_bam failed")
+        args = (self._h, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs, int(header),
+                C.byref(out), C.byref(length))
+        if on_device:
+            self._ctx._check(L.fxg_job_write_bam_device(self._ctx._h, *args))
+        else:
+            rc = L.fxg_job_write_bam(*args)
+            if rc != 0:
+                raise FloxerGpuError(rc, "fxg_job_write_bam failed")
         try:
             return C.string_at(out, length.value)
         finally:
@@ -451,6 +460,24 @@ class Context:
                                                 max_anchors_hard, max_anchors_soft, int(erase_useless), C.byref(st), C.byref(h)))
         seeded = ReadBatch(reads, batch.forward_pool, batch.reverse_pool, batch.nodes, np.zeros(0, dtype=abi.ANCHOR_DTYPE), dict(batch.meta))
         return Job(self, h, (seeded, cfg)), seeded, st.as_dict()
+
+    # ---- BAM output on the device ----
+    def write_bam(self, alignments, cigars, batch, reference_ids, reference_lengths, query_ids, qualities=None,
+                  header: bool = True) -> bytes:
+        """gpu.write_bam with the work on this context's device (fxg_write_bam_device): the same records and BGZF blocks,
+        deflated on the GPU."""
+        L = lib()
+        al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
+        cg = np.ascontiguousarray(cigars, dtype=np.uint32)
+        n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
+        out, length = C.c_void_p(), C.c_size_t(0)
+        self._check(L.fxg_write_bam_device(self._h, al.ctypes.data if len(al) else None, len(al), cg.ctypes.data if len(cg) else None,
+                                           n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs,
+                                           int(header), C.byref(out), C.byref(length)))
+        try:
+            return C.string_at(out, length.value)
+        finally:
+            L.fxg_free(out)
 
     # ---- accounting ----
     def counters(self) -> dict:

@@ -251,6 +251,29 @@ int fxg_job_write_bam(const fxg_job* job, size_t n_references, const char* const
                       const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool, const fxg_sam_query* queries,
                       int with_header, uint8_t** bytes, size_t* bytes_len);
 
+/* fxg_write_bam with the work on the device of ctx: record assembly and BGZF deflate run there and only the finished
+ * image comes back.  Contract:
+ *  - the same records: the uncompressed stream is byte-identical to fxg_write_bam's for the same arguments (header,
+ *    record order, primary choice, flags, MAPQ 255, bin, SEQ with '$' as N, QUAL or 0xff, NM, the CG:B,I tag);
+ *  - the same blocks: the stream is cut at the same 0xff00-byte boundaries, so block i has the ISIZE and CRC32 of
+ *    fxg_write_bam's block i, and the 28-byte end-of-file block is identical.  Only the deflate payloads differ: LZ77
+ *    with dynamic Huffman codes, or a stored block where that is not larger;
+ *  - the same refusals: an input fxg_write_bam refuses is refused with the same code before any device work
+ *    (FXG_ERR_STATE: alignments not grouped by read; FXG_ERR_INVALID_ARGUMENT: a reference id out of range, a name of
+ *    more than 254 characters; FXG_ERR_OVERFLOW: a CIGAR of more than 65535 operations spanning 2^28 bases or more);
+ *  - deterministic: the same input gives the same bytes;
+ *  - concurrent: the call works on a stream of its own and does not hold the context's lock, so several writers and
+ *    verification batches can run at once.  Its copies go through page-locked staging and are counted in fxg_counters
+ *    h2d_bytes / d2h_bytes.  Needs no references.
+ * Writes a malloc'ed buffer; release it with fxg_free. */
+int fxg_write_bam_device(fxg_ctx* ctx, const fxg_alignment* alignments, size_t n_alignments, const uint32_t* cigar_pool,
+                         size_t n_references, const char* const* reference_ids, const uint64_t* reference_lengths,
+                         const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool, const fxg_sam_query* queries,
+                         int with_header, uint8_t** bytes, size_t* bytes_len);
+int fxg_job_write_bam_device(fxg_ctx* ctx, const fxg_job* job, size_t n_references, const char* const* reference_ids,
+                             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool,
+                             const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len);
+
 /* ---- a q-gram seeder behind the anchor interface (host only; row N2 of the scope table) ----
  * Stands in for search::searcher::search_seeds (src/lib/search.cpp:143-324), whose FM-index library cannot be built
  * offline: per PEX leaf every reference position where the leaf matches a prefix of the reference with at most
