@@ -810,7 +810,6 @@ struct Walk2Launch {
     const uint32_t* ck;
     const uint32_t* ref_packed; const uint32_t* inline_packed;
     const uint32_t* peq_table; uint64_t peq_plane_words;
-    const uint8_t* query_pool;
     uint32_t* cigars;
     WalkResult* results;
     uint32_t two;

@@ -229,6 +229,20 @@ struct Worker {
         }
         return e;
     }
+    // n independent launches side by side: fork(main, n) before the first, fan_stream(main, q) for launch q -- `main` for
+    // the first, a side stream that waits for the fork for the others -- and join(main, n) after the last
+    cudaError_t fork(cudaStream_t main, int n) { return n > 1 ? cudaEventRecord(ev_fork, main) : cudaSuccess; }
+    cudaError_t fan_stream(cudaStream_t main, int q, cudaStream_t& s) {
+        if (q == 0) { s = main; return cudaSuccess; }
+        s = side[(q - 1) % kSide];
+        return q <= kSide ? cudaStreamWaitEvent(s, ev_fork, 0) : cudaSuccess;
+    }
+    cudaError_t join(cudaStream_t main, int n) {
+        cudaError_t e = cudaSuccess;
+        for (int q = 0; q < std::min(n - 1, kSide) && e == cudaSuccess; ++q)
+            if ((e = cudaEventRecord(ev_join[q], side[q])) == cudaSuccess) e = cudaStreamWaitEvent(main, ev_join[q], 0);
+        return e;
+    }
     // tracebacks are long chains of dependent steps: the root alignments of a wave are cut into chunks, each chunk's
     // tracebacks run on a stream of their own beside the score passes (and tracebacks) of the other chunks
     static constexpr int kWalkSlots = 4;
@@ -588,6 +602,12 @@ cudaError_t set_all_smem_attrs(size_t bytes) {
 
 inline uint32_t peq_stride_for(uint32_t words) { return (words + 3u) & ~3u; }   // rows stay 16-byte aligned for LDS.128
 
+// shared memory of an engine launch with ring size G and Eq tables of `words` words: a window buffer and a table per
+// task of the warp, or the multi-warp kernel's (G = kWideG)
+inline size_t engine_smem_bytes(uint32_t G, uint32_t words) {
+    return G == kWideG ? wide_smem_bytes() : size_t(32 / G) * (kWinBytes + size_t(kNumSymbols) * peq_stride_for(words) * 4);
+}
+
 // word-steps the engine issues for a pass: block b is active for columns cs(b)..ce(b)
 uint64_t word_steps_of(Pass const& p, uint32_t W, uint32_t nb) {
     uint32_t const rows = 32 * W;
@@ -634,7 +654,7 @@ bool choose_config(Pass const& p, size_t smem_limit, bool force_wide, Config& ou
         }
         uint32_t const tpw = 32 / G;
         G = 32 / tpw;                        // the lanes a smaller ring would leave idle cost nothing, and fewer classes mean fuller launches
-        size_t const smem = size_t(tpw) * (kWinBytes + size_t(kNumSymbols) * peq_stride_for(nb * W) * 4);
+        size_t const smem = engine_smem_bytes(G, nb * W);
         if (smem > smem_limit) continue;
         // The engine is bound by the ALU pipe: a warp step issues about 10 W + 6 instructions there, two cycles each on one
         // of the SM's four schedulers, whatever the number of lanes that do useful work.  Wide blocks need many registers
@@ -660,7 +680,7 @@ bool choose_config(Pass const& p, size_t smem_limit, bool force_wide, Config& ou
     if (!found) {
         // no ring of one warp holds this band: the multi-warp kernel (dp_wide_kernel), one block of 1 024 rows per thread
         uint32_t const nb = (nw + 31) / 32;
-        if (nb <= kWideThreads && wide_smem_bytes() <= smem_limit) { out = Config{5, uint8_t(kWideG), nb, 0}; found = true; }
+        if (nb <= kWideThreads && engine_smem_bytes(kWideG, nb * 32) <= smem_limit) { out = Config{5, uint8_t(kWideG), nb, 0}; found = true; }
     }
     if (found) out.word_steps = word_steps_of(p, uint32_t(kWidths[out.widx]), out.nb);
     return found;
@@ -722,6 +742,46 @@ void radix_sort(std::vector<uint64_t>& keys, std::vector<uint64_t>& tmp, int lo_
 std::vector<ConfigCacheEntry>& thread_config_cache(const fxg_ctx* c);
 
 // ------------------------------------------------------------------------------------------------ running passes
+
+// One engine launch over the tasks of class K: n_tasks of them, counted on the host, or -- n_tasks_dev set -- as many as
+// the device has counted there for class `cls` of class_active, n_tasks being an upper bound.  ck: the checkpoint buffer
+// of a launch that leaves checkpoint records, else nullptr.
+struct EngineLaunch { DpLaunch L; int widx; uint32_t grid; size_t smem; };      // widx -1: dp_wide_kernel
+int engine_launch(fxg_ctx* c, Worker& w, Pool const& pool, ClassDef const& K, const DpTask* tasks, DpResult* results, uint32_t* ck, uint32_t n_tasks,
+                  const uint32_t* n_tasks_dev, const uint32_t* class_active, uint32_t cls, EngineLaunch& X) {
+    bool const wide = K.G == kWideG;
+    uint32_t const tpw = wide ? 1u : 32u / K.G;
+    DpLaunch& L = X.L;
+    L = DpLaunch{};
+    L.tasks = tasks; L.n_tasks = n_tasks; L.n_tasks_dev = n_tasks_dev; L.class_active = class_active; L.cls = cls;
+    L.group = K.G; L.win_stride = kWinBytes; L.two = 2;
+    L.peq_stride = peq_stride_for(K.max_words);
+    L.ref_packed = c->refs.packed.as<uint32_t>(); L.ref_chunks = c->refs.total / 32 + 1;
+    // (read only for tasks flagged kFlagInlineRef: fxg_align_batch's against inline references; the device builds none)
+    L.inline_packed = pool.inline_packed.as<uint32_t>(); L.inline_chunks = pool.inline_len / 32 + 1;
+    L.peq_table = pool.peq.as<uint32_t>(); L.peq_plane_words = pool.plane_words;
+    L.results = results; L.trace = ck;
+    X.widx = wide ? -1 : int(K.widx);
+    X.smem = engine_smem_bytes(K.G, K.max_words);
+    if (X.smem > c->smem_limit) return fail(w.err, FXG_ERR_INVALID_ARGUMENT, "internal: launch needs %zu bytes of shared memory", X.smem);
+    if (n_tasks_dev)        // (no more CTAs than a few waves of the machine: the CTAs take the task groups in turn)
+        X.grid = uint32_t(std::min<size_t>((size_t(n_tasks) + tpw - 1) / tpw, size_t(c->num_sms) * (wide ? 2 : 32)));
+    else
+        X.grid = wide ? uint32_t(std::min<size_t>(n_tasks, size_t(c->num_sms) * 2)) : (n_tasks + tpw - 1) / tpw;
+    return FXG_OK;
+}
+
+// The tracebacks of n_tasks alignments whose score passes left their checkpoint records in ck; they write to the
+// worker's cigar buffer and traceback results.
+Walk2Launch walk_launch(fxg_ctx* c, Worker& w, Pool const& pool, const uint32_t* ck, const Walk2Task* tasks, uint32_t n_tasks) {
+    Walk2Launch WL{};
+    WL.tasks = tasks; WL.n_tasks = n_tasks; WL.ck = ck;
+    // (read only for tasks flagged kFlagInlineRef: fxg_align_batch's against inline references; the device builds none)
+    WL.ref_packed = c->refs.packed.as<uint32_t>(); WL.inline_packed = pool.inline_packed.as<uint32_t>();
+    WL.peq_table = pool.peq.as<uint32_t>(); WL.peq_plane_words = pool.plane_words;
+    WL.cigars = w.d_cigars.as<uint32_t>(); WL.results = w.d_wresults.as<WalkResult>(); WL.two = 2;
+    return WL;
+}
 
 // Runs `passes` on the worker's streams: plain score passes, or (ck_bases != nullptr) score passes that leave checkpoint
 // records at those offsets of the worker's checkpoint buffer.
@@ -788,7 +848,7 @@ int run_passes(fxg_ctx* c, Worker& w, Pool const& pool, std::vector<Pass> const&
     g_prof.lap(w, 5);
 
     CUDA_TRY(w.err, cudaEventRecord(w.ev0, w.stream));
-    struct Launch { DpLaunch L; int widx; uint32_t grid; size_t smem; uint64_t work, word_steps; };
+    struct Launch { EngineLaunch E; uint64_t work, word_steps; };
     std::vector<Launch> launches;
     size_t i = 0;
     while (i < N) {
@@ -796,8 +856,7 @@ int run_passes(fxg_ctx* c, Worker& w, Pool const& pool, std::vector<Pass> const&
         Config const& c0 = w.cfgs[uint32_t(w.keys[i])];
         int const widx = c0.widx; uint32_t const G = c0.G;
         uint32_t const W = uint32_t(kWidths[widx]);
-        bool const wide = G == kWideG;
-        uint32_t const tpw = wide ? 1 : 32 / G;
+        uint32_t const tpw = G == kWideG ? 1 : 32 / G;
         size_t j = i;
         uint32_t max_words = 0;
         uint64_t work = 0, ws = 0;
@@ -811,47 +870,27 @@ int run_passes(fxg_ctx* c, Worker& w, Pool const& pool, std::vector<Pass> const&
             ++j;
         }
         Launch X{};
-        DpLaunch& L = X.L;
-        L.tasks = w.d_tasks.as<DpTask>() + i;
-        L.n_tasks = uint32_t(j - i);
-        L.group = G;
-        L.win_stride = kWinBytes; L.two = 2;
-        L.ref_chunks = c->refs.total / 32 + 1; L.inline_chunks = pool.inline_len / 32 + 1;
-        L.peq_stride = peq_stride_for(max_words);
-        L.ref_packed = c->refs.packed.as<uint32_t>();
-        L.inline_packed = pool.inline_packed.as<uint32_t>();
-        L.peq_table = pool.peq.as<uint32_t>();
-        L.peq_plane_words = pool.plane_words;
-        L.results = w.d_results.as<DpResult>();
-        L.trace = ck_buffer;
-        X.smem = wide ? wide_smem_bytes() : size_t(tpw) * (kWinBytes + size_t(kNumSymbols) * L.peq_stride * 4);
-        if (X.smem > c->smem_limit) return fail(w.err, FXG_ERR_INVALID_ARGUMENT, "internal: launch needs %zu bytes of shared memory", X.smem);
-        X.grid = wide ? uint32_t(std::min<size_t>(L.n_tasks, size_t(c->num_sms) * 2)) : uint32_t((L.n_tasks + tpw - 1) / tpw);
-        X.widx = wide ? -1 : widx; X.work = work / tpw; X.word_steps = ws;
+        int const rc = engine_launch(c, w, pool, ClassDef{uint8_t(widx), uint8_t(G), max_words}, w.d_tasks.as<DpTask>() + i, w.d_results.as<DpResult>(),
+                                     ck_buffer, uint32_t(j - i), nullptr, nullptr, 0, X.E);
+        if (rc != FXG_OK) return rc;
+        X.work = work / tpw; X.word_steps = ws;
         launches.push_back(X);
         i = j;
     }
     // largest first on the worker's own stream, the rest spread over the side streams so that they fill the machine together
     std::sort(launches.begin(), launches.end(), [](Launch const& a, Launch const& b) { return a.work > b.work; });
-    bool const fan_out = launches.size() > 1;
-    if (fan_out) {
-        CUDA_TRY(w.err, cudaEventRecord(w.ev_fork, w.stream));
-        for (int q = 0; q < Worker::kSide; ++q) CUDA_TRY(w.err, cudaStreamWaitEvent(w.side[q], w.ev_fork, 0));
-    }
-    for (size_t q = 0; q < launches.size(); ++q) {
-        Launch const& X = launches[q];
-        cudaStream_t const st = q == 0 ? w.stream : w.side[(q - 1) % Worker::kSide];
+    int const n_launch = int(launches.size());
+    CUDA_TRY(w.err, w.fork(w.stream, n_launch));
+    for (int q = 0; q < n_launch; ++q) {
+        EngineLaunch const& X = launches[q].E;
+        cudaStream_t st;
+        CUDA_TRY(w.err, w.fan_stream(w.stream, q, st));
         if (q == 0 && trace) CUDA_TRY(w.err, cudaEventRecord(w.ev_b0, w.stream));
         CUDA_TRY(w.err, launch_dp(X.widx, trace, X.L, X.grid, X.smem, st));
         if (q == 0 && trace) CUDA_TRY(w.err, cudaEventRecord(w.ev_b1, w.stream));
         w.ctr.kernel_launches++;
     }
-    if (fan_out) {
-        for (int q = 0; q < Worker::kSide; ++q) {
-            CUDA_TRY(w.err, cudaEventRecord(w.ev_join[q], w.side[q]));
-            CUDA_TRY(w.err, cudaStreamWaitEvent(w.stream, w.ev_join[q], 0));
-        }
-    }
+    CUDA_TRY(w.err, w.join(w.stream, n_launch));
     CUDA_TRY(w.err, cudaEventRecord(w.ev1, w.stream));
     g_prof.lap(w, 6);
     CUDA_TRY(w.err, cudaMemcpyAsync(w.h_results.p, w.d_results.p, N * sizeof(DpResult), cudaMemcpyDeviceToHost, w.stream));
@@ -1185,34 +1224,21 @@ int run_root_passes(fxg_ctx* c, Worker& w, Pool const& pool, std::vector<Pass> c
             if (!walk_timed) { CUDA_TRY(w.err, cudaEventRecord(w.ev_w0, ws)); walk_timed = true; }
             // every traceback is one long chain of dependent steps, so launches of different block widths must not queue
             // behind each other: the first runs on the chunk's stream, the others fork onto side streams and join it again
-            CUDA_TRY(w.err, cudaEventRecord(w.ev_fork, ws));
-            size_t h0 = H0;
             int n_launch = 0;
-            while (h0 < H) {
+            for (size_t h = H0; h < H; ++h) n_launch += h == H0 || hit_widx[h] != hit_widx[h - 1];
+            CUDA_TRY(w.err, w.fork(ws, n_launch));
+            size_t h0 = H0;
+            for (int q = 0; q < n_launch; ++q) {
                 int const widx = hit_widx[h0];
                 size_t h1 = h0;
                 while (h1 < H && hit_widx[h1] == widx) ++h1;
-                Walk2Launch WL{};
-                WL.tasks = w.d_wtasks.as<Walk2Task>() + h0; WL.n_tasks = uint32_t(h1 - h0); WL.ck = ckb.as<uint32_t>();
-                WL.ref_packed = c->refs.packed.as<uint32_t>(); WL.inline_packed = pool.inline_packed.as<uint32_t>();
-                WL.peq_table = pool.peq.as<uint32_t>(); WL.peq_plane_words = pool.plane_words;
-                WL.query_pool = pool.bytes.as<uint8_t>(); WL.cigars = w.d_cigars.as<uint32_t>();
-                WL.results = w.d_wresults.as<WalkResult>(); WL.two = 2;
-                cudaStream_t st = ws;
-                if (n_launch > 0) {
-                    st = w.side[(n_launch - 1) % Worker::kSide];
-                    CUDA_TRY(w.err, cudaStreamWaitEvent(st, w.ev_fork, 0));
-                }
-                CUDA_TRY(w.err, launch_walk(widx, WL, st));
-                if (n_launch > 0) {
-                    int const sq = (n_launch - 1) % Worker::kSide;
-                    CUDA_TRY(w.err, cudaEventRecord(w.ev_join[sq], st));
-                    CUDA_TRY(w.err, cudaStreamWaitEvent(ws, w.ev_join[sq], 0));
-                }
+                cudaStream_t st;
+                CUDA_TRY(w.err, w.fan_stream(ws, q, st));
+                CUDA_TRY(w.err, launch_walk(widx, walk_launch(c, w, pool, ckb.as<uint32_t>(), w.d_wtasks.as<Walk2Task>() + h0, uint32_t(h1 - h0)), st));
                 w.ctr.kernel_launches++;
-                ++n_launch;
                 h0 = h1;
             }
+            CUDA_TRY(w.err, w.join(ws, n_launch));
             CUDA_TRY(w.err, cudaMemcpyAsync(wr + H0, w.d_wresults.as<WalkResult>() + H0, (H - H0) * sizeof(WalkResult), cudaMemcpyDeviceToHost, ws));
             w.ctr.d2h_bytes += (H - H0) * sizeof(WalkResult);
         }
@@ -1917,36 +1943,21 @@ int root_level_device(fxg_ctx* c, Worker& w, Batch& B, uint32_t r0, uint32_t n_r
         std::sort(order, order + n_used, [&](int a, int b) { return class_units[a] > class_units[b]; });
         uint32_t prefix[kMaxLevelClasses + 1] = {0};
         for (int ci = 0; ci < kMaxLevelClasses; ++ci) prefix[ci + 1] = prefix[ci] + class_units[ci];
-        if (n_used > 1) {
-            CUDA_TRY(w.err, cudaEventRecord(w.ev_fork, st));
-            for (int q = 0; q < std::min(n_used - 1, int(Worker::kSide)); ++q) CUDA_TRY(w.err, cudaStreamWaitEvent(w.side[q], w.ev_fork, 0));
-        }
+        CUDA_TRY(w.err, w.fork(st, n_used));
         for (int x = 0; x < n_used; ++x) {
             int const ci = order[x];
-            ClassDef const& K = classes[ci];
-            bool const wide = K.G == kWideG;
-            uint32_t const tpw = wide ? 1u : 32u / K.G;
-            DpLaunch L{};
-            L.tasks = C.tasks + prefix[ci]; L.n_tasks = class_units[ci];
-            L.group = K.G; L.win_stride = kWinBytes; L.two = 2;
-            L.ref_chunks = c->refs.total / 32 + 1; L.inline_chunks = 1;
-            L.peq_stride = peq_stride_for(K.max_words);
-            L.ref_packed = c->refs.packed.as<uint32_t>(); L.inline_packed = nullptr;
-            L.peq_table = pool.peq.as<uint32_t>(); L.peq_plane_words = pool.plane_words;
-            L.results = w.d_results.as<DpResult>(); L.trace = ckb.as<uint32_t>();
-            size_t const smem = wide ? wide_smem_bytes() : size_t(tpw) * (kWinBytes + size_t(kNumSymbols) * L.peq_stride * 4);
-            if (smem > c->smem_limit) return fail(w.err, FXG_ERR_INVALID_ARGUMENT, "internal: launch needs %zu bytes of shared memory", smem);
-            uint32_t const lgrid = wide ? uint32_t(std::min<size_t>(L.n_tasks, size_t(c->num_sms) * 2)) : (L.n_tasks + tpw - 1) / tpw;
-            cudaStream_t const s2 = x == 0 ? st : w.side[(x - 1) % Worker::kSide];
+            EngineLaunch X;
+            rc = engine_launch(c, w, pool, classes[ci], C.tasks + prefix[ci], w.d_results.as<DpResult>(), want_cigar ? ckb.as<uint32_t>() : nullptr,
+                               class_units[ci], nullptr, nullptr, 0, X);
+            if (rc != FXG_OK) return rc;
+            cudaStream_t s2;
+            CUDA_TRY(w.err, w.fan_stream(st, x, s2));
             if (x == 0) { timed_class = ci; CUDA_TRY(w.err, cudaEventRecord(w.ev_b0, st)); }
-            CUDA_TRY(w.err, launch_dp(wide ? -1 : int(K.widx), want_cigar, L, lgrid, smem, s2));
+            CUDA_TRY(w.err, launch_dp(X.widx, want_cigar, X.L, X.grid, X.smem, s2));
             if (x == 0) CUDA_TRY(w.err, cudaEventRecord(w.ev_b1, st));
             w.ctr.kernel_launches++;
         }
-        for (int q = 0; q < std::min(n_used - 1, int(Worker::kSide)); ++q) {
-            CUDA_TRY(w.err, cudaEventRecord(w.ev_join[q], w.side[q]));
-            CUDA_TRY(w.err, cudaStreamWaitEvent(st, w.ev_join[q], 0));
-        }
+        CUDA_TRY(w.err, w.join(st, n_used));
     }
     // ---- every member's result; which alignments share a traceback ----
     root_results_kernel<<<grid, 256, 0, st>>>(C);
@@ -1990,29 +2001,18 @@ int root_level_device(fxg_ctx* c, Worker& w, Batch& B, uint32_t r0, uint32_t n_r
         CUDA_TRY(w.err, cudaGetLastError());
         w.ctr.kernel_launches++;
         uint32_t width_tb[6], wprefix[7] = {0};
-        for (int wi = 0; wi < 6; ++wi) { width_tb[wi] = ctr[kCtrWidthTb + wi]; wprefix[wi + 1] = wprefix[wi] + width_tb[wi]; }
-        CUDA_TRY(w.err, cudaEventRecord(w.ev_w0, st));
-        CUDA_TRY(w.err, cudaEventRecord(w.ev_fork, st));
         int n_launch = 0;
-        for (int wi = 0; wi < 6; ++wi) {
+        for (int wi = 0; wi < 6; ++wi) { width_tb[wi] = ctr[kCtrWidthTb + wi]; wprefix[wi + 1] = wprefix[wi] + width_tb[wi]; n_launch += width_tb[wi] != 0; }
+        CUDA_TRY(w.err, cudaEventRecord(w.ev_w0, st));
+        CUDA_TRY(w.err, w.fork(st, n_launch));
+        for (int wi = 0, q = 0; wi < 6; ++wi) {
             if (!width_tb[wi]) continue;
-            Walk2Launch WL{};
-            WL.tasks = C.wtasks + wprefix[wi]; WL.n_tasks = width_tb[wi]; WL.ck = ckb.as<uint32_t>();
-            WL.ref_packed = c->refs.packed.as<uint32_t>(); WL.inline_packed = nullptr;
-            WL.peq_table = pool.peq.as<uint32_t>(); WL.peq_plane_words = pool.plane_words;
-            WL.query_pool = nullptr; WL.cigars = w.d_cigars.as<uint32_t>();
-            WL.results = w.d_wresults.as<WalkResult>(); WL.two = 2;
-            cudaStream_t s2 = st;
-            if (n_launch > 0) { s2 = w.side[(n_launch - 1) % Worker::kSide]; CUDA_TRY(w.err, cudaStreamWaitEvent(s2, w.ev_fork, 0)); }
-            CUDA_TRY(w.err, launch_walk(wi, WL, s2));
-            if (n_launch > 0) {
-                int const sq = (n_launch - 1) % Worker::kSide;
-                CUDA_TRY(w.err, cudaEventRecord(w.ev_join[sq], s2));
-                CUDA_TRY(w.err, cudaStreamWaitEvent(st, w.ev_join[sq], 0));
-            }
+            cudaStream_t s2;
+            CUDA_TRY(w.err, w.fan_stream(st, q++, s2));
+            CUDA_TRY(w.err, launch_walk(wi, walk_launch(c, w, pool, ckb.as<uint32_t>(), C.wtasks + wprefix[wi], width_tb[wi]), s2));
             w.ctr.kernel_launches++;
-            ++n_launch;
         }
+        CUDA_TRY(w.err, w.join(st, n_launch));
         CUDA_TRY(w.err, cudaEventRecord(w.ev_w1[0], st));
     }
     // ---- alignment records in anchor order ----
@@ -2160,39 +2160,20 @@ int run_device_walks(fxg_ctx* c, Worker& w, Batch& B, uint32_t r0, uint32_t r1, 
     Pool const& pool = *B.pool;
     auto engine = [&](uint32_t mask) -> int {
         // the classes of a level are independent: the first on the worker's stream, the others beside it
-        int n_launch = 0;
-        bool forked = false;
-        for (int ci = 0; ci < n_cls; ++ci) {
+        int const n_launch = __builtin_popcount(mask);           // (mask names classes below n_cls only: checked above)
+        CUDA_TRY(w.err, w.fork(st, n_launch));
+        for (int ci = 0, q = 0; ci < n_cls; ++ci) {
             if (!(mask >> ci & 1u)) continue;
-            ClassDef const& K = classes[ci];
-            bool const wide = K.G == kWideG;
-            uint32_t const tpw = wide ? 1u : 32u / K.G;
-            DpLaunch L{};
-            L.tasks = C.tasks; L.n_tasks = n_walks; L.n_tasks_dev = C.counts + ci; L.class_active = C.class_active; L.cls = uint32_t(ci);
-            L.group = K.G; L.win_stride = kWinBytes; L.two = 2;
-            L.ref_chunks = c->refs.total / 32 + 1; L.inline_chunks = 1;
-            L.peq_stride = peq_stride_for(K.max_words);
-            L.ref_packed = c->refs.packed.as<uint32_t>(); L.inline_packed = nullptr;
-            L.peq_table = pool.peq.as<uint32_t>(); L.peq_plane_words = pool.plane_words;
-            L.results = reinterpret_cast<DpResult*>(D + o_results); L.trace = nullptr;
-            size_t const smem = wide ? wide_smem_bytes() : size_t(tpw) * (kWinBytes + size_t(kNumSymbols) * L.peq_stride * 4);
-            if (smem > c->smem_limit) return fail(w.err, FXG_ERR_INVALID_ARGUMENT, "internal: launch needs %zu bytes of shared memory", smem);
-            cudaStream_t s2 = st;
-            if (n_launch > 0) {
-                if (!forked) { CUDA_TRY(w.err, cudaEventRecord(w.ev_fork, st)); forked = true; }
-                s2 = w.side[(n_launch - 1) % Worker::kSide];
-                if (n_launch <= Worker::kSide) CUDA_TRY(w.err, cudaStreamWaitEvent(s2, w.ev_fork, 0));
-            }
-            // (no more CTAs than a few waves of the machine: the CTAs take the task groups in turn)
-            uint32_t const grid = uint32_t(std::min<size_t>((size_t(n_walks) + tpw - 1) / tpw, size_t(c->num_sms) * (wide ? 2 : 32)));
-            CUDA_TRY(w.err, launch_dp(wide ? -1 : int(K.widx), false, L, grid, smem, s2));
+            EngineLaunch X;
+            int const rc = engine_launch(c, w, pool, classes[ci], C.tasks, reinterpret_cast<DpResult*>(D + o_results), nullptr, n_walks, C.counts + ci,
+                                         C.class_active, uint32_t(ci), X);
+            if (rc != FXG_OK) return rc;
+            cudaStream_t s2;
+            CUDA_TRY(w.err, w.fan_stream(st, q++, s2));
+            CUDA_TRY(w.err, launch_dp(X.widx, false, X.L, X.grid, X.smem, s2));
             w.ctr.kernel_launches++;
-            ++n_launch;
         }
-        for (int q = 0; q < std::min(n_launch - 1, int(Worker::kSide)); ++q) {
-            CUDA_TRY(w.err, cudaEventRecord(w.ev_join[q], w.side[q]));
-            CUDA_TRY(w.err, cudaStreamWaitEvent(st, w.ev_join[q], 0));
-        }
+        CUDA_TRY(w.err, w.join(st, n_launch));
         return FXG_OK;
     };
     g_prof.lap(w, 2);
