@@ -7,7 +7,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SOURCES = [os.path.join(HERE, "csrc", f) for f in ("floxer_gpu.cu", "pex_tree.cpp", "sam_output.cpp", "bam_output.cpp", "seeder.cpp")]
-HEADERS = [os.path.join(HERE, "csrc", "bam_kernels.cuh"), os.path.join(HERE, "csrc", "dp_kernels.cuh"), os.path.join(HERE, "csrc", "root_kernels.cuh"), os.path.join(HERE, "csrc", "seed_kernels.cuh"), os.path.join(os.path.dirname(HERE), "include", "floxer_gpu.h")]
+HEADERS = [os.path.join(HERE, "csrc", "bam_kernels.cuh"), os.path.join(HERE, "csrc", "dp_kernels.cuh"), os.path.join(HERE, "csrc", "root_kernels.cuh"), os.path.join(HERE, "csrc", "sam_kernels.cuh"), os.path.join(HERE, "csrc", "seed_kernels.cuh"), os.path.join(os.path.dirname(HERE), "include", "floxer_gpu.h")]
 OUTPUT = os.path.join(HERE, "libfloxer_gpu.so")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -84,6 +84,28 @@ __device__ __forceinline__ void put_le(uint8_t* p, uint32_t v, int n) { for (int
 
 // ------------------------------------------------------------------------------------------------ records
 
+// The record order of one read, for a whole warp (every lane calls emit(k, a, slot, primary) for k = 0 .. n_al-1):
+// slot is alignment k's place in the stable order of the read's alignments by reference id, primary tells whether it
+// is the first in that order with the read's fewest errors (output.cpp:57-67).  The SAM and BAM writers share it.
+template <class Emit>
+__device__ __forceinline__ void for_each_record_in_order(const fxg_alignment* al, uint32_t n_al, uint32_t lane, Emit&& emit) {
+    unsigned long long best = ~0ull;
+    for (uint32_t k = lane; k < n_al; k += 32) best = min(best, (unsigned long long)al[k].num_errors);
+    best = warp_min_u64(best);
+    unsigned long long primary = ~0ull;                                // (reference id, index) of the primary
+    for (uint32_t k = lane; k < n_al; k += 32)
+        if (al[k].num_errors == best) primary = min(primary, (unsigned long long)(uint64_t(al[k].reference_id) << 32 | k));
+    primary = warp_min_u64(primary);
+    for (uint32_t k = 0; k < n_al; ++k) {
+        fxg_alignment const a = al[k];
+        unsigned long long before = 0;
+        for (uint32_t j = lane; j < n_al; j += 32)
+            before += al[j].reference_id < a.reference_id || (al[j].reference_id == a.reference_id && j < k);
+        before = warp_sum_u64(before);
+        emit(k, a, uint32_t(before), (uint64_t(a.reference_id) << 32 | k) == primary);
+    }
+}
+
 __global__ void bam_size_kernel(BamArgs A) {
     uint32_t const r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     uint32_t const lane = threadIdx.x & 31;
@@ -97,16 +119,7 @@ __global__ void bam_size_kernel(BamArgs A) {
         }
         return;
     }
-    const fxg_alignment* const al = A.al + R.al0;
-    unsigned long long best = ~0ull;
-    for (uint32_t k = lane; k < R.n_al; k += 32) best = min(best, (unsigned long long)al[k].num_errors);
-    best = warp_min_u64(best);
-    unsigned long long primary = ~0ull;                                // (reference id, index) of the primary
-    for (uint32_t k = lane; k < R.n_al; k += 32)
-        if (al[k].num_errors == best) primary = min(primary, (unsigned long long)(uint64_t(al[k].reference_id) << 32 | k));
-    primary = warp_min_u64(primary);
-    for (uint32_t k = 0; k < R.n_al; ++k) {
-        fxg_alignment const a = al[k];
+    for_each_record_in_order(A.al + R.al0, R.n_al, lane, [&](uint32_t k, fxg_alignment const& a, uint32_t before, bool is_primary) {
         const uint32_t* const ops = A.cigars + (a.cigar_offset - A.cigar_lo);
         unsigned long long qs = 0, rs = 0;
         for (uint32_t i = lane; i < a.cigar_len; i += 32) {
@@ -115,22 +128,17 @@ __global__ void bam_size_kernel(BamArgs A) {
             if (op == FXG_CIGAR_I || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) qs += n;
         }
         qs = warp_sum_u64(qs); rs = warp_sum_u64(rs);
-        unsigned long long before = 0;                                        // its place in the stable order by reference id
-        for (uint32_t j = lane; j < R.n_al; j += 32)
-            before += al[j].reference_id < a.reference_id || (al[j].reference_id == a.reference_id && j < k);
-        before = warp_sum_u64(before);
         if (lane == 0) {
-            bool const is_primary = (uint64_t(a.reference_id) << 32 | k) == primary;
             bool const long_cigar = a.cigar_len > 65535;
             uint32_t const flag = (a.orientation == FXG_REVERSE_COMPLEMENT ? 16u : 0u) | (is_primary ? 0u : 256u);
             uint64_t size = 36 + R.l_name + 4 * uint64_t(long_cigar ? 2 : a.cigar_len) + bam_nm_bytes(a.num_errors);
             if (is_primary) size += seq_bytes;
             if (long_cigar) size += 8 + 4 * uint64_t(a.cigar_len);
-            uint32_t const slot = R.rec0 + uint32_t(before);
+            uint32_t const slot = R.rec0 + before;
             A.recs[slot] = BamRecord{qs, rs, r, R.al0 + k, flag, is_primary ? R.l_seq : 0u};
             A.rec_off[slot] = size;
         }
-    }
+    });
 }
 
 __global__ void bam_write_kernel(BamArgs A, uint32_t n_rec) {

@@ -13,6 +13,7 @@
 #include "bam_kernels.cuh"
 #include "dp_kernels.cuh"
 #include "root_kernels.cuh"
+#include "sam_kernels.cuh"
 #include "seed_kernels.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -4149,6 +4150,55 @@ static_assert(sizeof(DeflateSmem) <= 227 * 1024, "the deflate kernel's shared me
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// The BGZF image of the raw stream raw[0, raw_len) (raw_len > 0) in device memory, on K's stream: deflate per 0xff00-byte
+// chunk, block offsets, assembly, and the image copied to the start of K.host (img_len bytes).  Uses K.bufs[4] (scan
+// temporary) and K.bufs[6..11]; h_word is a page-locked word for the length's read-back.
+int bgzf_image_on_device(SeedCall& K, const uint8_t* raw, uint64_t raw_len, uint64_t* h_word, uint64_t& d2h, uint64_t& launches,
+                         size_t& img_len, std::string& err) {
+    cudaStream_t const s = K.st;
+    DevBuf &d_tmp = K.bufs[4], &d_work = K.bufs[6], &d_slots = K.bufs[7], &d_info = K.bufs[8], &d_bsize = K.bufs[9], &d_boff = K.bufs[10],
+           &d_img = K.bufs[11];
+    uint32_t const n_chunks = uint32_t((raw_len + kBgzfChunk - 1) / kBgzfChunk);
+    CUDA_TRY(err, d_work.ensure(raw_len * 4));
+    CUDA_TRY(err, d_slots.ensure(size_t(n_chunks) * kBgzfSlotWords * 4));
+    CUDA_TRY(err, d_info.ensure(size_t(n_chunks) * sizeof(BgzfBlockInfo)));
+    CUDA_TRY(err, d_bsize.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, d_boff.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, cudaFuncSetAttribute(bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(DeflateSmem))));
+    bgzf_deflate_kernel<<<n_chunks, kDeflateThreads, sizeof(DeflateSmem), s>>>(raw, raw_len, d_work.as<uint32_t>(), d_slots.as<uint32_t>(),
+                                                                              d_info.as<BgzfBlockInfo>(), d_bsize.as<uint64_t>(), n_chunks);
+    CUDA_TRY(err, cudaGetLastError());
+    size_t tmp_bytes = 0;
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
+    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
+    // (the image is at most the raw stream stored, plus framing)
+    CUDA_TRY(err, d_img.ensure(raw_len + (uint64_t(n_chunks) + 1) * 31 + 28));
+    bgzf_assemble_kernel<<<n_chunks + 1, 256, 0, s>>>(raw, d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(), d_boff.as<uint64_t>(),
+                                                      n_chunks, d_img.as<uint8_t>());
+    CUDA_TRY(err, cudaGetLastError());
+    launches += 2;
+    CUDA_TRY(err, cudaMemcpyAsync(h_word, d_boff.as<uint64_t>() + n_chunks + 1, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    d2h += 8;
+    img_len = size_t(h_word[0]);
+    CUDA_TRY(err, K.host.ensure(img_len));
+    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_img.p, img_len, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    d2h += img_len;
+    return FXG_OK;
+}
+
+// a malloc'ed copy of n bytes (and a NUL behind them) for the caller
+int hand_out(const void* src, size_t n, uint8_t** bytes, size_t* bytes_len) {
+    uint8_t* buf = static_cast<uint8_t*>(std::malloc(n + 1));
+    if (!buf) return FXG_ERR_OUT_OF_MEMORY;
+    if (n) std::memcpy(buf, src, n);
+    buf[n] = 0;
+    *bytes = buf; *bytes_len = n;
+    return FXG_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -4197,8 +4247,7 @@ int fxg_write_bam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const
         if (B.qual != ~uint64_t(0)) std::memcpy(h + o_quals + B.qual, queries[ri].quality, B.l_seq);
     }
     std::memcpy(h + o_header, P.header.data(), P.header.size());
-    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_raw = K.bufs[5],
-           &d_work = K.bufs[6], &d_slots = K.bufs[7], &d_info = K.bufs[8], &d_bsize = K.bufs[9], &d_boff = K.bufs[10], &d_img = K.bufs[11];
+    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_raw = K.bufs[5];
     CUDA_TRY(err, d_in.ensure(up));
     CUDA_TRY(err, cudaMemcpyAsync(d_in.p, h, up, cudaMemcpyHostToDevice, s));
     uint64_t h2d = up, d2h = 0, launches = 0;
@@ -4232,7 +4281,6 @@ int fxg_write_bam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const
         body = h_word[0];
     }
     uint64_t const raw_len = P.header.size() + body;
-    uint32_t const n_chunks = uint32_t((raw_len + kBgzfChunk - 1) / kBgzfChunk);
 
     // ---- the raw stream: the header, then the records ----
     CUDA_TRY(err, d_raw.ensure(raw_len + 16));
@@ -4244,35 +4292,9 @@ int fxg_write_bam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const
         ++launches;
     }
 
-    // ---- BGZF blocks: deflate per chunk, block offsets, the image ----
-    CUDA_TRY(err, d_work.ensure(raw_len * 4));
-    CUDA_TRY(err, d_slots.ensure(size_t(n_chunks) * kBgzfSlotWords * 4));
-    CUDA_TRY(err, d_info.ensure(size_t(n_chunks) * sizeof(BgzfBlockInfo)));
-    CUDA_TRY(err, d_bsize.ensure((size_t(n_chunks) + 2) * 8));
-    CUDA_TRY(err, d_boff.ensure((size_t(n_chunks) + 2) * 8));
-    CUDA_TRY(err, cudaFuncSetAttribute(bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(DeflateSmem))));
-    bgzf_deflate_kernel<<<n_chunks, kDeflateThreads, sizeof(DeflateSmem), s>>>(d_raw.as<uint8_t>(), raw_len, d_work.as<uint32_t>(),
-                                                                              d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(),
-                                                                              d_bsize.as<uint64_t>(), n_chunks);
-    CUDA_TRY(err, cudaGetLastError());
-    size_t tmp_bytes = 0;
-    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
-    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
-    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
-    // (the image is at most the raw stream stored, plus framing)
-    CUDA_TRY(err, d_img.ensure(raw_len + (uint64_t(n_chunks) + 1) * 31 + 28));
-    bgzf_assemble_kernel<<<n_chunks + 1, 256, 0, s>>>(d_raw.as<uint8_t>(), d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(),
-                                                      d_boff.as<uint64_t>(), n_chunks, d_img.as<uint8_t>());
-    CUDA_TRY(err, cudaGetLastError());
-    launches += 2;
-    CUDA_TRY(err, cudaMemcpyAsync(h_word, d_boff.as<uint64_t>() + n_chunks + 1, 8, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(err, cudaStreamSynchronize(s));
-    d2h += 8;
-    size_t const img_len = size_t(h_word[0]);
-    CUDA_TRY(err, K.host.ensure(img_len));
-    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_img.p, img_len, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(err, cudaStreamSynchronize(s));
-    d2h += img_len;
+    // ---- BGZF blocks ----
+    size_t img_len = 0;
+    if (int rc = bgzf_image_on_device(K, d_raw.as<uint8_t>(), raw_len, h_word, d2h, launches, img_len, err)) return rc;
     {
         std::lock_guard<std::mutex> lock(c->mu);
         c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
@@ -4291,6 +4313,197 @@ int fxg_job_write_bam_device(fxg_ctx* c, const fxg_job* job, size_t n_references
     if (!job) return FXG_ERR_INVALID_ARGUMENT;
     return fxg_write_bam_device(c, fxg_job_alignments(job), fxg_job_num_alignments(job), fxg_job_cigar_pool(job), n_references, reference_ids,
                                 reference_lengths, reads, n_reads, forward_pool, queries, with_header, bytes, bytes_len);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ SAM on the device
+
+namespace {
+
+// The batch as the SAM kernels read it, and what fxg_write_sam would refuse.  sam_output.cpp walks the reads in order and
+// checks a read's alignments before it moves on to the next read; the first failure it would meet decides the code.
+struct SamPlan {
+    std::vector<SamReadRec> reads;
+    std::vector<uint64_t> ref_off;                         // the reference names, concatenated: n_references + 1 offsets
+    std::string header;                                    // the @HD / @SQ lines (empty without them)
+    uint64_t cigar_lo = UINT64_MAX, cigar_hi = 0, seq_lo = UINT64_MAX, seq_hi = 0, names_len = 0, quals_len = 0;
+    uint64_t n_rec = 0;
+};
+
+int plan_sam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references, const char* const* reference_ids,
+             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const fxg_sam_query* queries, int with_header,
+             SamPlan& P, std::string& err) {
+    P.reads.resize(n_reads);
+    size_t a = 0;
+    for (size_t ri = 0; ri < n_reads; ++ri) {
+        size_t const a0 = a;
+        while (a < n_al && al[a].read_index == ri) ++a;
+        if (a < n_al && al[a].read_index < ri)
+            return fail(err, FXG_ERR_STATE, "alignment %zu (read %u) follows read %zu: alignments must be grouped by read", a, al[a].read_index, ri);
+        for (size_t k = a0; k < a; ++k) {
+            fxg_alignment const& A = al[k];
+            if (A.reference_id >= n_references || (A.cigar_len && !cigar_pool))
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: alignment %zu has a reference id out of range or a CIGAR without a pool", ri, k);
+            if (A.cigar_len) { P.cigar_lo = std::min<uint64_t>(P.cigar_lo, A.cigar_offset); P.cigar_hi = std::max<uint64_t>(P.cigar_hi, A.cigar_offset + A.cigar_len); }
+        }
+        fxg_read const& R = reads[ri];
+        const char* const q = queries[ri].quality;
+        SamReadRec& S = P.reads[ri];
+        S.seq = R.query_offset;
+        S.l_seq = R.query_len;
+        S.name = P.names_len;
+        S.l_name = uint32_t(std::strlen(queries[ri].id ? queries[ri].id : "*"));
+        S.qual = P.quals_len;
+        S.l_qual = q ? uint32_t(std::strlen(q)) : 0u;
+        S.al0 = uint32_t(a0); S.n_al = uint32_t(a - a0);
+        S.rec0 = uint32_t(P.n_rec);
+        P.names_len += S.l_name;
+        P.quals_len += S.l_qual;
+        if (R.query_len) { P.seq_lo = std::min<uint64_t>(P.seq_lo, R.query_offset); P.seq_hi = std::max<uint64_t>(P.seq_hi, R.query_offset + R.query_len); }
+        P.n_rec += std::max<size_t>(a - a0, 1);
+    }
+    if (a != n_al) return fail(err, FXG_ERR_STATE, "alignment %zu names read %u of %zu: alignments must be grouped by read in read order", a, al[a].read_index, n_reads);
+    if (P.n_rec >= (uint64_t(1) << 32) || n_al >= (uint64_t(1) << 32))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "%llu records: split the batch", (unsigned long long)P.n_rec);
+    if (P.seq_lo > P.seq_hi) P.seq_lo = P.seq_hi = 0;
+    if (P.cigar_lo > P.cigar_hi) P.cigar_lo = P.cigar_hi = 0;
+    for (SamReadRec& S : P.reads) S.seq -= std::min(S.seq, P.seq_lo);
+    P.ref_off.resize(n_references + 1);
+    P.ref_off[0] = 0;
+    for (size_t r = 0; r < n_references; ++r) P.ref_off[r + 1] = P.ref_off[r] + std::strlen(reference_ids[r]);
+    if (with_header) {                                     // sam_output.cpp's header, byte for byte
+        P.header = "@HD\tVN:1.6\tSO:unknown\tGO:none\n";
+        for (size_t r = 0; r < n_references; ++r) {
+            P.header += "@SQ\tSN:"; P.header += reference_ids[r]; P.header += "\tLN:"; P.header += std::to_string(reference_lengths[r]); P.header += '\n';
+        }
+    }
+    return FXG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fxg_write_sam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
+                         const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
+                         const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, int bgzf, uint8_t** bytes,
+                         size_t* bytes_len) {
+    std::string err;
+    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_write_sam_device: a required argument is null");
+    *bytes = nullptr; *bytes_len = 0;
+    try {
+    SamPlan P;
+    if (int rc = plan_sam(al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
+    if (P.n_rec == 0 && P.header.empty())                  // no text: the empty string, or nothing but the end-of-file block
+        return bgzf ? hand_out(kBgzfEof, sizeof kBgzfEof, bytes, bytes_len) : hand_out(nullptr, 0, bytes, bytes_len);
+
+    // ---- one upload through page-locked staging: reads, alignments, CIGAR range, forward-pool range, names, qualities,
+    //      reference names and their offsets, header ----
+    size_t const ref_names_len = P.ref_off.back();
+    size_t const o_reads = 0;
+    size_t const o_al = align_up(o_reads + n_reads * sizeof(SamReadRec), 256);
+    size_t const o_cig = align_up(o_al + n_al * sizeof(fxg_alignment), 256);
+    size_t const o_seq = align_up(o_cig + (P.cigar_hi - P.cigar_lo) * 4, 256);
+    size_t const o_names = align_up(o_seq + (P.seq_hi - P.seq_lo), 256);
+    size_t const o_quals = align_up(o_names + P.names_len, 256);
+    size_t const o_refoff = align_up(o_quals + P.quals_len, 256);
+    size_t const o_refnames = align_up(o_refoff + P.ref_off.size() * 8, 256);
+    size_t const o_header = align_up(o_refnames + ref_names_len, 256);
+    size_t const up = align_up(o_header + P.header.size(), 256);
+    CUDA_TRY(err, cudaSetDevice(c->device));
+    SeedCall K{c};
+    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    cudaStream_t const s = K.st;
+    CUDA_TRY(err, K.host.ensure(up + 64));
+    uint8_t* const h = K.host.as<uint8_t>();
+    if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(SamReadRec));
+    if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
+    if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
+    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
+    for (size_t ri = 0; ri < n_reads; ++ri) {
+        SamReadRec const& S = P.reads[ri];
+        std::memcpy(h + o_names + S.name, queries[ri].id ? queries[ri].id : "*", S.l_name);
+        if (S.l_qual) std::memcpy(h + o_quals + S.qual, queries[ri].quality, S.l_qual);
+    }
+    std::memcpy(h + o_refoff, P.ref_off.data(), P.ref_off.size() * 8);
+    for (size_t r = 0; r < n_references; ++r) std::memcpy(h + o_refnames + P.ref_off[r], reference_ids[r], P.ref_off[r + 1] - P.ref_off[r]);
+    std::memcpy(h + o_header, P.header.data(), P.header.size());
+    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_text = K.bufs[5];
+    CUDA_TRY(err, d_in.ensure(up));
+    CUDA_TRY(err, cudaMemcpyAsync(d_in.p, h, up, cudaMemcpyHostToDevice, s));
+    uint64_t h2d = up, d2h = 0, launches = 0;
+    uint8_t* const din = d_in.as<uint8_t>();
+    SamArgs A{};
+    A.reads = reinterpret_cast<const SamReadRec*>(din + o_reads); A.n_reads = uint32_t(n_reads);
+    A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
+    A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
+    A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = reinterpret_cast<const char*>(din + o_quals);
+    A.ref_off = reinterpret_cast<const uint64_t*>(din + o_refoff); A.ref_names = reinterpret_cast<const char*>(din + o_refnames);
+
+    // ---- record lengths, their offsets, the text's length ----
+    uint32_t const n_rec = uint32_t(P.n_rec);
+    uint64_t* const h_word = reinterpret_cast<uint64_t*>(h + up);           // (read-backs go behind the upload)
+    uint64_t body = 0;
+    if (n_rec) {
+        CUDA_TRY(err, d_rec.ensure(size_t(n_rec) * sizeof(SamRecord)));
+        CUDA_TRY(err, d_size.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, d_off.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, cudaMemsetAsync(d_size.as<uint64_t>() + n_rec, 0, 8, s));
+        A.recs = d_rec.as<SamRecord>(); A.rec_off = d_size.as<uint64_t>();
+        sam_size_kernel<<<uint32_t((uint64_t(n_reads) * 32 + 255) / 256), 256, 0, s>>>(A);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+        size_t tmp_bytes = 0;
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_word, d_off.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        d2h += 8;
+        body = h_word[0];
+    }
+    uint64_t const text_len = P.header.size() + body;
+
+    // ---- the text: the header, then the records ----
+    CUDA_TRY(err, d_text.ensure(text_len + 16));
+    if (!P.header.empty()) CUDA_TRY(err, cudaMemcpyAsync(d_text.p, din + o_header, P.header.size(), cudaMemcpyDeviceToDevice, s));
+    A.rec_off = d_off.as<uint64_t>(); A.text = d_text.as<char>(); A.body = P.header.size();
+    if (n_rec) {
+        sam_write_kernel<<<uint32_t((uint64_t(n_rec) * 32 + 255) / 256), 256, 0, s>>>(A, n_rec);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+    }
+
+    // ---- the text as it is, or its BGZF image ----
+    size_t out_len = 0;
+    if (bgzf) {
+        if (int rc = bgzf_image_on_device(K, d_text.as<uint8_t>(), text_len, h_word, d2h, launches, out_len, err)) return rc;
+    } else {
+        out_len = size_t(text_len);
+        CUDA_TRY(err, cudaStreamSynchronize(s));                           // (the upload may still read the staging)
+        CUDA_TRY(err, K.host.ensure(out_len));
+        CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_text.p, out_len, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        d2h += out_len;
+    }
+    {
+        std::lock_guard<std::mutex> lock(c->mu);
+        c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
+    }
+    return hand_out(K.host.p, out_len, bytes, bytes_len);
+    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+}
+
+int fxg_job_write_sam_device(fxg_ctx* c, const fxg_job* job, size_t n_references, const char* const* reference_ids,
+                             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool,
+                             const fxg_sam_query* queries, int with_header, int bgzf, uint8_t** bytes, size_t* bytes_len) {
+    std::string err;
+    if (!job) return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_job_write_sam_device: no job");
+    return fxg_write_sam_device(c, fxg_job_alignments(job), fxg_job_num_alignments(job), fxg_job_cigar_pool(job), n_references, reference_ids,
+                                reference_lengths, reads, n_reads, forward_pool, queries, with_header, bgzf, bytes, bytes_len);
 }
 
 }  // extern "C"

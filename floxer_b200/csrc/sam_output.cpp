@@ -12,6 +12,9 @@
 // and '*' conventions follow the SAM specification, the header line is the one SeqAn3 writes by default as recalled
 // ("@HD VN:1.6 SO:unknown GO:none"); byte-level parity of the text is unpinned, the record contents are pinned by
 // test/floxer_whole_program_via_cli_test.cpp:38-93 (tests/test_sam_output.py).
+//
+// Host-only code: the array entry point fxg_write_sam needs neither a context nor a GPU (tests/test_sam_arrays.py);
+// fxg_write_sam_device (floxer_gpu.cu, sam_kernels.cuh) writes the same text on the device.
 #include "../../include/floxer_gpu.h"
 
 #include <algorithm>
@@ -50,16 +53,13 @@ void append_cigar(std::string& s, const uint32_t* ops, uint32_t n) {
 
 extern "C" {
 
-int fxg_job_write_sam(const fxg_job* job, size_t n_references, const char* const* reference_ids, const uint64_t* reference_lengths,
-                      const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool, const fxg_sam_query* queries,
-                      int with_header, char** text, size_t* text_len) {
-    if (!job || !text || !text_len || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
+int fxg_write_sam(const fxg_alignment* al, size_t n_al, const uint32_t* ops, size_t n_references, const char* const* reference_ids,
+                  const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool,
+                  const fxg_sam_query* queries, int with_header, char** text, size_t* text_len) {
+    if (!text || !text_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
         return FXG_ERR_INVALID_ARGUMENT;
     *text = nullptr; *text_len = 0;
     try {
-    size_t const n_al = fxg_job_num_alignments(job);
-    const fxg_alignment* al = fxg_job_alignments(job);
-    const uint32_t* ops = fxg_job_cigar_pool(job);
     std::string out;
     out.reserve(size_t(1) << 20);
     if (with_header) {
@@ -98,14 +98,14 @@ int fxg_job_write_sam(const fxg_job* job, size_t n_references, const char* const
         bool primary_written = false;
         for (uint32_t k : order) {
             fxg_alignment const& A = al[k];
-            if (A.reference_id >= n_references) return FXG_ERR_INVALID_ARGUMENT;
+            if (A.reference_id >= n_references || (A.cigar_len && !ops)) return FXG_ERR_INVALID_ARGUMENT;
             uint32_t flag = A.orientation == FXG_REVERSE_COMPLEMENT ? 16u : 0u;
             bool const primary = !primary_written && A.num_errors == best;
             if (primary) primary_written = true; else flag |= 256u;
             uint64_t const pos0 = std::min<uint64_t>(A.start_in_reference, uint64_t(std::numeric_limits<int32_t>::max()));   // math.hpp:10-16
             out += qname; out.push_back('\t'); append_uint(out, flag); out.push_back('\t'); out += reference_ids[A.reference_id]; out.push_back('\t');
             append_uint(out, pos0 + 1); out += "\t255\t";
-            append_cigar(out, ops + A.cigar_offset, A.cigar_len);
+            append_cigar(out, A.cigar_len ? ops + A.cigar_offset : nullptr, A.cigar_len);
             out += "\t*\t0\t0\t";
             if (primary) { out += seq; out.push_back('\t'); out += qual; } else out += "*\t*";
             out += "\tNM:i:"; append_uint(out, A.num_errors); out.push_back('\n');
@@ -119,6 +119,14 @@ int fxg_job_write_sam(const fxg_job* job, size_t n_references, const char* const
     *text = buf; *text_len = out.size();
     return FXG_OK;
     } catch (...) { return FXG_ERR_OUT_OF_MEMORY; }              // (std::bad_alloc / length_error of the text buffer: nothing crosses the C ABI)
+}
+
+int fxg_job_write_sam(const fxg_job* job, size_t n_references, const char* const* reference_ids, const uint64_t* reference_lengths,
+                      const fxg_read* reads, size_t n_reads, const uint8_t* forward_pool, const fxg_sam_query* queries,
+                      int with_header, char** text, size_t* text_len) {
+    if (!job) return FXG_ERR_INVALID_ARGUMENT;
+    return fxg_write_sam(fxg_job_alignments(job), fxg_job_num_alignments(job), fxg_job_cigar_pool(job), n_references, reference_ids,
+                         reference_lengths, reads, n_reads, forward_pool, queries, with_header, text, text_len);
 }
 
 void fxg_free(void* p) { std::free(p); }
