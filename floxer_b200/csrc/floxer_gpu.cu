@@ -10,10 +10,10 @@
 // split over one or more host workers with their own CUDA streams and buffers.
 // No CPU fallback exists: every alignment result comes from dp_kernels.cuh.
 #include "../../include/floxer_gpu.h"
-#include "bam_kernels.cuh"
+#include "bgzf_kernels.cuh"
 #include "dp_kernels.cuh"
+#include "record_kernels.cuh"
 #include "root_kernels.cuh"
-#include "sam_kernels.cuh"
 #include "seed_kernels.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -3589,14 +3589,15 @@ struct StoreReader {
     ~StoreReader() { if (on) { std::lock_guard<std::mutex> lock(c->mu); c->seeders_reading--; } }
 };
 
-// a call's own stream and buffers; the stream is drained before the buffers go back to the pool
-struct SeedCall {
-    explicit SeedCall(fxg_ctx* ctx) : c(ctx) {}
+// a call's own stream, device buffers and page-locked staging; the stream is drained before the buffers go back to the
+// pool
+struct CallScratch {
+    explicit CallScratch(fxg_ctx* ctx) : c(ctx) {}
     fxg_ctx* c;
     cudaStream_t st = nullptr;
     DevBuf bufs[20];
     PinnedBuf host;
-    ~SeedCall() {
+    ~CallScratch() {
         if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
         for (DevBuf& b : bufs) b.release();
         if (host.p) { std::lock_guard<std::mutex> lock(c->mu); give_staging(c, host); }
@@ -3698,7 +3699,7 @@ void set_read_anchors(fxg_read* reads, size_t n_reads, std::vector<uint32_t> con
 
 // The device seeder on a planned batch (plan.n_seeds > 0) whose query pools -- forward, then reverse complement -- are at
 // d_pool on the device, on K's stream (which first waits for `pool_ready`, if given).  Returns with the stream drained.
-int seed_batch(fxg_ctx* c, const fxg_gpu_seeder* S, const uint32_t* packed, SeedPlan const& plan, size_t n_reads, SeedCall& K,
+int seed_batch(fxg_ctx* c, const fxg_gpu_seeder* S, const uint32_t* packed, SeedPlan const& plan, size_t n_reads, CallScratch& K,
                const uint8_t* d_pool, uint64_t pool_len, cudaEvent_t pool_ready, uint64_t max_anchors_hard, uint64_t max_anchors_soft,
                int erase_useless_anchors, SeedSink& out, fxg_seed_stats& st, std::string& err) {
     uint32_t const n_seeds = plan.n_seeds;
@@ -3898,7 +3899,7 @@ int fxg_gpu_seeder_create(fxg_ctx* c, uint32_t q, fxg_gpu_seeder** out) {
     if (total >= (uint64_t(1) << 32))
         return fail(err, FXG_ERR_INVALID_ARGUMENT, "the references hold %llu bases: positions are 32-bit, index below 4 Gbp", (unsigned long long)total);
     S->budget = uint64_t(env_int("FXG_SEED_CANDIDATES", 1 << 26, 1, INT32_MAX));
-    SeedCall K{c};
+    CallScratch K{c};
     CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
     size_t const nr = std::max<size_t>(len.size(), 1);
     CUDA_TRY(err, S->ubase.ensure(nr * 8));
@@ -3966,7 +3967,7 @@ int fxg_seed_reads(fxg_ctx* c, const fxg_gpu_seeder* S, fxg_read* reads, size_t 
     SeedSink sink;
     if (plan.n_seeds) {
         CUDA_TRY(err, cudaSetDevice(c->device));
-        SeedCall K{c};
+        CallScratch K{c};
         CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
         DevBuf& d_pool = K.bufs[0];
         CUDA_TRY(err, d_pool.ensure(2 * pool_len + 64));
@@ -4027,7 +4028,7 @@ int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_
         sink.dev_offset = layout.o_anchors;
     }
     if (rc == FXG_OK && plan.n_seeds) {
-        SeedCall K{c};
+        CallScratch K{c};
         if (cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "cannot create a stream");
         if (rc == FXG_OK) rc = seed_batch(c, S, packed, plan, n_reads, K, j->pool.bytes.as<uint8_t>(), pool_len, j->pool_ready, max_anchors_hard,
                                           max_anchors_soft, erase_useless_anchors, sink, st, err);
@@ -4057,23 +4058,25 @@ int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_
 
 }  // extern "C"
 
-// ------------------------------------------------------------------------------------------------ BAM on the device
+// ------------------------------------------------------------------------------------------------ BAM and SAM on the device
 
 namespace {
 
-// The batch as the BAM kernels read it, and what fxg_write_bam would refuse.  bam_output.cpp walks the reads in order,
-// a read's alignments in their stable order by reference id, and checks every record as it appends it; the first
-// failure it would meet decides the code returned here.
-struct BamPlan {
-    std::vector<BamReadRec> reads;
-    std::string header;                                    // the BAM header bytes (empty without it)
+// The batch as the record kernels read it, and what the format's host writer would refuse.  Both host writers walk the
+// reads in order and check a read's alignments before they move on; the first failure they would meet decides the code
+// returned here.  bam_output.cpp meets a read's alignments in their stable order by reference id, sam_output.cpp in
+// index order.
+struct OutPlan {
+    std::vector<OutReadRec> reads;
+    std::vector<uint64_t> ref_off;                         // (SAM) the reference names, concatenated: n_references + 1 offsets
+    std::string header;                                    // the header bytes (empty without it)
     uint64_t cigar_lo = UINT64_MAX, cigar_hi = 0, seq_lo = UINT64_MAX, seq_hi = 0, names_len = 0, quals_len = 0;
     uint64_t n_rec = 0;
 };
 
-int plan_bam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references, const char* const* reference_ids,
-             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const fxg_sam_query* queries, int with_header,
-             BamPlan& P, std::string& err) {
+int plan_output(bool bam, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
+                const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
+                const fxg_sam_query* queries, int with_header, OutPlan& P, std::string& err) {
     P.reads.resize(n_reads);
     size_t a = 0;
     for (size_t ri = 0; ri < n_reads; ++ri) {
@@ -4081,27 +4084,31 @@ int plan_bam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, s
         while (a < n_al && al[a].read_index == ri) ++a;
         if (a < n_al && al[a].read_index < ri)
             return fail(err, FXG_ERR_STATE, "alignment %zu (read %u) follows read %zu: alignments must be grouped by read", a, al[a].read_index, ri);
-        const char* const qname = queries[ri].id ? queries[ri].id : "*";
-        size_t const l_name = std::strlen(qname) + 1;
-        if (a == a0 && l_name > 255) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: the name has %zu characters (254 at most)", ri, l_name - 1);
-        // the first failing alignment in (reference id, index) order
+        size_t const l_name = std::strlen(queries[ri].id ? queries[ri].id : "*") + (bam ? 1 : 0);     // BAM names carry their NUL
+        if (bam && a == a0 && l_name > 255) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: the name has %zu characters (254 at most)", ri, l_name - 1);
+        // (BAM) the first failing alignment in (reference id, index) order
         uint64_t first = UINT64_MAX;
         int code = FXG_OK;
         for (size_t k = a0; k < a; ++k) {
             fxg_alignment const& A = al[k];
-            int e = FXG_OK;
-            if (A.reference_id >= n_references || (A.cigar_len && !cigar_pool) || l_name > 255) e = FXG_ERR_INVALID_ARGUMENT;
-            else if (A.cigar_len > 65535) {
-                int64_t rs = 0, qs = 0;
-                for (uint32_t i = 0; i < A.cigar_len; ++i) {
-                    uint32_t const v = cigar_pool[A.cigar_offset + i], op = v & 15u;
-                    if (op == FXG_CIGAR_D || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) rs += v >> 4;
-                    if (op == FXG_CIGAR_I || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) qs += v >> 4;
+            bool const bad = A.reference_id >= n_references || (A.cigar_len && !cigar_pool);
+            if (!bam && bad)
+                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: alignment %zu has a reference id out of range or a CIGAR without a pool", ri, k);
+            if (bam) {
+                int e = FXG_OK;
+                if (bad || l_name > 255) e = FXG_ERR_INVALID_ARGUMENT;
+                else if (A.cigar_len > 65535) {
+                    int64_t rs = 0, qs = 0;
+                    for (uint32_t i = 0; i < A.cigar_len; ++i) {
+                        uint32_t const v = cigar_pool[A.cigar_offset + i], op = v & 15u;
+                        if (op == FXG_CIGAR_D || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) rs += v >> 4;
+                        if (op == FXG_CIGAR_I || op == FXG_CIGAR_EQ || op == FXG_CIGAR_X) qs += v >> 4;
+                    }
+                    if (qs >= (int64_t(1) << 28) || rs >= (int64_t(1) << 28)) e = FXG_ERR_OVERFLOW;
                 }
-                if (qs >= (int64_t(1) << 28) || rs >= (int64_t(1) << 28)) e = FXG_ERR_OVERFLOW;
+                uint64_t const key = uint64_t(A.reference_id) << 32 | (k - a0);
+                if (e != FXG_OK && key < first) { first = key; code = e; }
             }
-            uint64_t const key = uint64_t(A.reference_id) << 32 | (k - a0);
-            if (e != FXG_OK && key < first) { first = key; code = e; }
             if (A.cigar_len) { P.cigar_lo = std::min<uint64_t>(P.cigar_lo, A.cigar_offset); P.cigar_hi = std::max<uint64_t>(P.cigar_hi, A.cigar_offset + A.cigar_len); }
         }
         if (code == FXG_ERR_OVERFLOW)
@@ -4109,36 +4116,45 @@ int plan_bam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, s
         if (code != FXG_OK) return fail(err, code, "read %zu: a reference id out of range, a CIGAR without a pool or a name of more than 254 characters", ri);
         fxg_read const& R = reads[ri];
         const char* const q = queries[ri].quality;
-        bool const have_qual = q && q[0] && std::strlen(q) == R.query_len;
-        BamReadRec& B = P.reads[ri];
-        B.seq = R.query_offset;
-        B.qual = have_qual ? P.quals_len : ~uint64_t(0);
-        B.l_seq = R.query_len;
-        B.name = uint32_t(P.names_len);
-        B.al0 = uint32_t(a0); B.n_al = uint32_t(a - a0);
-        B.rec0 = uint32_t(P.n_rec); B.l_name = uint32_t(l_name);
-        P.names_len += l_name;
-        if (have_qual) P.quals_len += R.query_len;
+        OutReadRec& O = P.reads[ri];
+        O.seq = R.query_offset;
+        O.name = P.names_len;
+        O.qual = P.quals_len;
+        O.l_seq = R.query_len;
+        O.l_name = uint32_t(l_name);
+        // SAM writes every quality at its own length, BAM only one of exactly query_len characters
+        O.l_qual = !q ? 0u : !bam ? uint32_t(std::strlen(q)) : q[0] && std::strlen(q) == R.query_len ? R.query_len : 0u;
+        O.al0 = uint32_t(a0); O.n_al = uint32_t(a - a0);
+        O.rec0 = uint32_t(P.n_rec);
+        P.names_len += O.l_name;
+        P.quals_len += O.l_qual;
         if (R.query_len) { P.seq_lo = std::min<uint64_t>(P.seq_lo, R.query_offset); P.seq_hi = std::max<uint64_t>(P.seq_hi, R.query_offset + R.query_len); }
         P.n_rec += std::max<size_t>(a - a0, 1);
     }
     if (a != n_al) return fail(err, FXG_ERR_STATE, "alignment %zu names read %u of %zu: alignments must be grouped by read in read order", a, al[a].read_index, n_reads);
-    if (P.n_rec >= (uint64_t(1) << 32) || P.names_len >= (uint64_t(1) << 32))
+    if (P.n_rec >= (uint64_t(1) << 32) || (bam ? P.names_len : uint64_t(n_al)) >= (uint64_t(1) << 32))
         return fail(err, FXG_ERR_INVALID_ARGUMENT, "%llu records: split the batch", (unsigned long long)P.n_rec);
     if (P.seq_lo > P.seq_hi) P.seq_lo = P.seq_hi = 0;
     if (P.cigar_lo > P.cigar_hi) P.cigar_lo = P.cigar_hi = 0;
-    for (BamReadRec& B : P.reads) B.seq -= std::min(B.seq, P.seq_lo);
-    if (with_header) {                                     // bam_output.cpp's header, byte for byte
+    for (OutReadRec& O : P.reads) O.seq -= std::min(O.seq, P.seq_lo);
+    if (!bam) {
+        P.ref_off.resize(n_references + 1);
+        for (size_t r = 0; r < n_references; ++r) P.ref_off[r + 1] = P.ref_off[r] + std::strlen(reference_ids[r]);
+    }
+    if (with_header) {                                     // the host writers' header, byte for byte
         std::string text = "@HD\tVN:1.6\tSO:unknown\tGO:none\n";
         for (size_t r = 0; r < n_references; ++r) { text += "@SQ\tSN:"; text += reference_ids[r]; text += "\tLN:"; text += std::to_string(reference_lengths[r]); text += '\n'; }
-        auto u32 = [&](uint32_t v) { for (int i = 0; i < 4; ++i) P.header += char(uint8_t(v >> (8 * i))); };
-        P.header += "BAM\1";
-        u32(uint32_t(text.size())); P.header += text;
-        u32(uint32_t(n_references));
-        for (size_t r = 0; r < n_references; ++r) {
-            size_t const l = std::strlen(reference_ids[r]) + 1;
-            u32(uint32_t(l)); P.header.append(reference_ids[r], l);
-            u32(uint32_t(std::min<uint64_t>(reference_lengths[r], uint64_t(INT32_MAX))));
+        if (!bam) P.header = std::move(text);
+        else {                                             // BAM: the text inside the binary header
+            auto u32 = [&](uint32_t v) { for (int i = 0; i < 4; ++i) P.header += char(uint8_t(v >> (8 * i))); };
+            P.header += "BAM\1";
+            u32(uint32_t(text.size())); P.header += text;
+            u32(uint32_t(n_references));
+            for (size_t r = 0; r < n_references; ++r) {
+                size_t const l = std::strlen(reference_ids[r]) + 1;
+                u32(uint32_t(l)); P.header.append(reference_ids[r], l);
+                u32(uint32_t(std::min<uint64_t>(reference_lengths[r], uint64_t(INT32_MAX))));
+            }
         }
     }
     return FXG_OK;
@@ -4150,40 +4166,47 @@ static_assert(sizeof(DeflateSmem) <= 227 * 1024, "the deflate kernel's shared me
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// The BGZF image of the raw stream raw[0, raw_len) (raw_len > 0) in device memory, on K's stream: deflate per 0xff00-byte
-// chunk, block offsets, assembly, and the image copied to the start of K.host (img_len bytes).  Uses K.bufs[4] (scan
-// temporary) and K.bufs[6..11]; h_word is a page-locked word for the length's read-back.
-int bgzf_image_on_device(SeedCall& K, const uint8_t* raw, uint64_t raw_len, uint64_t* h_word, uint64_t& d2h, uint64_t& launches,
-                         size_t& img_len, std::string& err) {
+// An output call's scratch: the CallScratch buffers by name, the BGZF tail's apart from the records'
+struct OutScratch : CallScratch {
+    using CallScratch::CallScratch;
+    DevBuf &in = bufs[0], &recs = bufs[1], &sizes = bufs[2], &offs = bufs[3];        // the upload; records, their sizes and offsets
+    DevBuf &scan_tmp = bufs[4], &raw = bufs[5];                                      // cub's temporary; the uncompressed output
+    DevBuf &work = bufs[6], &slots = bufs[7], &info = bufs[8], &bsize = bufs[9], &boff = bufs[10], &img = bufs[11];     // BGZF
+};
+
+// The BGZF image of the uncompressed output K.raw[0, raw_len) (raw_len > 0), on K's stream: deflate per 0xff00-byte
+// chunk, block offsets, assembly, and the image copied to the start of K.host (img_len bytes).  h_word is a page-locked
+// word for the length's read-back.
+int bgzf_image_on_device(OutScratch& K, uint64_t raw_len, uint64_t* h_word, uint64_t& d2h, uint64_t& launches, size_t& img_len,
+                         std::string& err) {
     cudaStream_t const s = K.st;
-    DevBuf &d_tmp = K.bufs[4], &d_work = K.bufs[6], &d_slots = K.bufs[7], &d_info = K.bufs[8], &d_bsize = K.bufs[9], &d_boff = K.bufs[10],
-           &d_img = K.bufs[11];
+    const uint8_t* const raw = K.raw.as<uint8_t>();
     uint32_t const n_chunks = uint32_t((raw_len + kBgzfChunk - 1) / kBgzfChunk);
-    CUDA_TRY(err, d_work.ensure(raw_len * 4));
-    CUDA_TRY(err, d_slots.ensure(size_t(n_chunks) * kBgzfSlotWords * 4));
-    CUDA_TRY(err, d_info.ensure(size_t(n_chunks) * sizeof(BgzfBlockInfo)));
-    CUDA_TRY(err, d_bsize.ensure((size_t(n_chunks) + 2) * 8));
-    CUDA_TRY(err, d_boff.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, K.work.ensure(raw_len * 4));
+    CUDA_TRY(err, K.slots.ensure(size_t(n_chunks) * kBgzfSlotWords * 4));
+    CUDA_TRY(err, K.info.ensure(size_t(n_chunks) * sizeof(BgzfBlockInfo)));
+    CUDA_TRY(err, K.bsize.ensure((size_t(n_chunks) + 2) * 8));
+    CUDA_TRY(err, K.boff.ensure((size_t(n_chunks) + 2) * 8));
     CUDA_TRY(err, cudaFuncSetAttribute(bgzf_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(DeflateSmem))));
-    bgzf_deflate_kernel<<<n_chunks, kDeflateThreads, sizeof(DeflateSmem), s>>>(raw, raw_len, d_work.as<uint32_t>(), d_slots.as<uint32_t>(),
-                                                                              d_info.as<BgzfBlockInfo>(), d_bsize.as<uint64_t>(), n_chunks);
+    bgzf_deflate_kernel<<<n_chunks, kDeflateThreads, sizeof(DeflateSmem), s>>>(raw, raw_len, K.work.as<uint32_t>(), K.slots.as<uint32_t>(),
+                                                                              K.info.as<BgzfBlockInfo>(), K.bsize.as<uint64_t>(), n_chunks);
     CUDA_TRY(err, cudaGetLastError());
     size_t tmp_bytes = 0;
-    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
-    CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
-    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_bsize.as<uint64_t>(), d_boff.as<uint64_t>(), n_chunks + 2, s));
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, K.bsize.as<uint64_t>(), K.boff.as<uint64_t>(), n_chunks + 2, s));
+    CUDA_TRY(err, K.scan_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+    CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(K.scan_tmp.p, tmp_bytes, K.bsize.as<uint64_t>(), K.boff.as<uint64_t>(), n_chunks + 2, s));
     // (the image is at most the raw stream stored, plus framing)
-    CUDA_TRY(err, d_img.ensure(raw_len + (uint64_t(n_chunks) + 1) * 31 + 28));
-    bgzf_assemble_kernel<<<n_chunks + 1, 256, 0, s>>>(raw, d_slots.as<uint32_t>(), d_info.as<BgzfBlockInfo>(), d_boff.as<uint64_t>(),
-                                                      n_chunks, d_img.as<uint8_t>());
+    CUDA_TRY(err, K.img.ensure(raw_len + (uint64_t(n_chunks) + 1) * 31 + 28));
+    bgzf_assemble_kernel<<<n_chunks + 1, 256, 0, s>>>(raw, K.slots.as<uint32_t>(), K.info.as<BgzfBlockInfo>(), K.boff.as<uint64_t>(),
+                                                      n_chunks, K.img.as<uint8_t>());
     CUDA_TRY(err, cudaGetLastError());
     launches += 2;
-    CUDA_TRY(err, cudaMemcpyAsync(h_word, d_boff.as<uint64_t>() + n_chunks + 1, 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaMemcpyAsync(h_word, K.boff.as<uint64_t>() + n_chunks + 1, 8, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(err, cudaStreamSynchronize(s));
     d2h += 8;
     img_len = size_t(h_word[0]);
     CUDA_TRY(err, K.host.ensure(img_len));
-    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_img.p, img_len, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(err, cudaMemcpyAsync(K.host.p, K.img.p, img_len, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(err, cudaStreamSynchronize(s));
     d2h += img_len;
     return FXG_OK;
@@ -4199,6 +4222,115 @@ int hand_out(const void* src, size_t n, uint8_t** bytes, size_t* bytes_len) {
     return FXG_OK;
 }
 
+// fxg_write_bam_device (bam, always bgzf) and fxg_write_sam_device: refusals before any device work, then on a stream of
+// the call's own one upload through page-locked staging, the format's size kernel, the scan of the sizes into offsets,
+// the header and the format's write kernel, and the output as it is or (bgzf) its BGZF image, malloc'ed for the caller.
+int write_on_device(bool bam, int bgzf, fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
+                    const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
+                    const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len) {
+    std::string err;
+    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "%s: a required argument is null", bam ? "fxg_write_bam_device" : "fxg_write_sam_device");
+    *bytes = nullptr; *bytes_len = 0;
+    try {
+    OutPlan P;
+    if (int rc = plan_output(bam, al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
+    if (P.n_rec == 0 && P.header.empty())                  // no output: nothing but the end-of-file block, or the empty text
+        return bgzf ? hand_out(kBgzfEof, sizeof kBgzfEof, bytes, bytes_len) : hand_out(nullptr, 0, bytes, bytes_len);
+
+    // ---- one upload through page-locked staging, every segment at a 256-byte boundary: reads, alignments, CIGAR range,
+    //      forward-pool range, names, qualities, (SAM) reference name offsets and names, header ----
+    size_t up = 0;
+    auto place = [&up](size_t n) { size_t const at = up; up = align_up(at + n, 256); return at; };
+    size_t const o_reads = place(n_reads * sizeof(OutReadRec)), o_al = place(n_al * sizeof(fxg_alignment)),
+                 o_cig = place((P.cigar_hi - P.cigar_lo) * 4), o_seq = place(P.seq_hi - P.seq_lo), o_names = place(P.names_len),
+                 o_quals = place(P.quals_len), o_refoff = place(P.ref_off.size() * 8),
+                 o_refnames = place(P.ref_off.empty() ? 0 : P.ref_off.back()), o_header = place(P.header.size());
+    CUDA_TRY(err, cudaSetDevice(c->device));
+    OutScratch K{c};
+    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    cudaStream_t const s = K.st;
+    CUDA_TRY(err, K.host.ensure(up + 64));
+    uint8_t* const h = K.host.as<uint8_t>();
+    if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(OutReadRec));
+    if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
+    if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
+    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
+    for (size_t ri = 0; ri < n_reads; ++ri) {
+        OutReadRec const& O = P.reads[ri];
+        std::memcpy(h + o_names + O.name, queries[ri].id ? queries[ri].id : "*", O.l_name);
+        if (O.l_qual) std::memcpy(h + o_quals + O.qual, queries[ri].quality, O.l_qual);
+    }
+    if (!P.ref_off.empty()) std::memcpy(h + o_refoff, P.ref_off.data(), P.ref_off.size() * 8);
+    for (size_t r = 0; r + 1 < P.ref_off.size(); ++r) std::memcpy(h + o_refnames + P.ref_off[r], reference_ids[r], P.ref_off[r + 1] - P.ref_off[r]);
+    std::memcpy(h + o_header, P.header.data(), P.header.size());
+    CUDA_TRY(err, K.in.ensure(up));
+    CUDA_TRY(err, cudaMemcpyAsync(K.in.p, h, up, cudaMemcpyHostToDevice, s));
+    uint64_t h2d = up, d2h = 0, launches = 0;
+    uint8_t* const din = K.in.as<uint8_t>();
+    OutArgs A{};
+    A.reads = reinterpret_cast<const OutReadRec*>(din + o_reads); A.n_reads = uint32_t(n_reads);
+    A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
+    A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
+    A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = reinterpret_cast<const char*>(din + o_quals);
+    A.ref_off = reinterpret_cast<const uint64_t*>(din + o_refoff); A.ref_names = reinterpret_cast<const char*>(din + o_refnames);
+    auto const size_kernel = bam ? bam_size_kernel : sam_size_kernel;
+    auto const write_kernel = bam ? bam_write_kernel : sam_write_kernel;
+
+    // ---- record sizes, their offsets, the output's length ----
+    uint32_t const n_rec = uint32_t(P.n_rec);
+    uint64_t* const h_word = reinterpret_cast<uint64_t*>(h + up);           // (read-backs go behind the upload)
+    uint64_t body = 0;
+    if (n_rec) {
+        CUDA_TRY(err, K.recs.ensure(size_t(n_rec) * (bam ? sizeof(BamRecord) : sizeof(SamRecord))));
+        CUDA_TRY(err, K.sizes.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, K.offs.ensure((size_t(n_rec) + 1) * 8));
+        CUDA_TRY(err, cudaMemsetAsync(K.sizes.as<uint64_t>() + n_rec, 0, 8, s));
+        A.recs = K.recs.p; A.rec_off = K.sizes.as<uint64_t>();
+        size_kernel<<<uint32_t((uint64_t(n_reads) * 32 + 255) / 256), 256, 0, s>>>(A);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+        size_t tmp_bytes = 0;
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, K.sizes.as<uint64_t>(), K.offs.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, K.scan_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(K.scan_tmp.p, tmp_bytes, K.sizes.as<uint64_t>(), K.offs.as<uint64_t>(), n_rec + 1, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_word, K.offs.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        d2h += 8;
+        body = h_word[0];
+    }
+    uint64_t const raw_len = P.header.size() + body;
+
+    // ---- the uncompressed output: the header, then the records ----
+    CUDA_TRY(err, K.raw.ensure(raw_len + 16));
+    if (!P.header.empty()) CUDA_TRY(err, cudaMemcpyAsync(K.raw.p, din + o_header, P.header.size(), cudaMemcpyDeviceToDevice, s));
+    A.rec_off = K.offs.as<uint64_t>(); A.out = K.raw.as<uint8_t>(); A.body = P.header.size();
+    if (n_rec) {
+        write_kernel<<<uint32_t((uint64_t(n_rec) * 32 + 255) / 256), 256, 0, s>>>(A, n_rec);
+        CUDA_TRY(err, cudaGetLastError());
+        ++launches;
+    }
+
+    // ---- the output as it is, or its BGZF image ----
+    size_t out_len = size_t(raw_len);
+    if (bgzf) {
+        if (int rc = bgzf_image_on_device(K, raw_len, h_word, d2h, launches, out_len, err)) return rc;
+    } else {
+        CUDA_TRY(err, cudaStreamSynchronize(s));                           // (the upload may still read the staging)
+        CUDA_TRY(err, K.host.ensure(out_len));
+        CUDA_TRY(err, cudaMemcpyAsync(K.host.p, K.raw.p, out_len, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        d2h += out_len;
+    }
+    {
+        std::lock_guard<std::mutex> lock(c->mu);
+        c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
+    }
+    return hand_out(K.host.p, out_len, bytes, bytes_len);
+    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+}
+
 }  // namespace
 
 extern "C" {
@@ -4206,105 +4338,8 @@ extern "C" {
 int fxg_write_bam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
                          const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
                          const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len) {
-    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
-        return FXG_ERR_INVALID_ARGUMENT;
-    *bytes = nullptr; *bytes_len = 0;
-    std::string err;
-    try {
-    BamPlan P;
-    if (int rc = plan_bam(al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
-    if (P.n_rec == 0 && P.header.empty()) {                // nothing but the end-of-file block
-        uint8_t* buf = static_cast<uint8_t*>(std::malloc(sizeof kBgzfEof));
-        if (!buf) return FXG_ERR_OUT_OF_MEMORY;
-        std::memcpy(buf, kBgzfEof, sizeof kBgzfEof);
-        *bytes = buf; *bytes_len = sizeof kBgzfEof;
-        return FXG_OK;
-    }
-
-    // ---- one upload through page-locked staging: reads, alignments, CIGAR range, forward-pool range, names, qualities, header ----
-    size_t const o_reads = 0;
-    size_t const o_al = align_up(o_reads + n_reads * sizeof(BamReadRec), 256);
-    size_t const o_cig = align_up(o_al + n_al * sizeof(fxg_alignment), 256);
-    size_t const o_seq = align_up(o_cig + (P.cigar_hi - P.cigar_lo) * 4, 256);
-    size_t const o_names = align_up(o_seq + (P.seq_hi - P.seq_lo), 256);
-    size_t const o_quals = align_up(o_names + P.names_len, 256);
-    size_t const o_header = align_up(o_quals + P.quals_len, 256);
-    size_t const up = align_up(o_header + P.header.size(), 256);
-    CUDA_TRY(err, cudaSetDevice(c->device));
-    SeedCall K{c};
-    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
-    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
-    cudaStream_t const s = K.st;
-    CUDA_TRY(err, K.host.ensure(up + 64));
-    uint8_t* const h = K.host.as<uint8_t>();
-    if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(BamReadRec));
-    if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
-    if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
-    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
-    for (size_t ri = 0; ri < n_reads; ++ri) {
-        BamReadRec const& B = P.reads[ri];
-        std::memcpy(h + o_names + B.name, queries[ri].id ? queries[ri].id : "*", B.l_name);
-        if (B.qual != ~uint64_t(0)) std::memcpy(h + o_quals + B.qual, queries[ri].quality, B.l_seq);
-    }
-    std::memcpy(h + o_header, P.header.data(), P.header.size());
-    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_raw = K.bufs[5];
-    CUDA_TRY(err, d_in.ensure(up));
-    CUDA_TRY(err, cudaMemcpyAsync(d_in.p, h, up, cudaMemcpyHostToDevice, s));
-    uint64_t h2d = up, d2h = 0, launches = 0;
-    uint8_t* const din = d_in.as<uint8_t>();
-    BamArgs A{};
-    A.reads = reinterpret_cast<const BamReadRec*>(din + o_reads); A.n_reads = uint32_t(n_reads);
-    A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
-    A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
-    A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = din + o_quals;
-
-    // ---- record sizes, their offsets, the stream's length ----
-    uint32_t const n_rec = uint32_t(P.n_rec);
-    uint64_t* const h_word = reinterpret_cast<uint64_t*>(h + up);           // (read-backs go behind the upload)
-    uint64_t body = 0;
-    if (n_rec) {
-        CUDA_TRY(err, d_rec.ensure(size_t(n_rec) * sizeof(BamRecord)));
-        CUDA_TRY(err, d_size.ensure((size_t(n_rec) + 1) * 8));
-        CUDA_TRY(err, d_off.ensure((size_t(n_rec) + 1) * 8));
-        CUDA_TRY(err, cudaMemsetAsync(d_size.as<uint64_t>() + n_rec, 0, 8, s));
-        A.recs = d_rec.as<BamRecord>(); A.rec_off = d_size.as<uint64_t>();
-        bam_size_kernel<<<uint32_t((uint64_t(n_reads) * 32 + 255) / 256), 256, 0, s>>>(A);
-        CUDA_TRY(err, cudaGetLastError());
-        ++launches;
-        size_t tmp_bytes = 0;
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
-        CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
-        CUDA_TRY(err, cudaMemcpyAsync(h_word, d_off.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
-        d2h += 8;
-        body = h_word[0];
-    }
-    uint64_t const raw_len = P.header.size() + body;
-
-    // ---- the raw stream: the header, then the records ----
-    CUDA_TRY(err, d_raw.ensure(raw_len + 16));
-    if (!P.header.empty()) CUDA_TRY(err, cudaMemcpyAsync(d_raw.p, din + o_header, P.header.size(), cudaMemcpyDeviceToDevice, s));
-    A.rec_off = d_off.as<uint64_t>(); A.raw = d_raw.as<uint8_t>(); A.body = P.header.size();
-    if (n_rec) {
-        bam_write_kernel<<<uint32_t((uint64_t(n_rec) * 32 + 255) / 256), 256, 0, s>>>(A, n_rec);
-        CUDA_TRY(err, cudaGetLastError());
-        ++launches;
-    }
-
-    // ---- BGZF blocks ----
-    size_t img_len = 0;
-    if (int rc = bgzf_image_on_device(K, d_raw.as<uint8_t>(), raw_len, h_word, d2h, launches, img_len, err)) return rc;
-    {
-        std::lock_guard<std::mutex> lock(c->mu);
-        c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
-    }
-    uint8_t* buf = static_cast<uint8_t*>(std::malloc(img_len));
-    if (!buf) return FXG_ERR_OUT_OF_MEMORY;
-    std::memcpy(buf, K.host.p, img_len);
-    *bytes = buf; *bytes_len = img_len;
-    return FXG_OK;
-    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+    return write_on_device(true, 1, c, al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, forward_pool,
+                           queries, with_header, bytes, bytes_len);
 }
 
 int fxg_job_write_bam_device(fxg_ctx* c, const fxg_job* job, size_t n_references, const char* const* reference_ids,
@@ -4315,186 +4350,12 @@ int fxg_job_write_bam_device(fxg_ctx* c, const fxg_job* job, size_t n_references
                                 reference_lengths, reads, n_reads, forward_pool, queries, with_header, bytes, bytes_len);
 }
 
-}  // extern "C"
-
-// ------------------------------------------------------------------------------------------------ SAM on the device
-
-namespace {
-
-// The batch as the SAM kernels read it, and what fxg_write_sam would refuse.  sam_output.cpp walks the reads in order and
-// checks a read's alignments before it moves on to the next read; the first failure it would meet decides the code.
-struct SamPlan {
-    std::vector<SamReadRec> reads;
-    std::vector<uint64_t> ref_off;                         // the reference names, concatenated: n_references + 1 offsets
-    std::string header;                                    // the @HD / @SQ lines (empty without them)
-    uint64_t cigar_lo = UINT64_MAX, cigar_hi = 0, seq_lo = UINT64_MAX, seq_hi = 0, names_len = 0, quals_len = 0;
-    uint64_t n_rec = 0;
-};
-
-int plan_sam(const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references, const char* const* reference_ids,
-             const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads, const fxg_sam_query* queries, int with_header,
-             SamPlan& P, std::string& err) {
-    P.reads.resize(n_reads);
-    size_t a = 0;
-    for (size_t ri = 0; ri < n_reads; ++ri) {
-        size_t const a0 = a;
-        while (a < n_al && al[a].read_index == ri) ++a;
-        if (a < n_al && al[a].read_index < ri)
-            return fail(err, FXG_ERR_STATE, "alignment %zu (read %u) follows read %zu: alignments must be grouped by read", a, al[a].read_index, ri);
-        for (size_t k = a0; k < a; ++k) {
-            fxg_alignment const& A = al[k];
-            if (A.reference_id >= n_references || (A.cigar_len && !cigar_pool))
-                return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: alignment %zu has a reference id out of range or a CIGAR without a pool", ri, k);
-            if (A.cigar_len) { P.cigar_lo = std::min<uint64_t>(P.cigar_lo, A.cigar_offset); P.cigar_hi = std::max<uint64_t>(P.cigar_hi, A.cigar_offset + A.cigar_len); }
-        }
-        fxg_read const& R = reads[ri];
-        const char* const q = queries[ri].quality;
-        SamReadRec& S = P.reads[ri];
-        S.seq = R.query_offset;
-        S.l_seq = R.query_len;
-        S.name = P.names_len;
-        S.l_name = uint32_t(std::strlen(queries[ri].id ? queries[ri].id : "*"));
-        S.qual = P.quals_len;
-        S.l_qual = q ? uint32_t(std::strlen(q)) : 0u;
-        S.al0 = uint32_t(a0); S.n_al = uint32_t(a - a0);
-        S.rec0 = uint32_t(P.n_rec);
-        P.names_len += S.l_name;
-        P.quals_len += S.l_qual;
-        if (R.query_len) { P.seq_lo = std::min<uint64_t>(P.seq_lo, R.query_offset); P.seq_hi = std::max<uint64_t>(P.seq_hi, R.query_offset + R.query_len); }
-        P.n_rec += std::max<size_t>(a - a0, 1);
-    }
-    if (a != n_al) return fail(err, FXG_ERR_STATE, "alignment %zu names read %u of %zu: alignments must be grouped by read in read order", a, al[a].read_index, n_reads);
-    if (P.n_rec >= (uint64_t(1) << 32) || n_al >= (uint64_t(1) << 32))
-        return fail(err, FXG_ERR_INVALID_ARGUMENT, "%llu records: split the batch", (unsigned long long)P.n_rec);
-    if (P.seq_lo > P.seq_hi) P.seq_lo = P.seq_hi = 0;
-    if (P.cigar_lo > P.cigar_hi) P.cigar_lo = P.cigar_hi = 0;
-    for (SamReadRec& S : P.reads) S.seq -= std::min(S.seq, P.seq_lo);
-    P.ref_off.resize(n_references + 1);
-    P.ref_off[0] = 0;
-    for (size_t r = 0; r < n_references; ++r) P.ref_off[r + 1] = P.ref_off[r] + std::strlen(reference_ids[r]);
-    if (with_header) {                                     // sam_output.cpp's header, byte for byte
-        P.header = "@HD\tVN:1.6\tSO:unknown\tGO:none\n";
-        for (size_t r = 0; r < n_references; ++r) {
-            P.header += "@SQ\tSN:"; P.header += reference_ids[r]; P.header += "\tLN:"; P.header += std::to_string(reference_lengths[r]); P.header += '\n';
-        }
-    }
-    return FXG_OK;
-}
-
-}  // namespace
-
-extern "C" {
-
 int fxg_write_sam_device(fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
                          const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
                          const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, int bgzf, uint8_t** bytes,
                          size_t* bytes_len) {
-    std::string err;
-    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
-        return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_write_sam_device: a required argument is null");
-    *bytes = nullptr; *bytes_len = 0;
-    try {
-    SamPlan P;
-    if (int rc = plan_sam(al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
-    if (P.n_rec == 0 && P.header.empty())                  // no text: the empty string, or nothing but the end-of-file block
-        return bgzf ? hand_out(kBgzfEof, sizeof kBgzfEof, bytes, bytes_len) : hand_out(nullptr, 0, bytes, bytes_len);
-
-    // ---- one upload through page-locked staging: reads, alignments, CIGAR range, forward-pool range, names, qualities,
-    //      reference names and their offsets, header ----
-    size_t const ref_names_len = P.ref_off.back();
-    size_t const o_reads = 0;
-    size_t const o_al = align_up(o_reads + n_reads * sizeof(SamReadRec), 256);
-    size_t const o_cig = align_up(o_al + n_al * sizeof(fxg_alignment), 256);
-    size_t const o_seq = align_up(o_cig + (P.cigar_hi - P.cigar_lo) * 4, 256);
-    size_t const o_names = align_up(o_seq + (P.seq_hi - P.seq_lo), 256);
-    size_t const o_quals = align_up(o_names + P.names_len, 256);
-    size_t const o_refoff = align_up(o_quals + P.quals_len, 256);
-    size_t const o_refnames = align_up(o_refoff + P.ref_off.size() * 8, 256);
-    size_t const o_header = align_up(o_refnames + ref_names_len, 256);
-    size_t const up = align_up(o_header + P.header.size(), 256);
-    CUDA_TRY(err, cudaSetDevice(c->device));
-    SeedCall K{c};
-    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
-    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
-    cudaStream_t const s = K.st;
-    CUDA_TRY(err, K.host.ensure(up + 64));
-    uint8_t* const h = K.host.as<uint8_t>();
-    if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(SamReadRec));
-    if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
-    if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
-    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
-    for (size_t ri = 0; ri < n_reads; ++ri) {
-        SamReadRec const& S = P.reads[ri];
-        std::memcpy(h + o_names + S.name, queries[ri].id ? queries[ri].id : "*", S.l_name);
-        if (S.l_qual) std::memcpy(h + o_quals + S.qual, queries[ri].quality, S.l_qual);
-    }
-    std::memcpy(h + o_refoff, P.ref_off.data(), P.ref_off.size() * 8);
-    for (size_t r = 0; r < n_references; ++r) std::memcpy(h + o_refnames + P.ref_off[r], reference_ids[r], P.ref_off[r + 1] - P.ref_off[r]);
-    std::memcpy(h + o_header, P.header.data(), P.header.size());
-    DevBuf &d_in = K.bufs[0], &d_rec = K.bufs[1], &d_size = K.bufs[2], &d_off = K.bufs[3], &d_tmp = K.bufs[4], &d_text = K.bufs[5];
-    CUDA_TRY(err, d_in.ensure(up));
-    CUDA_TRY(err, cudaMemcpyAsync(d_in.p, h, up, cudaMemcpyHostToDevice, s));
-    uint64_t h2d = up, d2h = 0, launches = 0;
-    uint8_t* const din = d_in.as<uint8_t>();
-    SamArgs A{};
-    A.reads = reinterpret_cast<const SamReadRec*>(din + o_reads); A.n_reads = uint32_t(n_reads);
-    A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
-    A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
-    A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = reinterpret_cast<const char*>(din + o_quals);
-    A.ref_off = reinterpret_cast<const uint64_t*>(din + o_refoff); A.ref_names = reinterpret_cast<const char*>(din + o_refnames);
-
-    // ---- record lengths, their offsets, the text's length ----
-    uint32_t const n_rec = uint32_t(P.n_rec);
-    uint64_t* const h_word = reinterpret_cast<uint64_t*>(h + up);           // (read-backs go behind the upload)
-    uint64_t body = 0;
-    if (n_rec) {
-        CUDA_TRY(err, d_rec.ensure(size_t(n_rec) * sizeof(SamRecord)));
-        CUDA_TRY(err, d_size.ensure((size_t(n_rec) + 1) * 8));
-        CUDA_TRY(err, d_off.ensure((size_t(n_rec) + 1) * 8));
-        CUDA_TRY(err, cudaMemsetAsync(d_size.as<uint64_t>() + n_rec, 0, 8, s));
-        A.recs = d_rec.as<SamRecord>(); A.rec_off = d_size.as<uint64_t>();
-        sam_size_kernel<<<uint32_t((uint64_t(n_reads) * 32 + 255) / 256), 256, 0, s>>>(A);
-        CUDA_TRY(err, cudaGetLastError());
-        ++launches;
-        size_t tmp_bytes = 0;
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
-        CUDA_TRY(err, d_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
-        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_size.as<uint64_t>(), d_off.as<uint64_t>(), n_rec + 1, s));
-        CUDA_TRY(err, cudaMemcpyAsync(h_word, d_off.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
-        d2h += 8;
-        body = h_word[0];
-    }
-    uint64_t const text_len = P.header.size() + body;
-
-    // ---- the text: the header, then the records ----
-    CUDA_TRY(err, d_text.ensure(text_len + 16));
-    if (!P.header.empty()) CUDA_TRY(err, cudaMemcpyAsync(d_text.p, din + o_header, P.header.size(), cudaMemcpyDeviceToDevice, s));
-    A.rec_off = d_off.as<uint64_t>(); A.text = d_text.as<char>(); A.body = P.header.size();
-    if (n_rec) {
-        sam_write_kernel<<<uint32_t((uint64_t(n_rec) * 32 + 255) / 256), 256, 0, s>>>(A, n_rec);
-        CUDA_TRY(err, cudaGetLastError());
-        ++launches;
-    }
-
-    // ---- the text as it is, or its BGZF image ----
-    size_t out_len = 0;
-    if (bgzf) {
-        if (int rc = bgzf_image_on_device(K, d_text.as<uint8_t>(), text_len, h_word, d2h, launches, out_len, err)) return rc;
-    } else {
-        out_len = size_t(text_len);
-        CUDA_TRY(err, cudaStreamSynchronize(s));                           // (the upload may still read the staging)
-        CUDA_TRY(err, K.host.ensure(out_len));
-        CUDA_TRY(err, cudaMemcpyAsync(K.host.p, d_text.p, out_len, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(err, cudaStreamSynchronize(s));
-        d2h += out_len;
-    }
-    {
-        std::lock_guard<std::mutex> lock(c->mu);
-        c->ctr.h2d_bytes += h2d; c->ctr.d2h_bytes += d2h; c->ctr.kernel_launches += launches;
-    }
-    return hand_out(K.host.p, out_len, bytes, bytes_len);
-    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+    return write_on_device(false, bgzf, c, al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, forward_pool,
+                           queries, with_header, bytes, bytes_len);
 }
 
 int fxg_job_write_sam_device(fxg_ctx* c, const fxg_job* job, size_t n_references, const char* const* reference_ids,

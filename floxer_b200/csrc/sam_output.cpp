@@ -14,7 +14,7 @@
 // test/floxer_whole_program_via_cli_test.cpp:38-93 (tests/test_sam_output.py).
 //
 // Host-only code: the array entry point fxg_write_sam needs neither a context nor a GPU (tests/test_sam_arrays.py);
-// fxg_write_sam_device (floxer_gpu.cu, sam_kernels.cuh) writes the same text on the device.
+// fxg_write_sam_device (floxer_gpu.cu, record_kernels.cuh) writes the same text on the device.
 #include "../../include/floxer_gpu.h"
 
 #include <algorithm>

@@ -110,7 +110,17 @@ class _SamQuery(C.Structure):
     _fields_ = [("id", C.c_char_p), ("quality", C.c_char_p)]
 
 
-def _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities):
+def _alignment_arrays(alignments, cigars):
+    """The alignment records (abi.ALIGNMENT_DTYPE) and their cigar pool as the array forms take them: pointer, count,
+    pointer.  The ctypes views keep the contiguous copies alive through the call."""
+    al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
+    cg = np.ascontiguousarray(cigars, dtype=np.uint32)
+    return (al.ctypes if len(al) else None, len(al), cg.ctypes if len(cg) else None)
+
+
+def _write(fn, lead, batch, reference_ids, reference_lengths, query_ids, qualities, header, *trail, ctx=None) -> bytes:
+    """fn(*lead, <the references, reads and queries>, header, *trail, &bytes, &length) of a SAM / BAM writer: the bytes it
+    hands out, freed with fxg_free.  A refusal raises FloxerGpuError, with the context's error text when ctx is given."""
     n_ref, n = len(reference_ids), len(batch.reads)
     ref_ids = (C.c_char_p * max(n_ref, 1))(*[r.encode() for r in reference_ids])
     ref_lens = (C.c_uint64 * max(n_ref, 1))(*[int(x) for x in reference_lengths])
@@ -118,43 +128,31 @@ def _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualit
     for i in range(n):
         qs[i].id = query_ids[i].encode()
         qs[i].quality = (qualities[i] if qualities is not None else "").encode()
-    return n_ref, ref_ids, ref_lens, n, qs
+    out, length = C.c_void_p(), C.c_size_t(0)
+    rc = fn(*lead, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs, int(header), *trail,
+            C.byref(out), C.byref(length))
+    if ctx is not None:
+        ctx._check(rc)
+    elif rc != 0:
+        raise FloxerGpuError(rc, f"{fn.__name__} failed")
+    try:
+        return C.string_at(out, length.value)
+    finally:
+        lib().fxg_free(out)
 
 
 def write_bam(alignments, cigars, batch, reference_ids, reference_lengths, query_ids, qualities=None, header: bool = True) -> bytes:
     """BAM file image (BGZF) of alignment records given as arrays (abi.ALIGNMENT_DTYPE, grouped by read in read order, and
     their cigar pool): fxg_write_bam, host only -- no context, no GPU."""
-    L = lib()
-    al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
-    cg = np.ascontiguousarray(cigars, dtype=np.uint32)
-    n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-    out, length = C.c_void_p(), C.c_size_t(0)
-    rc = L.fxg_write_bam(al.ctypes.data if len(al) else None, len(al), cg.ctypes.data if len(cg) else None, n_ref, ref_ids, ref_lens,
-                         batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs, int(header), C.byref(out), C.byref(length))
-    if rc != 0:
-        raise FloxerGpuError(rc, "fxg_write_bam failed")
-    try:
-        return C.string_at(out, length.value)
-    finally:
-        L.fxg_free(out)
+    return _write(lib().fxg_write_bam, _alignment_arrays(alignments, cigars), batch, reference_ids, reference_lengths, query_ids,
+                  qualities, header)
 
 
 def write_sam(alignments, cigars, batch, reference_ids, reference_lengths, query_ids, qualities=None, header: bool = True) -> str:
     """SAM text of alignment records given as arrays (abi.ALIGNMENT_DTYPE, grouped by read in read order, and their cigar
     pool): fxg_write_sam, host only -- no context, no GPU."""
-    L = lib()
-    al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
-    cg = np.ascontiguousarray(cigars, dtype=np.uint32)
-    n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-    out, length = C.c_void_p(), C.c_size_t(0)
-    rc = L.fxg_write_sam(al.ctypes.data if len(al) else None, len(al), cg.ctypes.data if len(cg) else None, n_ref, ref_ids, ref_lens,
-                         batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs, int(header), C.byref(out), C.byref(length))
-    if rc != 0:
-        raise FloxerGpuError(rc, "fxg_write_sam failed")
-    try:
-        return C.string_at(out, length.value).decode()
-    finally:
-        L.fxg_free(out)
+    return _write(lib().fxg_write_sam, _alignment_arrays(alignments, cigars), batch, reference_ids, reference_lengths, query_ids,
+                  qualities, header).decode()
 
 
 def pex_build(total_len: int, num_errors: int, leaf_max_errors: int, strategy: int = 0):
@@ -285,59 +283,22 @@ class Job:
         """SAM text of the job's alignments (output::alignment_output::write_alignments_for_query, src/lib/output.cpp:49-108):
         fxg_job_write_sam, or with on_device=True fxg_job_write_sam_device on the job's context (the same text, formatted on
         the GPU).  bgzf=True (device only) returns the BGZF-compressed text as bytes instead of a str."""
-        L = lib()
         if bgzf and not on_device:
             raise ValueError("bgzf=True needs on_device=True")
+        args = (batch, reference_ids, reference_lengths, query_ids, qualities, header)
         if on_device:
-            n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-            out, length = C.c_void_p(), C.c_size_t(0)
-            self._ctx._check(L.fxg_job_write_sam_device(self._ctx._h, self._h, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n,
-                                                        batch.forward_pool.ctypes.data, qs, int(header), int(bgzf), C.byref(out),
-                                                        C.byref(length)))
-            try:
-                data = C.string_at(out, length.value)
-            finally:
-                L.fxg_free(out)
+            data = _write(lib().fxg_job_write_sam_device, (self._ctx._h, self._h), *args, int(bgzf), ctx=self._ctx)
             return data if bgzf else data.decode()
-        n_ref, n = len(reference_ids), len(batch.reads)
-        ref_ids = (C.c_char_p * max(n_ref, 1))(*[r.encode() for r in reference_ids])
-        ref_lens = (C.c_uint64 * max(n_ref, 1))(*[int(x) for x in reference_lengths])
-
-        class SamQuery(C.Structure):
-            _fields_ = [("id", C.c_char_p), ("quality", C.c_char_p)]
-        qs = (SamQuery * max(n, 1))()
-        for i in range(n):
-            qs[i].id = query_ids[i].encode()
-            qs[i].quality = (qualities[i] if qualities is not None else "").encode()
-        text, length = C.c_void_p(), C.c_size_t(0)
-        rc = L.fxg_job_write_sam(self._h, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data,
-                                 qs, int(header), C.byref(text), C.byref(length))
-        if rc != 0:
-            raise FloxerGpuError(rc, "fxg_job_write_sam failed")
-        try:
-            return C.string_at(text, length.value).decode()
-        finally:
-            L.fxg_free(text)
+        return _write(lib().fxg_job_write_sam, (self._h,), *args).decode()
 
     def bam(self, batch: ReadBatch, reference_ids, reference_lengths, query_ids, qualities=None, header: bool = True,
             on_device: bool = False) -> bytes:
         """The same records as a BAM file image (BGZF blocks incl. the end-of-file block): fxg_job_write_bam, or with
         on_device=True fxg_job_write_bam_device on the job's context (the same records and blocks, compressed on the GPU)."""
-        L = lib()
-        n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-        out, length = C.c_void_p(), C.c_size_t(0)
-        args = (self._h, n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs, int(header),
-                C.byref(out), C.byref(length))
+        args = (batch, reference_ids, reference_lengths, query_ids, qualities, header)
         if on_device:
-            self._ctx._check(L.fxg_job_write_bam_device(self._ctx._h, *args))
-        else:
-            rc = L.fxg_job_write_bam(*args)
-            if rc != 0:
-                raise FloxerGpuError(rc, "fxg_job_write_bam failed")
-        try:
-            return C.string_at(out, length.value)
-        finally:
-            L.fxg_free(out)
+            return _write(lib().fxg_job_write_bam_device, (self._ctx._h, self._h), *args, ctx=self._ctx)
+        return _write(lib().fxg_job_write_bam, (self._h,), *args)
 
     def free(self):
         if self._h:
@@ -503,36 +464,16 @@ class Context:
                   header: bool = True) -> bytes:
         """gpu.write_bam with the work on this context's device (fxg_write_bam_device): the same records and BGZF blocks,
         deflated on the GPU."""
-        L = lib()
-        al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
-        cg = np.ascontiguousarray(cigars, dtype=np.uint32)
-        n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-        out, length = C.c_void_p(), C.c_size_t(0)
-        self._check(L.fxg_write_bam_device(self._h, al.ctypes.data if len(al) else None, len(al), cg.ctypes.data if len(cg) else None,
-                                           n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs,
-                                           int(header), C.byref(out), C.byref(length)))
-        try:
-            return C.string_at(out, length.value)
-        finally:
-            L.fxg_free(out)
+        return _write(lib().fxg_write_bam_device, (self._h, *_alignment_arrays(alignments, cigars)), batch, reference_ids,
+                      reference_lengths, query_ids, qualities, header, ctx=self)
 
     # ---- SAM output on the device ----
     def write_sam(self, alignments, cigars, batch, reference_ids, reference_lengths, query_ids, qualities=None,
                   header: bool = True, bgzf: bool = False):
         """gpu.write_sam with the work on this context's device (fxg_write_sam_device): the same text as a str, or with
         bgzf=True its BGZF image (.sam.gz) as bytes."""
-        L = lib()
-        al = np.ascontiguousarray(alignments, dtype=abi.ALIGNMENT_DTYPE)
-        cg = np.ascontiguousarray(cigars, dtype=np.uint32)
-        n_ref, ref_ids, ref_lens, n, qs = _output_arguments(batch, reference_ids, reference_lengths, query_ids, qualities)
-        out, length = C.c_void_p(), C.c_size_t(0)
-        self._check(L.fxg_write_sam_device(self._h, al.ctypes.data if len(al) else None, len(al), cg.ctypes.data if len(cg) else None,
-                                           n_ref, ref_ids, ref_lens, batch.reads.ctypes.data, n, batch.forward_pool.ctypes.data, qs,
-                                           int(header), int(bgzf), C.byref(out), C.byref(length)))
-        try:
-            data = C.string_at(out, length.value)
-        finally:
-            L.fxg_free(out)
+        data = _write(lib().fxg_write_sam_device, (self._h, *_alignment_arrays(alignments, cigars)), batch, reference_ids,
+                      reference_lengths, query_ids, qualities, header, int(bgzf), ctx=self)
         return data if bgzf else data.decode()
 
     # ---- accounting ----
