@@ -14,6 +14,9 @@ FORWARD, REVERSE_COMPLEMENT = 0, 1
 KIND_DIRECT_FULL, KIND_HIERARCHICAL = 0, 1
 CIGAR_CHARS = {1: "I", 2: "D", 7: "=", 8: "X"}
 
+READ_KEPT, READ_TOO_FEW_ERRORS, READ_BAD_LENGTH, READ_UNSEEDABLE = 0, 1, 2, 3
+FORMAT_BAM, FORMAT_SAM, FORMAT_SAM_BGZF = 0, 1, 2
+
 OK, ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_OUT_OF_MEMORY, ERR_OVERFLOW, ERR_STATE = 0, -1, -2, -3, -4, -5
 
 PEX_NODE_DTYPE = np.dtype([("parent_id", "<u8"), ("query_index_from", "<u8"),
@@ -32,9 +35,11 @@ READ_DTYPE = np.dtype([("query_offset", "<u8"), ("node_offset", "<u8"), ("anchor
 ALIGNMENT_DTYPE = np.dtype([("start_in_reference", "<u8"), ("cigar_offset", "<u8"), ("cigar_len", "<u4"),
                             ("num_errors", "<u4"), ("read_index", "<u4"), ("reference_id", "<u4"),
                             ("orientation", "u1"), ("reserved", "u1", (7,))])
+READ_SPAN_DTYPE = np.dtype([("record", "<u8"), ("id_offset", "<u8"), ("quality_offset", "<u8"),
+                            ("id_len", "<u4"), ("quality_len", "<u4")])
 
 assert ALIGN_TASK_DTYPE.itemsize == 48 and ALIGN_RESULT_DTYPE.itemsize == 32
-assert READ_DTYPE.itemsize == 48 and ALIGNMENT_DTYPE.itemsize == 40
+assert READ_DTYPE.itemsize == 48 and ALIGNMENT_DTYPE.itemsize == 40 and READ_SPAN_DTYPE.itemsize == 32
 
 
 class VerifyConfig(C.Structure):
@@ -71,6 +76,26 @@ class SeedStats(C.Structure):
 
     def as_dict(self) -> dict:
         return {n: int(getattr(self, n)) for n, _ in self._fields_ if n != "reserved"}
+
+
+class ReadConfig(C.Structure):
+    _fields_ = [("error_probability", C.c_double), ("query_errors", C.c_uint64), ("seed_errors", C.c_uint64),
+                ("build_strategy", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class ParsedView(C.Structure):
+    vp, sz = C.c_void_p, C.c_size_t
+    _fields_ = [("n_records", sz), ("statuses", vp), ("n_reads", sz), ("reads", vp), ("spans", vp),
+                ("pool_len", sz), ("forward_pool", vp), ("reverse_complement_pool", vp), ("n_nodes", sz), ("nodes", vp)]
+
+
+class MapSummary(C.Structure):
+    _fields_ = [("records", C.c_uint64), ("reads", C.c_uint64 * 4), ("alignments", C.c_uint64), ("seed", SeedStats)]
+
+    def as_dict(self) -> dict:
+        return {"records": int(self.records), "kept": int(self.reads[READ_KEPT]),
+                "too_few_errors": int(self.reads[READ_TOO_FEW_ERRORS]), "bad_length": int(self.reads[READ_BAD_LENGTH]),
+                "unseedable": int(self.reads[READ_UNSEEDABLE]), "alignments": int(self.alignments), "seed": self.seed.as_dict()}
 
 
 def cigar_to_string(ops) -> str:

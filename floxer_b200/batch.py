@@ -22,6 +22,21 @@ class VerifyConfig:
 
 
 @dataclass
+class ReadConfig:
+    """How reads are taken from a FASTQ text (--query-errors / --error-probability, --seed-errors,
+    --pex-tree-build-strategy): k is query_errors when given, else ceil(m * error_probability); a read with
+    k < seed_errors is skipped (src/lib/input.cpp:26-34,114-129)."""
+    error_probability: float = 0.05
+    query_errors: int | None = None
+    seed_errors: int = 2                         # include/floxer_cli.hpp, default 2
+    bottom_up: bool = False                      # pex tree build strategy: recursive (0) or bottom_up (1)
+
+    def to_c(self) -> abi.ReadConfig:
+        qe = abi.NULL_ID if self.query_errors is None else int(self.query_errors)
+        return abi.ReadConfig(float(self.error_probability), qe, int(self.seed_errors), int(bool(self.bottom_up)), 0)
+
+
+@dataclass
 class ReadBatch:
     reads: np.ndarray                     # abi.READ_DTYPE
     forward_pool: np.ndarray              # uint8 ranks

@@ -12,6 +12,7 @@
 #include "../../include/floxer_gpu.h"
 #include "bgzf_kernels.cuh"
 #include "dp_kernels.cuh"
+#include "read_kernels.cuh"
 #include "record_kernels.cuh"
 #include "root_kernels.cuh"
 #include "seed_kernels.cuh"
@@ -19,6 +20,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 #include <algorithm>
 #include <atomic>
@@ -1387,18 +1389,19 @@ int upload_packed(fxg_ctx* c, const uint8_t* ranks, uint64_t len, DevBuf& dst, u
 }
 
 // uploads up to two byte ranges back to back (forward / reverse pools) and builds the Peq planes; errors and
-// accounting go to the caller's objects (fxg_verify_reads runs this beside the workers)
+// accounting go to the caller's objects (fxg_verify_reads runs this beside the workers).  kind = cudaMemcpyDeviceToDevice:
+// the ranges are in device memory already (fxg_map_fastq's parsed pools) and are not counted as uploads.
 int stage_pool(fxg_ctx* c, Pool& pool, const uint8_t* a, size_t a_len, const uint8_t* b, size_t b_len, std::string& err, fxg_counters& ctr,
-               bool check_ranks_on_device = false) {
+               bool check_ranks_on_device = false, cudaMemcpyKind kind = cudaMemcpyHostToDevice) {
     cudaStream_t const st = c->stage_stream;
     pool.len = a_len + b_len;
     pool.plane_words = (pool.len + 31) / 32 + kPeqFrontPadWords + kPeqBackPadWords;
     CUDA_TRY(err, pool.bytes.ensure(pool.len + 64));
     CUDA_TRY(err, pool.peq.ensure(pool.plane_words * kNumSymbols * 4));
     CUDA_TRY(err, pool.bad_rank.ensure(4));
-    if (a_len) CUDA_TRY(err, cudaMemcpyAsync(pool.bytes.p, a, a_len, cudaMemcpyHostToDevice, st));
-    if (b_len) CUDA_TRY(err, cudaMemcpyAsync(pool.bytes.as<uint8_t>() + a_len, b, b_len, cudaMemcpyHostToDevice, st));
-    ctr.h2d_bytes += pool.len;
+    if (a_len) CUDA_TRY(err, cudaMemcpyAsync(pool.bytes.p, a, a_len, kind, st));
+    if (b_len) CUDA_TRY(err, cudaMemcpyAsync(pool.bytes.as<uint8_t>() + a_len, b, b_len, kind, st));
+    if (kind == cudaMemcpyHostToDevice) ctr.h2d_bytes += pool.len;
     CUDA_TRY(err, cudaMemsetAsync(pool.peq.p, 0, pool.plane_words * kNumSymbols * 4, st));
     CUDA_TRY(err, cudaMemsetAsync(pool.bad_rank.p, 0, 4, st));
     if (pool.len) {
@@ -3985,11 +3988,17 @@ int fxg_seed_reads(fxg_ctx* c, const fxg_gpu_seeder* S, fxg_read* reads, size_t 
     return FXG_OK;
 }
 
-int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_config* cfg, fxg_read* reads, size_t n_reads,
-                          const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
-                          const fxg_pex_node* nodes, size_t n_nodes,
-                          uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
-                          fxg_seed_stats* stats, fxg_job** out) {
+}  // extern "C"
+
+namespace {
+
+// fxg_seed_verify_reads; pool_kind = cudaMemcpyDeviceToDevice: the pools are in device memory (fxg_map_fastq) and fill the
+// job's pool from there
+int seed_verify(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_config* cfg, fxg_read* reads, size_t n_reads,
+                const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                const fxg_pex_node* nodes, size_t n_nodes,
+                uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                fxg_seed_stats* stats, fxg_job** out, cudaMemcpyKind pool_kind) {
     if (!c || !S || !cfg || !out || (n_reads && !reads) || (pool_len && (!forward_pool || !reverse_complement_pool)) || (n_nodes && !nodes))
         return FXG_ERR_INVALID_ARGUMENT;
     *out = nullptr;
@@ -4012,7 +4021,7 @@ int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_
 
     // ---- the pools go up once: the seeder reads the job's pool (forward, then reverse complement, as SeedBatch wants) ----
     fxg_counters ctr{};
-    int rc = stage_pool(c, j->pool, forward_pool, pool_len, reverse_complement_pool, pool_len, err, ctr, true);
+    int rc = stage_pool(c, j->pool, forward_pool, pool_len, reverse_complement_pool, pool_len, err, ctr, true, pool_kind);
     if (rc == FXG_OK && cudaEventCreateWithFlags(&j->pool_ready, cudaEventDisableTiming | cudaEventBlockingSync) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "cannot create an event");
     if (rc == FXG_OK && cudaEventRecord(j->pool_ready, c->stage_stream) != cudaSuccess) rc = fail(err, FXG_ERR_CUDA, "staging failed");
     // ---- seeding: the survivors land in the job's record buffer where prepare_job's layout puts the anchors ----
@@ -4056,6 +4065,19 @@ int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_
     return rc;
 }
 
+}  // namespace
+
+extern "C" {
+
+int fxg_seed_verify_reads(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_verify_config* cfg, fxg_read* reads, size_t n_reads,
+                          const uint8_t* forward_pool, const uint8_t* reverse_complement_pool, size_t pool_len,
+                          const fxg_pex_node* nodes, size_t n_nodes,
+                          uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                          fxg_seed_stats* stats, fxg_job** out) {
+    return seed_verify(c, S, cfg, reads, n_reads, forward_pool, reverse_complement_pool, pool_len, nodes, n_nodes, max_anchors_hard,
+                       max_anchors_soft, erase_useless_anchors, stats, out, cudaMemcpyHostToDevice);
+}
+
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------ BAM and SAM on the device
@@ -4074,9 +4096,13 @@ struct OutPlan {
     uint64_t n_rec = 0;
 };
 
+// (fxg_map_fastq) the reads' SEQ, names and qualities in device memory already: SEQ in the parsed forward pool, the names
+// and qualities in the uploaded text at each read's spans.  The record kernels read them there instead of an upload.
+struct DeviceReads { const uint8_t* forward_pool; const char* text; const fxg_read_span* spans; };
+
 int plan_output(bool bam, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
                 const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
-                const fxg_sam_query* queries, int with_header, OutPlan& P, std::string& err) {
+                const fxg_sam_query* queries, int with_header, OutPlan& P, std::string& err, const DeviceReads* dev = nullptr) {
     P.reads.resize(n_reads);
     size_t a = 0;
     for (size_t ri = 0; ri < n_reads; ++ri) {
@@ -4084,7 +4110,7 @@ int plan_output(bool bam, const fxg_alignment* al, size_t n_al, const uint32_t* 
         while (a < n_al && al[a].read_index == ri) ++a;
         if (a < n_al && al[a].read_index < ri)
             return fail(err, FXG_ERR_STATE, "alignment %zu (read %u) follows read %zu: alignments must be grouped by read", a, al[a].read_index, ri);
-        size_t const l_name = std::strlen(queries[ri].id ? queries[ri].id : "*") + (bam ? 1 : 0);     // BAM names carry their NUL
+        size_t const l_name = (dev ? dev->spans[ri].id_len : std::strlen(queries[ri].id ? queries[ri].id : "*")) + (bam ? 1 : 0);     // BAM names carry their NUL
         if (bam && a == a0 && l_name > 255) return fail(err, FXG_ERR_INVALID_ARGUMENT, "read %zu: the name has %zu characters (254 at most)", ri, l_name - 1);
         // (BAM) the first failing alignment in (reference id, index) order
         uint64_t first = UINT64_MAX;
@@ -4115,15 +4141,17 @@ int plan_output(bool bam, const fxg_alignment* al, size_t n_al, const uint32_t* 
             return fail(err, code, "read %zu: a CIGAR of more than 65535 operations spans 2^28 bases or more (the CG tag's placeholder cannot hold it)", ri);
         if (code != FXG_OK) return fail(err, code, "read %zu: a reference id out of range, a CIGAR without a pool or a name of more than 254 characters", ri);
         fxg_read const& R = reads[ri];
-        const char* const q = queries[ri].quality;
+        const char* const q = dev ? nullptr : queries[ri].quality;
+        bool const have_q = dev || q;
+        size_t const l_q = dev ? dev->spans[ri].quality_len : q ? std::strlen(q) : 0;
         OutReadRec& O = P.reads[ri];
         O.seq = R.query_offset;
-        O.name = P.names_len;
-        O.qual = P.quals_len;
+        O.name = dev ? dev->spans[ri].id_offset : P.names_len;
+        O.qual = dev ? dev->spans[ri].quality_offset : P.quals_len;
         O.l_seq = R.query_len;
         O.l_name = uint32_t(l_name);
         // SAM writes every quality at its own length, BAM only one of exactly query_len characters
-        O.l_qual = !q ? 0u : !bam ? uint32_t(std::strlen(q)) : q[0] && std::strlen(q) == R.query_len ? R.query_len : 0u;
+        O.l_qual = !have_q ? 0u : !bam ? uint32_t(l_q) : l_q && l_q == R.query_len ? R.query_len : 0u;
         O.al0 = uint32_t(a0); O.n_al = uint32_t(a - a0);
         O.rec0 = uint32_t(P.n_rec);
         P.names_len += O.l_name;
@@ -4225,26 +4253,31 @@ int hand_out(const void* src, size_t n, uint8_t** bytes, size_t* bytes_len) {
 // fxg_write_bam_device (bam, always bgzf) and fxg_write_sam_device: refusals before any device work, then on a stream of
 // the call's own one upload through page-locked staging, the format's size kernel, the scan of the sizes into offsets,
 // the header and the format's write kernel, and the output as it is or (bgzf) its BGZF image, malloc'ed for the caller.
+// With `dev`, SEQ, names and qualities are read in device memory (forward_pool and queries are not used).
 int write_on_device(bool bam, int bgzf, fxg_ctx* c, const fxg_alignment* al, size_t n_al, const uint32_t* cigar_pool, size_t n_references,
                     const char* const* reference_ids, const uint64_t* reference_lengths, const fxg_read* reads, size_t n_reads,
-                    const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len) {
+                    const uint8_t* forward_pool, const fxg_sam_query* queries, int with_header, uint8_t** bytes, size_t* bytes_len,
+                    const DeviceReads* dev = nullptr) {
     std::string err;
-    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || !forward_pool || !queries)) || (n_references && (!reference_ids || !reference_lengths)))
+    if (!c || !bytes || !bytes_len || (n_al && !al) || (n_reads && (!reads || (!dev && (!forward_pool || !queries)))) ||
+        (n_references && (!reference_ids || !reference_lengths)))
         return fail(err, FXG_ERR_INVALID_ARGUMENT, "%s: a required argument is null", bam ? "fxg_write_bam_device" : "fxg_write_sam_device");
     *bytes = nullptr; *bytes_len = 0;
     try {
     OutPlan P;
-    if (int rc = plan_output(bam, al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err)) return rc;
+    if (int rc = plan_output(bam, al, n_al, cigar_pool, n_references, reference_ids, reference_lengths, reads, n_reads, queries, with_header, P, err, dev))
+        return rc;
     if (P.n_rec == 0 && P.header.empty())                  // no output: nothing but the end-of-file block, or the empty text
         return bgzf ? hand_out(kBgzfEof, sizeof kBgzfEof, bytes, bytes_len) : hand_out(nullptr, 0, bytes, bytes_len);
 
     // ---- one upload through page-locked staging, every segment at a 256-byte boundary: reads, alignments, CIGAR range,
-    //      forward-pool range, names, qualities, (SAM) reference name offsets and names, header ----
+    //      forward-pool range, names, qualities (these three not with `dev`), (SAM) reference name offsets and names,
+    //      header ----
     size_t up = 0;
     auto place = [&up](size_t n) { size_t const at = up; up = align_up(at + n, 256); return at; };
     size_t const o_reads = place(n_reads * sizeof(OutReadRec)), o_al = place(n_al * sizeof(fxg_alignment)),
-                 o_cig = place((P.cigar_hi - P.cigar_lo) * 4), o_seq = place(P.seq_hi - P.seq_lo), o_names = place(P.names_len),
-                 o_quals = place(P.quals_len), o_refoff = place(P.ref_off.size() * 8),
+                 o_cig = place((P.cigar_hi - P.cigar_lo) * 4), o_seq = place(dev ? 0 : P.seq_hi - P.seq_lo),
+                 o_names = place(dev ? 0 : P.names_len), o_quals = place(dev ? 0 : P.quals_len), o_refoff = place(P.ref_off.size() * 8),
                  o_refnames = place(P.ref_off.empty() ? 0 : P.ref_off.back()), o_header = place(P.header.size());
     CUDA_TRY(err, cudaSetDevice(c->device));
     OutScratch K{c};
@@ -4256,8 +4289,8 @@ int write_on_device(bool bam, int bgzf, fxg_ctx* c, const fxg_alignment* al, siz
     if (n_reads) std::memcpy(h + o_reads, P.reads.data(), n_reads * sizeof(OutReadRec));
     if (n_al) std::memcpy(h + o_al, al, n_al * sizeof(fxg_alignment));
     if (P.cigar_hi > P.cigar_lo) std::memcpy(h + o_cig, cigar_pool + P.cigar_lo, (P.cigar_hi - P.cigar_lo) * 4);
-    if (P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
-    for (size_t ri = 0; ri < n_reads; ++ri) {
+    if (!dev && P.seq_hi > P.seq_lo) std::memcpy(h + o_seq, forward_pool + P.seq_lo, P.seq_hi - P.seq_lo);
+    for (size_t ri = 0; ri < (dev ? 0 : n_reads); ++ri) {
         OutReadRec const& O = P.reads[ri];
         std::memcpy(h + o_names + O.name, queries[ri].id ? queries[ri].id : "*", O.l_name);
         if (O.l_qual) std::memcpy(h + o_quals + O.qual, queries[ri].quality, O.l_qual);
@@ -4274,6 +4307,7 @@ int write_on_device(bool bam, int bgzf, fxg_ctx* c, const fxg_alignment* al, siz
     A.al = reinterpret_cast<const fxg_alignment*>(din + o_al);
     A.cigars = reinterpret_cast<const uint32_t*>(din + o_cig); A.cigar_lo = P.cigar_lo;
     A.seq = din + o_seq; A.names = reinterpret_cast<const char*>(din + o_names); A.quals = reinterpret_cast<const char*>(din + o_quals);
+    if (dev) { A.seq = dev->forward_pool + P.seq_lo; A.names = A.quals = dev->text; }
     A.ref_off = reinterpret_cast<const uint64_t*>(din + o_refoff); A.ref_names = reinterpret_cast<const char*>(din + o_refnames);
     auto const size_kernel = bam ? bam_size_kernel : sam_size_kernel;
     auto const write_kernel = bam ? bam_write_kernel : sam_write_kernel;
@@ -4365,6 +4399,267 @@ int fxg_job_write_sam_device(fxg_ctx* c, const fxg_job* job, size_t n_references
     if (!job) return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_job_write_sam_device: no job");
     return fxg_write_sam_device(c, fxg_job_alignments(job), fxg_job_num_alignments(job), fxg_job_cigar_pool(job), n_references, reference_ids,
                                 reference_lengths, reads, n_reads, forward_pool, queries, with_header, bgzf, bytes, bytes_len);
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------ FASTQ input on the device
+
+struct fxg_parsed {
+    std::vector<uint8_t> statuses;               // per record
+    std::vector<fxg_read> reads;                 // the kept reads, in record order
+    std::vector<fxg_read_span> spans;
+    std::vector<fxg_pex_node> nodes;
+    std::vector<uint8_t> pools;                  // (fxg_parse_fastq) forward, then reverse complement
+    uint64_t pool_len = 0;
+};
+
+namespace {
+
+// A parse call's scratch.  The text and the pools (forward, then reverse complement) stay on the device for the steps
+// that follow in fxg_map_fastq.
+struct ParseScratch : CallScratch {
+    using CallScratch::CallScratch;
+    DevBuf &text = bufs[0], &nl = bufs[1], &n_nl = bufs[2], &recs = bufs[3], &lens = bufs[4], &offs = bufs[5], &scan_tmp = bufs[6],
+           &pool = bufs[7], &first_bad = bufs[8];
+};
+
+// Parses text[0, text_len) on a stream of K's own into `out` (all but the pools, which stay in K.pool): the text goes up
+// once through page-locked staging, the device finds the records, checks and converts them, and the host builds the kept
+// reads' trees on several threads while the ranks are written.  The copies and launches are added to ctr.
+int parse_on_device(fxg_ctx* c, const fxg_read_config* cfg, const char* text, size_t text_len, ParseScratch& K, fxg_parsed& out,
+                    fxg_counters& ctr, std::string& err) {
+    if (cfg->build_strategy > 1) return fail(err, FXG_ERR_INVALID_ARGUMENT, "build_strategy %u: 0 (recursive) or 1 (bottom_up)", cfg->build_strategy);
+    if (cfg->query_errors == FXG_NULL_ID && !(cfg->error_probability >= 0.0 && cfg->error_probability <= 1.0))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "error_probability %g: it must lie in [0, 1]", cfg->error_probability);
+    if (text_len >= (size_t(1) << 31))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "a text of %zu bytes: at most 2^31 - 1, split it at a record boundary", text_len);
+    CUDA_TRY(err, cudaSetDevice(c->device));
+    { std::lock_guard<std::mutex> lock(c->mu); K.host = take_staging(c); }
+    CUDA_TRY(err, cudaStreamCreateWithFlags(&K.st, cudaStreamNonBlocking));
+    cudaStream_t const s = K.st;
+    size_t const o_word = align_up(text_len, 64);              // read-backs go behind the text in the staging buffer
+    CUDA_TRY(err, K.host.ensure(o_word + 64));
+    uint64_t* const h_word = reinterpret_cast<uint64_t*>(K.host.as<uint8_t>() + o_word);
+    if (text_len) std::memcpy(K.host.p, text, text_len);
+    CUDA_TRY(err, K.text.ensure(text_len + 16));
+    if (text_len) CUDA_TRY(err, cudaMemcpyAsync(K.text.p, K.host.p, text_len, cudaMemcpyHostToDevice, s));
+    ctr.h2d_bytes += text_len;
+    const char* const dt = K.text.as<char>();
+
+    // ---- the newlines, the lines, the records ----
+    uint64_t n_nl = 0;
+    if (text_len) {
+        CUDA_TRY(err, K.nl.ensure(text_len * 4));
+        CUDA_TRY(err, K.n_nl.ensure(8));
+        thrust::counting_iterator<uint32_t> const at(0);
+        size_t tmp_bytes = 0;
+        CUDA_TRY(err, cub::DeviceSelect::If(nullptr, tmp_bytes, at, K.nl.as<uint32_t>(), K.n_nl.as<uint32_t>(), int(text_len), FastqNewline{dt}, s));
+        CUDA_TRY(err, K.scan_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        CUDA_TRY(err, cub::DeviceSelect::If(K.scan_tmp.p, tmp_bytes, at, K.nl.as<uint32_t>(), K.n_nl.as<uint32_t>(), int(text_len), FastqNewline{dt}, s));
+        CUDA_TRY(err, cudaMemcpyAsync(h_word, K.n_nl.p, 4, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        ctr.d2h_bytes += 4;
+        ctr.kernel_launches += 1;
+        n_nl = *reinterpret_cast<uint32_t*>(h_word);
+    }
+    uint64_t const n_lines = n_nl + (text_len && text[text_len - 1] != '\n' ? 1 : 0);
+    uint64_t const n_full = n_lines / 4;
+    FastqArgs const A{dt, text_len, K.nl.as<uint32_t>(), n_nl, n_full, cfg->error_probability, cfg->query_errors, cfg->seed_errors};
+    uint64_t first_bad = n_lines % 4 ? n_full : UINT64_MAX;    // a record cut short can only be the last one
+    uint64_t pool_len = 0;
+    const FastqRec* recs = nullptr;
+    if (n_full) {
+        CUDA_TRY(err, K.recs.ensure(n_full * sizeof(FastqRec)));
+        CUDA_TRY(err, K.lens.ensure((n_full + 1) * 8));
+        CUDA_TRY(err, K.offs.ensure((n_full + 1) * 8));
+        CUDA_TRY(err, K.first_bad.ensure(8));
+        CUDA_TRY(err, cudaMemsetAsync(K.lens.as<uint64_t>() + n_full, 0, 8, s));
+        CUDA_TRY(err, cudaMemsetAsync(K.first_bad.p, 0xff, 8, s));
+        fastq_record_kernel<<<uint32_t((n_full + 255) / 256), 256, 0, s>>>(A, K.recs.as<FastqRec>(), K.lens.as<uint64_t>(),
+                                                                          K.first_bad.as<unsigned long long>());
+        CUDA_TRY(err, cudaGetLastError());
+        size_t tmp_bytes = 0;
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, K.lens.as<uint64_t>(), K.offs.as<uint64_t>(), int(n_full + 1), s));
+        CUDA_TRY(err, K.scan_tmp.ensure(std::max<size_t>(tmp_bytes, 16)));
+        CUDA_TRY(err, cub::DeviceScan::ExclusiveSum(K.scan_tmp.p, tmp_bytes, K.lens.as<uint64_t>(), K.offs.as<uint64_t>(), int(n_full + 1), s));
+        ctr.kernel_launches += 2;
+        // the records, the first malformed one and the pools' length come back
+        size_t const o_recs = o_word + 64;
+        CUDA_TRY(err, K.host.ensure(o_recs + n_full * sizeof(FastqRec)));          // (the text's upload is through: the stream was drained)
+        uint64_t* const hw = reinterpret_cast<uint64_t*>(K.host.as<uint8_t>() + o_word);
+        CUDA_TRY(err, cudaMemcpyAsync(hw, K.first_bad.p, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaMemcpyAsync(hw + 1, K.offs.as<uint64_t>() + n_full, 8, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaMemcpyAsync(K.host.as<uint8_t>() + o_recs, K.recs.p, n_full * sizeof(FastqRec), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(err, cudaStreamSynchronize(s));
+        ctr.d2h_bytes += 16 + n_full * sizeof(FastqRec);
+        first_bad = std::min<uint64_t>(first_bad, hw[0]);
+        pool_len = hw[1];
+        recs = reinterpret_cast<const FastqRec*>(K.host.as<uint8_t>() + o_recs);
+    }
+    if (first_bad != UINT64_MAX) {
+        unsigned long long const r = first_bad;
+        if (first_bad == n_full) return fail(err, FXG_ERR_INVALID_ARGUMENT, "record %llu is cut short: it has %llu of its 4 lines", r, (unsigned long long)(n_lines % 4));
+        if (recs[first_bad].fault == kFastqNoAt) return fail(err, FXG_ERR_INVALID_ARGUMENT, "record %llu: the header line does not start with '@'", r);
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "record %llu: the third line does not start with '+'", r);
+    }
+
+    // ---- the ranks into the pools on the device, the kept reads' trees on the host meanwhile ----
+    CUDA_TRY(err, K.pool.ensure(2 * pool_len + 64));
+    if (pool_len) {
+        fastq_ranks_kernel<<<uint32_t((n_full * 32 + 255) / 256), 256, 0, s>>>(A, K.recs.as<FastqRec>(), K.offs.as<uint64_t>(), K.pool.as<uint8_t>());
+        CUDA_TRY(err, cudaGetLastError());
+        ctr.kernel_launches += 1;
+    }
+    out.pool_len = pool_len;
+    out.statuses.resize(n_full);
+    std::vector<uint64_t> kept;
+    for (uint64_t r = 0; r < n_full; ++r) {
+        out.statuses[r] = recs[r].status;
+        if (recs[r].status == FXG_READ_KEPT) kept.push_back(r);
+    }
+    size_t const n = kept.size();
+    out.reads.assign(n, fxg_read{});
+    out.spans.resize(n);
+    size_t const T = parallel_threads(n, 512);
+    std::vector<std::vector<fxg_pex_node>> chunk_nodes(T);
+    std::vector<int> chunk_rc(T, FXG_OK);
+    parallel_chunks(T, n, [&](size_t t, size_t lo, size_t hi) {
+        for (size_t i = lo; i < hi && chunk_rc[t] == FXG_OK; ++i) {
+            FastqRec const& F = recs[kept[i]];
+            fxg_pex_node *inner = nullptr, *leaves = nullptr;
+            size_t ni = 0, nlv = 0;
+            chunk_rc[t] = fxg_pex_build(F.l_seq, F.errors, cfg->seed_errors, int(cfg->build_strategy), &inner, &ni, &leaves, &nlv);
+            if (chunk_rc[t] == FXG_OK) {
+                fxg_read& R = out.reads[i];
+                R.node_offset = chunk_nodes[t].size();           // (within the chunk for now)
+                R.query_len = F.l_seq; R.num_inner = uint32_t(ni); R.num_leaves = uint32_t(nlv);
+                chunk_nodes[t].insert(chunk_nodes[t].end(), inner, inner + ni);
+                chunk_nodes[t].insert(chunk_nodes[t].end(), leaves, leaves + nlv);
+            }
+            fxg_pex_free(inner); fxg_pex_free(leaves);
+            out.spans[i] = fxg_read_span{kept[i], F.id, F.qual, F.l_id, F.l_qual};
+        }
+    });
+    for (int rc : chunk_rc) if (rc != FXG_OK) return fail(err, rc, "cannot build the PEX trees");
+    std::vector<uint64_t> chunk_base(T + 1, 0);
+    for (size_t t = 0; t < T; ++t) chunk_base[t + 1] = chunk_base[t] + chunk_nodes[t].size();
+    out.nodes.resize(chunk_base[T]);
+    for (size_t t = 0; t < T; ++t) std::copy(chunk_nodes[t].begin(), chunk_nodes[t].end(), out.nodes.begin() + long(chunk_base[t]));
+    uint64_t q = 0;
+    for (size_t t = 0; t < T; ++t)
+        for (size_t i = n * t / T; i < n * (t + 1) / T; ++i) {           // parallel_chunks' split
+            out.reads[i].node_offset += chunk_base[t];
+            out.reads[i].query_offset = q;
+            q += out.reads[i].query_len;
+        }
+    if (q != pool_len) return fail(err, FXG_ERR_CUDA, "internal: the kept reads hold %llu bases, the pools %llu", (unsigned long long)q, (unsigned long long)pool_len);
+    CUDA_TRY(err, cudaStreamSynchronize(s));
+    return FXG_OK;
+}
+
+void add_call_counters(fxg_ctx* c, fxg_counters const& ctr) {
+    std::lock_guard<std::mutex> lock(c->mu);
+    c->ctr.h2d_bytes += ctr.h2d_bytes; c->ctr.d2h_bytes += ctr.d2h_bytes; c->ctr.kernel_launches += ctr.kernel_launches;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fxg_parse_fastq(fxg_ctx* c, const fxg_read_config* cfg, const char* text, size_t text_len, fxg_parsed** out) {
+    std::string err;
+    if (!c || !cfg || !out || (text_len && !text)) return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_parse_fastq: a required argument is null");
+    *out = nullptr;
+    try {
+        std::unique_ptr<fxg_parsed> P(new fxg_parsed());
+        fxg_counters ctr{};
+        ParseScratch K{c};
+        int rc = parse_on_device(c, cfg, text, text_len, K, *P, ctr, err);
+        size_t const n = 2 * P->pool_len;
+        if (rc == FXG_OK && n) {                                   // the pools come back
+            P->pools.resize(n);
+            if (K.host.ensure(n) != cudaSuccess || cudaMemcpyAsync(K.host.p, K.pool.p, n, cudaMemcpyDeviceToHost, K.st) != cudaSuccess ||
+                cudaStreamSynchronize(K.st) != cudaSuccess)
+                rc = fail(err, FXG_ERR_CUDA, "cannot copy the pools back");
+            else std::memcpy(P->pools.data(), K.host.p, n);
+            ctr.d2h_bytes += n;
+        }
+        add_call_counters(c, ctr);
+        if (rc == FXG_OK) *out = P.release();
+        return rc;
+    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
+}
+
+int fxg_parsed_get(const fxg_parsed* P, fxg_parsed_view* v) {
+    if (!P || !v) return FXG_ERR_INVALID_ARGUMENT;
+    v->n_records = P->statuses.size(); v->statuses = P->statuses.data();
+    v->n_reads = P->reads.size(); v->reads = P->reads.data(); v->spans = P->spans.data();
+    v->pool_len = P->pool_len; v->forward_pool = P->pools.data(); v->reverse_complement_pool = P->pools.data() + P->pool_len;
+    v->n_nodes = P->nodes.size(); v->nodes = P->nodes.data();
+    return FXG_OK;
+}
+
+void fxg_parsed_free(fxg_parsed* P) { delete P; }
+
+int fxg_map_fastq(fxg_ctx* c, const fxg_gpu_seeder* S, const fxg_read_config* rcfg, const fxg_verify_config* vcfg,
+                  uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                  const char* text, size_t text_len, size_t n_references, const char* const* reference_ids, const uint64_t* reference_lengths,
+                  int format, int with_header, uint8_t** bytes, size_t* bytes_len, fxg_map_summary* summary) {
+    std::string err;
+    if (!c || !S || !rcfg || !vcfg || !bytes || !bytes_len || (text_len && !text) || (n_references && (!reference_ids || !reference_lengths)))
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "fxg_map_fastq: a required argument is null");
+    if (format != FXG_FORMAT_BAM && format != FXG_FORMAT_SAM && format != FXG_FORMAT_SAM_BGZF)
+        return fail(err, FXG_ERR_INVALID_ARGUMENT, "format %d: FXG_FORMAT_BAM, _SAM or _SAM_BGZF", format);
+    *bytes = nullptr; *bytes_len = 0;
+    try {
+        fxg_parsed P;
+        fxg_counters ctr{};
+        ParseScratch K{c};
+        int rc = parse_on_device(c, rcfg, text, text_len, K, P, ctr, err);
+        add_call_counters(c, ctr);
+        if (rc != FXG_OK) return rc;
+        // ---- the reads the q-gram seeder takes (seeder.cpp:162); the others are counted and not written ----
+        std::vector<fxg_read> reads;
+        std::vector<fxg_read_span> spans;
+        reads.reserve(P.reads.size()); spans.reserve(P.reads.size());
+        for (size_t i = 0; i < P.reads.size(); ++i) {
+            fxg_read const& R = P.reads[i];
+            const fxg_pex_node* lv = P.nodes.data() + R.node_offset + R.num_inner;
+            bool ok = true;
+            for (uint32_t li = 0; li < R.num_leaves && ok; ++li) {
+                uint64_t const m = lv[li].query_index_to - lv[li].query_index_from + 1, e = lv[li].num_errors;
+                ok = e <= uint64_t(kSeedMaxErrors) && m / (e + 1) >= S->q;
+            }
+            if (ok) { reads.push_back(R); spans.push_back(P.spans[i]); }
+            else P.statuses[P.spans[i].record] = FXG_READ_UNSEEDABLE;
+        }
+        // ---- seeding and verification: the job's pool is filled from the parsed pools on the device ----
+        fxg_job* job = nullptr;
+        fxg_seed_stats st{};
+        if (!reads.empty()) {
+            const uint8_t* const fwd = K.pool.as<uint8_t>();
+            rc = seed_verify(c, S, vcfg, reads.data(), reads.size(), fwd, fwd + P.pool_len, P.pool_len, P.nodes.data(), P.nodes.size(),
+                             max_anchors_hard, max_anchors_soft, erase_useless_anchors, &st, &job, cudaMemcpyDeviceToDevice);
+            if (rc != FXG_OK) return rc;
+        }
+        // ---- the records: SEQ from the parsed forward pool, names and qualities from the text, on the device ----
+        DeviceReads const dev{K.pool.as<uint8_t>(), K.text.as<char>(), spans.data()};
+        size_t const n_al = job ? fxg_job_num_alignments(job) : 0;
+        rc = write_on_device(format == FXG_FORMAT_BAM, format != FXG_FORMAT_SAM, c, job ? fxg_job_alignments(job) : nullptr, n_al,
+                             job ? fxg_job_cigar_pool(job) : nullptr, n_references, reference_ids, reference_lengths, reads.data(), reads.size(),
+                             nullptr, nullptr, with_header, bytes, bytes_len, &dev);
+        fxg_job_free(c, job);
+        if (rc != FXG_OK) return rc;
+        if (summary) {
+            *summary = fxg_map_summary{};
+            summary->records = P.statuses.size();
+            for (uint8_t x : P.statuses) summary->reads[x]++;
+            summary->alignments = n_al;
+            summary->seed = st;
+        }
+        return FXG_OK;
+    } catch (...) { return fail(err, FXG_ERR_OUT_OF_MEMORY, "cannot allocate host memory"); }
 }
 
 }  // extern "C"

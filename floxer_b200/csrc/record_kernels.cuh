@@ -25,7 +25,7 @@ namespace fxg {
 // one read as the record kernels see it (built by the host from fxg_read / fxg_sam_query)
 struct OutReadRec {
     uint64_t seq;                // its ranks in the uploaded forward-pool range
-    uint64_t name, qual;         // offsets of its name and its quality string in their buffers
+    uint64_t name, qual;         // offsets of its name and its quality string in their buffers (or both in the text)
     uint32_t l_seq, l_name;      // l_seq = 0: SEQ '*' (SAM); l_name: BAM's counts the NUL
     uint32_t l_qual, al0;        // l_qual = 0: no usable quality (SAM: QUAL '*'; BAM: QUAL 0xff)
     uint32_t n_al, rec0;         // its alignments; its first record
@@ -169,7 +169,7 @@ __global__ void bam_write_kernel(OutArgs A, uint32_t n_rec) {
         put_le(p + 24, ~0u, 4); put_le(p + 28, ~0u, 4); put_le(p + 32, 0, 4);     // no mate
     }
     p += 36;
-    for (uint32_t j = lane; j < R.l_name; j += 32) p[j] = uint8_t(A.names[R.name + j]);
+    for (uint32_t j = lane; j < R.l_name; j += 32) p[j] = j + 1 < R.l_name ? uint8_t(A.names[R.name + j]) : uint8_t(0);     // (the NUL)
     p += R.l_name;
     for (uint32_t j = lane; j < n_written; j += 32) put_le(p + 4 * j, long_cigar ? placeholder[j] : ops[j], 4);
     p += 4 * size_t(n_written);

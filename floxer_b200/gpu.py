@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import abi
-from .batch import ReadBatch, VerifyConfig
+from .batch import ReadBatch, ReadConfig, VerifyConfig
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libfloxer_gpu.so")
@@ -25,6 +25,7 @@ EXPORTS = [
     "fxg_seeder_create", "fxg_seeder_free", "fxg_seeder_search",
     "fxg_gpu_seeder_create", "fxg_gpu_seeder_free", "fxg_seed_reads", "fxg_seed_verify_reads",
     "fxg_write_bam_device", "fxg_job_write_bam_device", "fxg_write_sam", "fxg_write_sam_device", "fxg_job_write_sam_device",
+    "fxg_parse_fastq", "fxg_parsed_get", "fxg_parsed_free", "fxg_map_fastq",
 ]
 
 _lib = None
@@ -102,8 +103,37 @@ def lib() -> C.CDLL:
                                  C.POINTER(abi.SeedStats)]
     L.fxg_seed_verify_reads.argtypes = [vp, vp, vp, vp, sz, vp, vp, sz, vp, sz, C.c_uint64, C.c_uint64, C.c_int,
                                         C.POINTER(abi.SeedStats), C.POINTER(vp)]
+    L.fxg_parse_fastq.argtypes = [vp, C.POINTER(abi.ReadConfig), C.c_char_p, sz, C.POINTER(vp)]
+    L.fxg_parsed_get.argtypes = [vp, C.POINTER(abi.ParsedView)]
+    L.fxg_parsed_free.argtypes = [vp]
+    L.fxg_parsed_free.restype = None
+    L.fxg_map_fastq.argtypes = [vp, vp, C.POINTER(abi.ReadConfig), C.POINTER(abi.VerifyConfig), C.c_uint64, C.c_uint64, C.c_int,
+                                C.c_char_p, sz, sz, vp, vp, C.c_int, C.c_int, C.POINTER(vp), C.POINTER(sz), C.POINTER(abi.MapSummary)]
     _lib = L
     return L
+
+
+FORMATS = {"bam": abi.FORMAT_BAM, "sam": abi.FORMAT_SAM, "sam.gz": abi.FORMAT_SAM_BGZF}
+
+
+class ParsedFastq:
+    """What fxg_parse_fastq made of a FASTQ text, copied out: `statuses` (abi.READ_* per record), `batch` (the kept reads
+    as a ReadBatch without anchors, ready for seed_reads / seed_verify_reads / verify_reads), `spans`
+    (abi.READ_SPAN_DTYPE per kept read: its record index and the spans of its id and quality in the text), and the ids
+    and qualities those spans cut from the text."""
+
+    def __init__(self, text: bytes, view: abi.ParsedView):
+        def arr(p, n, dt):
+            dt = np.dtype(dt)
+            return np.frombuffer(C.string_at(p, n * dt.itemsize), dtype=dt).copy() if n else np.zeros(0, dtype=dt)
+        self.statuses = arr(view.statuses, view.n_records, np.uint8)
+        self.spans = arr(view.spans, view.n_reads, abi.READ_SPAN_DTYPE)
+        self.batch = ReadBatch(arr(view.reads, view.n_reads, abi.READ_DTYPE), arr(view.forward_pool, view.pool_len, np.uint8),
+                               arr(view.reverse_complement_pool, view.pool_len, np.uint8), arr(view.nodes, view.n_nodes, abi.PEX_NODE_DTYPE),
+                               np.zeros(0, dtype=abi.ANCHOR_DTYPE))
+        cut = lambda o, n: text[int(o): int(o) + int(n)].decode("latin-1")
+        self.ids = [cut(s["id_offset"], s["id_len"]) for s in self.spans]
+        self.qualities = [cut(s["quality_offset"], s["quality_len"]) for s in self.spans]
 
 
 class _SamQuery(C.Structure):
@@ -475,6 +505,41 @@ class Context:
         data = _write(lib().fxg_write_sam_device, (self._h, *_alignment_arrays(alignments, cigars)), batch, reference_ids,
                       reference_lengths, query_ids, qualities, header, int(bgzf), ctx=self)
         return data if bgzf else data.decode()
+
+    # ---- FASTQ input on the device ----
+    def parse_fastq(self, text: bytes, config: ReadConfig) -> ParsedFastq:
+        """fxg_parse_fastq: the records of a FASTQ text parsed on this context's device, the trees built on the host."""
+        text = bytes(text)
+        cfg, h = config.to_c(), C.c_void_p()
+        self._check(lib().fxg_parse_fastq(self._h, C.byref(cfg), text, len(text), C.byref(h)))
+        try:
+            view = abi.ParsedView()
+            self._check(lib().fxg_parsed_get(h, C.byref(view)))
+            return ParsedFastq(text, view)
+        finally:
+            lib().fxg_parsed_free(h)
+
+    def map_fastq(self, seeder: GpuSeeder, text: bytes, read_config: ReadConfig, verify_config: VerifyConfig, reference_ids,
+                  reference_lengths, fmt: str = "bam", header: bool = True, max_anchors_hard: int = 500, max_anchors_soft: int = 50,
+                  erase_useless: bool = True):
+        """fxg_map_fastq: a FASTQ text parsed, seeded, verified and written in one call.  fmt is "bam", "sam" or "sam.gz"
+        (BGZF-compressed SAM).  Returns (the output bytes, summary dict: records, kept, too_few_errors, bad_length,
+        unseedable, alignments, seed)."""
+        if fmt not in FORMATS:
+            raise ValueError(f"fmt {fmt!r}: one of {sorted(FORMATS)}")
+        text = bytes(text)
+        n_ref = len(reference_ids)
+        ref_ids = (C.c_char_p * max(n_ref, 1))(*[r.encode() for r in reference_ids])
+        ref_lens = (C.c_uint64 * max(n_ref, 1))(*[int(x) for x in reference_lengths])
+        rcfg, vcfg, summary = read_config.to_c(), verify_config.to_c(), abi.MapSummary()
+        out, length = C.c_void_p(), C.c_size_t(0)
+        self._check(lib().fxg_map_fastq(self._h, seeder._h, C.byref(rcfg), C.byref(vcfg), max_anchors_hard, max_anchors_soft,
+                                        int(erase_useless), text, len(text), n_ref, ref_ids, ref_lens, FORMATS[fmt], int(header),
+                                        C.byref(out), C.byref(length), C.byref(summary)))
+        try:
+            return C.string_at(out, length.value), summary.as_dict()
+        finally:
+            lib().fxg_free(out)
 
     # ---- accounting ----
     def counters(self) -> dict:

@@ -21,6 +21,8 @@
  *                        fxg_seeder_search with its index (fxg_gpu_seeder_create) built from the resident references.
  *   fxg_seed_verify_reads a search task's seeding and verification of a batch in one call (src/lib/parallelization.cpp:94-101
  *                        then :230-249): fxg_seed_reads + fxg_verify_reads with the anchors kept in device memory.
+ *   fxg_parse_fastq      the queries' reader (input::read_queries, src/lib/input.cpp) for a FASTQ text, on the device.
+ *   fxg_map_fastq        a whole run over one FASTQ text: parsing, seeding, verification and BAM / SAM output.
  *
  * Struct layouts fxg_pex_node and fxg_anchor are byte-identical to pex::pex_tree::node
  * (include/pex.hpp:59-70) and search::anchor_t (include/search.hpp:27-31) on LP64, so the
@@ -371,6 +373,69 @@ int  fxg_seed_verify_reads(fxg_ctx* ctx, const fxg_gpu_seeder* seeder, const fxg
                            const fxg_pex_node* nodes, size_t n_nodes,
                            uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
                            fxg_seed_stats* stats, fxg_job** out);
+
+/* ---- FASTQ input on the device ----
+ * The text of fxg_parse_fastq / fxg_map_fastq holds whole FASTQ records of four lines: '@' and a header, the sequence,
+ * '+' and anything, the quality.  Lines end at '\n'; one '\r' before the end of a line is dropped; the last line may lack
+ * its '\n' (multi-line records are not read).  A read's id is its header after '@' up to the first space or tab.  Its
+ * ranks follow input.cpp:165-176 ('$' -> 0, A C G T in either case -> 1..4, any other byte -> 5), its reverse complement
+ * swaps A<->T and C<->G.  Its error budget k is query_errors, or floating_point_error_aware_ceil(m * error_probability)
+ * when query_errors is FXG_NULL_ID (math.hpp:22-27, input.cpp:26-34), and its PEX tree is fxg_pex_build(m, k,
+ * seed_errors, build_strategy).  The text is uploaded once, through page-locked staging, on a stream of the call's own;
+ * the device finds the lines and records, checks them, cuts the ids, converts the ranks and lays out the kept reads'
+ * pools; the trees are built on the host.  A text of 2^31 bytes or more is refused (split it at a record boundary). */
+typedef struct {
+    double error_probability;   /* used when query_errors == FXG_NULL_ID */
+    uint64_t query_errors;      /* k of every read, or FXG_NULL_ID */
+    uint64_t seed_errors;       /* the leaves' error budget (leaf_max_num_errors) */
+    uint32_t build_strategy;    /* 0 recursive, 1 bottom_up */
+    uint32_t reserved;
+} fxg_read_config;
+/* a record's status: kept, or skipped and not written -- k < seed_errors (input.cpp:114-129), m = 0 or
+ * m > FXG_MAX_QUERY_LENGTH (input.cpp:106-110), or (fxg_map_fastq) a leaf the q-gram seeder refuses */
+enum { FXG_READ_KEPT = 0, FXG_READ_TOO_FEW_ERRORS = 1, FXG_READ_BAD_LENGTH = 2, FXG_READ_UNSEEDABLE = 3 };
+enum { FXG_FORMAT_BAM = 0, FXG_FORMAT_SAM = 1, FXG_FORMAT_SAM_BGZF = 2 };
+
+/* where a kept read came from: its record's index and the spans of its id and its quality in the text */
+typedef struct { uint64_t record, id_offset, quality_offset; uint32_t id_len, quality_len; } fxg_read_span;
+
+typedef struct fxg_parsed fxg_parsed;
+/* the arrays of a parsed text; they live as long as the fxg_parsed.  reads / pools / nodes go into fxg_seed_reads,
+ * fxg_seed_verify_reads and fxg_verify_reads as they are (the reads' anchor fields are zero). */
+typedef struct {
+    size_t n_records; const uint8_t* statuses;           /* per record: FXG_READ_* */
+    size_t n_reads; const fxg_read* reads; const fxg_read_span* spans;    /* the kept reads, in record order */
+    size_t pool_len; const uint8_t* forward_pool; const uint8_t* reverse_complement_pool;
+    size_t n_nodes; const fxg_pex_node* nodes;
+} fxg_parsed_view;
+
+/* Parses text[0, text_len).  A malformed record (a header without '@', a third line without '+', a record cut short)
+ * fails the call with FXG_ERR_INVALID_ARGUMENT and fxg_last_error names the first one's index.  Copies the pools back. */
+int fxg_parse_fastq(fxg_ctx* ctx, const fxg_read_config* config, const char* text, size_t text_len, fxg_parsed** out);
+int fxg_parsed_get(const fxg_parsed* parsed, fxg_parsed_view* view);
+void fxg_parsed_free(fxg_parsed* parsed);
+
+typedef struct {
+    uint64_t records;            /* FASTQ records in the text */
+    uint64_t reads[4];           /* records per FXG_READ_* status; reads[FXG_READ_KEPT] were mapped and written */
+    uint64_t alignments;
+    fxg_seed_stats seed;
+} fxg_map_summary;
+
+/* Maps a FASTQ text in one call: fxg_parse_fastq on the device, the trees on the host, then the kept reads -- less those
+ * with a leaf the q-gram seeder refuses (fewer than q * (errors + 1) bases or more than 8 errors: FXG_READ_UNSEEDABLE, a
+ * limit of the stand-in seeder, counted and not written) -- through fxg_seed_verify_reads and the device record writer
+ * (format FXG_FORMAT_*: fxg_write_bam_device, fxg_write_sam_device with bgzf 0 or 1).  The output is that of those calls
+ * composed on the kept reads in record order, with each read's id and quality: SAM the same bytes, BAM and BGZF SAM the
+ * same uncompressed stream and blocks.  The query pools do not go up a second time: the job's pool is filled from the
+ * parsed pool on the device, SEQ is read from it and the names and qualities from the device copy of the text.  Refusals
+ * keep the codes of the calls composed (for example a name of more than 254 characters in BAM).  Several threads may map
+ * on one context.  Copies are counted in fxg_counters h2d_bytes / d2h_bytes.  summary may be NULL.
+ * Writes a malloc'ed buffer; release it with fxg_free. */
+int fxg_map_fastq(fxg_ctx* ctx, const fxg_gpu_seeder* seeder, const fxg_read_config* read_config, const fxg_verify_config* verify_config,
+                  uint64_t max_anchors_hard, uint64_t max_anchors_soft, int erase_useless_anchors,
+                  const char* text, size_t text_len, size_t n_references, const char* const* reference_ids, const uint64_t* reference_lengths,
+                  int format, int with_header, uint8_t** bytes, size_t* bytes_len, fxg_map_summary* summary);
 
 /* ---- accounting / measurement helpers ---- */
 int fxg_get_counters(const fxg_ctx* ctx, fxg_counters* out);
